@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            # the CUDA engine (this repo)
     python bench.py --impl reference [--gpus N] --steps K --warmup W   # the reference's CPU algorithm
+    python bench.py ... --dump-outputs DIR     # also write what the last timed step computed as DIR/<name>.npy
 
 One "step" = one ply of lock-step self-play for every game of the batch: MCTS.search_batch(100, 8)
 (= 800 descents, lib/mcts.py:162-176) on each of the G games, then the policy / sampling / move of
@@ -353,6 +354,61 @@ def extra_configs(torch, dist, world, rank, seed, small=False, net_sms=0):
     return out
 
 
+# ----------------------------------------------------------------------------------------- outputs of the timed path
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def last_ply_outputs(engs):
+    """What the self-play path hands its caller after a ply, as float32 / float64 host arrays (parts in order):
+    every game's position (device board words: occupied mask, black stones; exact in float64, Connect4 uses bits < 49),
+    side to move and ply count after the move, the search policy of the move each game that goes on just made, and the
+    replay tuples of the games that ended in the ply (re-seated: ply 0).  The ring holds those games' blocks in the order
+    the device reserved them, which varies from run to run, so the tuples are sorted.  Needs auto-restarted play with at
+    least one ply before the last one (bench.py's pre-roll)."""
+    import numpy as np
+    import torch
+    boards, players, plies, move_pi, rows = [], [], [], [], []
+    for e in engs:
+        ply = e.region("ply").long()
+        hist = e.fregion("hist_pi")                                   # [games, max plies, A]
+        idx = (ply - 1).clamp(0, hist.shape[1] - 1)
+        pi = hist[torch.arange(e.G, device=hist.device), idx] * (ply > 0).unsqueeze(1)
+        boards.append(e.region("root_board").cpu().numpy().astype(np.float64))
+        players.append(e.region("root_player").cpu().numpy().astype(np.float32))
+        plies.append(ply.cpu().numpy().astype(np.float32))
+        move_pi.append(pi.cpu().numpy())
+        cursor, cap = e.replay_cursor(), e.cfg.replay_capacity
+        live = min(cursor, cap)
+        slots = torch.arange(cursor - live, cursor, device=hist.device) % cap
+        ring = np.concatenate([e.region("replay_board")[slots].cpu().numpy().astype(np.float64),
+                               e.region("replay_player")[slots].cpu().numpy().astype(np.float64)[:, None],
+                               e.fregion("replay_pi")[slots].cpu().numpy().astype(np.float64),
+                               e.fregion("replay_z")[slots].cpu().numpy().astype(np.float64)[:, None]], axis=1)
+        ended = int((plies[-1] == 0).sum())
+        starts = np.flatnonzero(ring[:, 0] == 0)                       # a game's block opens with the empty board
+        assert ended <= len(starts), "the replay ring no longer holds the games that ended in the last ply"
+        rows.append(ring[starts[len(starts) - ended]:] if ended else ring[:0])
+    rows = np.concatenate(rows)
+    rows = rows[np.lexsort(rows.T[::-1])]
+    out = {"root_board": np.concatenate(boards), "root_player": np.concatenate(players), "root_ply": np.concatenate(plies),
+           "move_pi": np.concatenate(move_pi)}
+    budget = DUMP_LIMIT_BYTES - sum(a.nbytes for a in out.values())
+    row_bytes = 2 * 8 + 4 + 4 * (rows.shape[1] - 4) + 4
+    if len(rows) * row_bytes > budget:  # a fixed, seeded sample of the tuples keeps the dump within its limit
+        keep = np.sort(np.random.default_rng(0).choice(len(rows), budget // row_bytes, replace=False))
+        rows = rows[keep]
+    out.update(replay_board=rows[:, :2], replay_player=rows[:, 2].astype(np.float32),
+               replay_pi=rows[:, 3:-1].astype(np.float32), replay_z=rows[:, -1].astype(np.float32))
+    return out
+
+
+def dump_outputs(path, arrays):
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 # ----------------------------------------------------------------------------------------- CUDA engine
 def engine_arm(args):
     import numpy as np
@@ -434,6 +490,8 @@ def engine_arm(args):
             prof[k] = prof.get(k, 0) + v
         e.profile(0)
     c1 = counters()
+    if args.dump_outputs:  # before the legs below play on with the same engines
+        dump_outputs(args.dump_outputs if world == 1 else os.path.join(args.dump_outputs, "rank%d" % rank), last_ply_outputs(engs))
 
     # ---- end-to-end: same plies driven through HOST buffers: pinned H2D of every game's root position + side to move,
     # D2H of the positions after the move AND of the self-play product -- the replay tuples (position, side, pi, z;
@@ -611,7 +669,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--extra-small", action="store_true", help="toy sizes for extra.configs (tests)")
     ap.add_argument("--no-extra", action="store_true", help="skip the extra.train / extra.configs measurements after the headline")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy (under torchrun: DIR/rank<r>/)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "engine":
+        ap.error("--dump-outputs writes the CUDA engine's outputs (--impl engine)")
     if args.impl == "reference":
         return reference_arm(args)
     return engine_arm(args)

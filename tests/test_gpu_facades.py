@@ -356,6 +356,37 @@ def test_bench_engine_arm_prints_the_contract_line():
     assert "workload" in d["config"] and d["dtype"] == "f16" and d["scaling"] == "weak"
 
 
+def test_bench_dumps_the_same_outputs_of_its_last_step_on_every_run(tmp_path):
+    """`bench.py --dump-outputs DIR`: float32 / float64 arrays within 64 MB, identical from run to run with the same
+    arguments; one position, side, ply and policy per game, and exactly one replay block (opened by the empty board)
+    per game that ended in the last ply."""
+    import subprocess
+    import sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    G = 512
+    runs = []
+    for i in range(2):
+        d = tmp_path / ("run%d" % i)
+        out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--games", str(G), "--steps", "3", "--warmup", "1",
+                              "--preroll", "20", "--no-cpu-baseline", "--no-extra", "--node-capacity", "8192", "--dump-outputs", str(d)],
+                             capture_output=True, text=True, timeout=900, cwd=root)
+        assert out.returncode == 0, out.stderr[-3000:]
+        runs.append({f[:-4]: np.load(d / f) for f in sorted(os.listdir(d))})
+    a, b = runs
+    assert set(a) == {"move_pi", "replay_board", "replay_pi", "replay_player", "replay_z", "root_board", "root_ply", "root_player"}
+    assert sum(x.nbytes for x in a.values()) <= 64 << 20
+    for name in a:
+        assert a[name].dtype in (np.float32, np.float64), name
+        np.testing.assert_array_equal(a[name], b[name], err_msg=name)
+    assert a["root_board"].shape == (G, 2) and a["move_pi"].shape == (G, 7) and a["root_ply"].shape == a["root_player"].shape == (G,)
+    going_on = a["root_ply"] > 0
+    np.testing.assert_allclose(a["move_pi"][going_on].sum(axis=1), 1.0, atol=1e-5)
+    assert (a["move_pi"][~going_on] == 0).all()
+    assert int((a["replay_board"][:, 0] == 0).sum()) == int((~going_on).sum())
+    assert set(np.unique(a["replay_z"])) <= {-1.0, 0.0, 1.0}
+    np.testing.assert_allclose(a["replay_pi"].sum(axis=1), 1.0, atol=1e-5)
+
+
 def test_connect4_pipeline_matches_single_engine_play():
     """The parts pipeline (CUDA graph per ply, expand+backup with eight lanes per game, noise prefetched under the network
     pass) vs a single engine's play() (separate launches, expand+backup with one warp per game): same seeds => the same

@@ -182,6 +182,16 @@ def test_bench_reference_arm_prints_the_contract_line():
     assert out.returncode == 0 and out.stdout.strip() == ""
 
 
+def test_bench_refuses_zero_steps_and_a_dump_of_the_cpu_arm(tmp_path):
+    import subprocess
+    import sys
+    for extra in (["--steps", "0"], ["--impl", "reference", "--steps", "1", "--dump-outputs", str(tmp_path / "d")]):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + extra, capture_output=True, text=True, timeout=120,
+                             cwd=ROOT)
+        assert out.returncode == 2 and out.stdout == "", (extra, out.stderr)
+    assert not os.path.exists(tmp_path / "d")
+
+
 def test_render_strings_match_the_reference(golden_render):
     """game.render (connect_four.py:267-281, tictactoe.py:237-259) and Session.render (play_session.py:38-49) byte for
     byte against strings produced by the unmodified reference (tests/golden/make_golden2.py)."""
