@@ -34,7 +34,9 @@ _SIGNATURES = {
     "caro_backup_path": (C.c_int, [_P, _P, _P, _P, C.c_int, C.c_float, _P]),
     "caro_net_blob_floats": (C.c_size_t, [C.c_int, C.c_int, C.c_int]),
     "caro_net_blob_floats_deep": (C.c_size_t, [C.c_int, C.c_int, C.c_int, C.c_int]),
+    "caro_net_blob_floats_shape": (C.c_size_t, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int]),
     "caro_net_create": (C.c_int, [C.c_int, C.c_int, C.c_int, _P, C.c_size_t, C.POINTER(_P)]),
+    "caro_net_create_shape": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P, C.c_size_t, C.POINTER(_P)]),
     "caro_net_update": (C.c_int, [_P, _P, C.c_size_t]),
     "caro_net_destroy": (None, [_P]),
     "caro_net_set_trace": (C.c_int, [_P, _P]),

@@ -6,7 +6,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libcaro_b200.so")
-SOURCES = ["common.cu", "boards.cu", "engine.cu", "net.cu", "net_tc.cu", "net_rt.cu", "net_rx.cu", "net_heads.cu"]
+SOURCES = ["common.cu", "boards.cu", "engine.cu", "net.cu", "net_tc.cu", "net_rt.cu", "net_rx.cu", "net_heads.cu", "net_wide.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xptxas", "-v"]
 

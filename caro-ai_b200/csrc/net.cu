@@ -17,8 +17,10 @@ namespace caro {
 
 __device__ __forceinline__ float lrelu(float x) { return x > 0.0f ? x : kLeaky * x; }
 
-// One block per leaf.  Dynamic smem: 2 x [64][HW] activations + head scratch.
-template <class R>
+// One block per leaf, F filters.  Dynamic smem: 2 x [F][HW] activations + head scratch.  For F = 128 the two activation
+// buffers alone take 230,400 B at 15 x 15, so the head scratch reuses the buffer the last layer read from: everything
+// stays in the block's own shared memory, and launches that overlap on other streams share nothing.
+template <class R, int F>
 __global__ void __launch_bounds__(256)
 net_simt_kernel(R rules, const typename R::Board* __restrict__ boards, const uint8_t* __restrict__ who,
                 const int32_t* __restrict__ d_count, long long max_count, const float* __restrict__ blob, BlobLayout L,
@@ -27,8 +29,7 @@ net_simt_kernel(R rules, const typename R::Board* __restrict__ boards, const uin
   const int H = rules.rows(), W = rules.cols(), HW = H * W;
   const long long count = d_count ? min((long long)*d_count, max_count) : max_count;
   float* buf0 = sm;
-  float* buf1 = sm + kFilters * HW;
-  float* head = buf1 + kFilters * HW;  // [3*HW + 32 + A]
+  float* buf1 = sm + F * HW;
   for (long long leaf = blockIdx.x; leaf < count; leaf += gridDim.x) {
     const typename R::Board s = boards[leaf];
     const int wm = who[leaf];
@@ -36,8 +37,8 @@ net_simt_kernel(R rules, const typename R::Board* __restrict__ boards, const uin
     for (int i = threadIdx.x; i < 2 * HW; i += blockDim.x)
       buf1[i] = (float)rules.plane_value(s, wm, i / HW, (i % HW) / W, i % W);
     __syncthreads();
-    // conv_in: 2 -> 64
-    for (int o = threadIdx.x; o < kFilters * HW; o += blockDim.x) {
+    // conv_in: 2 -> F
+    for (int o = threadIdx.x; o < F * HW; o += blockDim.x) {
       const int co = o / HW, pos = o % HW, r = pos / W, c = pos % W;
       float acc = blob[L.conv_in_b + co];
       for (int ci = 0; ci < 2; ++ci)
@@ -58,11 +59,11 @@ net_simt_kernel(R rules, const typename R::Board* __restrict__ boards, const uin
     for (int layer = 0; layer < L.blocks; ++layer) {
       const float* wgt = blob + L.conv_w[layer];
       const float* bias = blob + L.conv_b[layer];
-      for (int o = threadIdx.x; o < kFilters * HW; o += blockDim.x) {
+      for (int o = threadIdx.x; o < F * HW; o += blockDim.x) {
         const int co = o / HW, pos = o % HW, r = pos / W, c = pos % W;
         float acc = bias[co];
-        for (int ci = 0; ci < kFilters; ++ci) {
-          const float* wk = wgt + (size_t)(co * kFilters + ci) * 9;
+        for (int ci = 0; ci < F; ++ci) {
+          const float* wk = wgt + (size_t)(co * F + ci) * 9;
           const float* in = cur + ci * HW;
           for (int ky = 0; ky < 3; ++ky) {
             const int rr = r + ky - 1;
@@ -81,12 +82,13 @@ net_simt_kernel(R rules, const typename R::Board* __restrict__ boards, const uin
       cur = nxt;
       nxt = t;
     }
+    float* head = F == kFilters ? buf1 + F * HW : nxt;  // [3*HW + 32 + A]
     // heads: 1x1 convs (value: 1 channel, policy: 2 channels)
     for (int i = threadIdx.x; i < 3 * HW; i += blockDim.x) {
       const int ch = i / HW, pos = i % HW;
-      const float* wv = ch == 0 ? blob + L.val_conv_w : blob + L.pol_conv_w + (ch - 1) * kFilters;
+      const float* wv = ch == 0 ? blob + L.val_conv_w : blob + L.pol_conv_w + (ch - 1) * F;
       float acc = ch == 0 ? blob[L.val_conv_b] : blob[L.pol_conv_b + ch - 1];
-      for (int ci = 0; ci < kFilters; ++ci) acc += wv[ci] * cur[ci * HW + pos];
+      for (int ci = 0; ci < F; ++ci) acc += wv[ci] * cur[ci * HW + pos];
       head[i] = lrelu(acc);  // [0,HW) value plane, [HW,3HW) policy planes (channel-major, lib/model.py:93)
     }
     __syncthreads();
@@ -126,11 +128,20 @@ template <class R>
 int launch_simt(const R& rules, const caro_net* net, const void* boards, const uint8_t* who, const int32_t* d_count,
                 int64_t max_count, float* probs, float* values, cudaStream_t st) {
   const int HW = net->H * net->W;
+  const unsigned grid = (unsigned)(max_count < 148 * 8 ? (max_count > 0 ? max_count : 1) : 148 * 8);
+  if (net->layout.filters == kWideFilters) {  // the head scratch lives in the spare activation buffer
+    const size_t smem = sizeof(float) * ((size_t)2 * kWideFilters * HW + 8);
+    auto kern = net_simt_kernel<R, kWideFilters>;
+    cudaError_t ce = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (ce != cudaSuccess) return caro_fail(CARO_E_CUDA, cudaGetErrorString(ce));
+    kern<<<grid, 256, smem, st>>>(rules, (const typename R::Board*)boards, who, d_count, (long long)max_count, net->d_blob,
+                                  net->layout, net->A, probs, values);
+    return caro_check_launch("net_simt_kernel");
+  }
   const size_t smem = sizeof(float) * ((size_t)2 * kFilters * HW + 3 * HW + 32 + net->A + 8);
-  auto kern = net_simt_kernel<R>;
+  auto kern = net_simt_kernel<R, kFilters>;
   cudaError_t ce = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (ce != cudaSuccess) return caro_fail(CARO_E_CUDA, cudaGetErrorString(ce));
-  const unsigned grid = (unsigned)(max_count < 148 * 8 ? (max_count > 0 ? max_count : 1) : 148 * 8);
   kern<<<grid, 256, smem, st>>>(rules, (const typename R::Board*)boards, who, d_count, (long long)max_count, net->d_blob,
                                 net->layout, net->A, probs, values);
   return caro_check_launch("net_simt_kernel");
@@ -149,6 +160,11 @@ size_t caro_net_blob_floats_deep(int rows, int cols, int actions, int blocks) {
   return blob_layout(rows, cols, actions, blocks).total;
 }
 
+size_t caro_net_blob_floats_shape(int rows, int cols, int actions, int blocks, int filters) {
+  if (blocks < 1 || blocks > kMaxBlocks || (filters != kFilters && filters != kWideFilters)) return 0;
+  return blob_layout(rows, cols, actions, blocks, filters).total;
+}
+
 int caro_net_update(caro_net* net, const float* h_blob, size_t n_floats) {
   if (!net || !h_blob) return caro_fail(CARO_E_ARG, "null argument");
   if (n_floats != net->layout.total) return caro_fail(CARO_E_ARG, "weight blob has the wrong size");
@@ -159,6 +175,7 @@ int caro_net_update(caro_net* net, const float* h_blob, size_t n_floats) {
   if (cudaDeviceSynchronize() != cudaSuccess) return caro_fail(CARO_E_CUDA, "device error before the weight update");
   cudaError_t ce = cudaMemcpy(net->d_blob, h_blob, n_floats * sizeof(float), cudaMemcpyHostToDevice);
   if (ce != cudaSuccess) return caro_fail(CARO_E_CUDA, cudaGetErrorString(ce));
+  if (net->layout.filters == kWideFilters) return caro_net_wide_pack(net, h_blob);
   const int rc = caro_net_tc_pack(net, h_blob);
   if (rc != CARO_OK) return rc;
   if (!caro_net_rt_supports(net)) return CARO_OK;
@@ -166,10 +183,8 @@ int caro_net_update(caro_net* net, const float* h_blob, size_t n_floats) {
   return rc2 != CARO_OK ? rc2 : caro_net_rx_pack(net, h_blob);
 }
 
-int caro_net_create(int rows, int cols, int actions, const float* h_blob, size_t n_floats, caro_net** out) {
-  if (!out || !h_blob) return caro_fail(CARO_E_ARG, "null argument");
-  if (rows < 2 || cols < 2 || rows > 15 || cols > 15 || actions < 1 || actions > 255) return caro_fail(CARO_E_ARG, "bad net shape");
-  if (caro_device_count() <= 0) return caro_fail(CARO_E_CUDA, "no CUDA device: the network has no CPU fallback");
+// Allocates and fills a handle once the caller has validated the shape and found a device.
+static int net_create(int rows, int cols, int actions, const BlobLayout& layout, const float* h_blob, size_t n_floats, caro_net** out) {
   static std::atomic<unsigned long long> next_serial{0};
   caro_net* net = new caro_net();
   net->serial = ++next_serial;
@@ -177,16 +192,7 @@ int caro_net_create(int rows, int cols, int actions, const float* h_blob, size_t
   net->H = rows;
   net->W = cols;
   net->A = actions;
-  {  // the depth of the tower is read off the blob's length: base + blocks x (64 x 64 x 9 + 64) floats
-    const size_t per_block = (size_t)kFilters * kFilters * 9 + kFilters;
-    const size_t base = blob_layout(rows, cols, actions, 1).total - per_block;
-    const size_t blocks = n_floats > base ? (n_floats - base) / per_block : 0;
-    if (blocks < 1 || blocks > (size_t)kMaxBlocks || base + blocks * per_block != n_floats) {
-      delete net;
-      return caro_fail(CARO_E_ARG, "weight blob has the wrong size");
-    }
-    net->layout = blob_layout(rows, cols, actions, (int)blocks);
-  }
+  net->layout = layout;
   net->d_blob = nullptr;
   net->d_tc_weights = nullptr;
   net->d_rt_weights = nullptr;
@@ -196,6 +202,7 @@ int caro_net_create(int rows, int cols, int actions, const float* h_blob, size_t
   net->d_rt_scratch = nullptr;
   net->rt_scratch_seq = 0;
   net->d_rx_weights = nullptr;
+  net->d_wide_weights = nullptr;
   net->d_tc_bias = nullptr;
   net->d_pol_fc_t = nullptr;
   net->d_trace = nullptr;
@@ -214,6 +221,7 @@ int caro_net_create(int rows, int cols, int actions, const float* h_blob, size_t
     if (prc == CARO_OK) prc = caro_net_rt_prepare();
     if (prc == CARO_OK) prc = caro_net_rx_prepare();
     if (prc == CARO_OK) prc = caro_net_heads_prepare();
+    if (prc == CARO_OK) prc = caro_net_wide_prepare();
     if (prc != CARO_OK) {
       delete net;
       return prc;
@@ -225,7 +233,7 @@ int caro_net_create(int rows, int cols, int actions, const float* h_blob, size_t
   }
   cudaError_t ce = cudaMalloc(&net->d_blob, n_floats * sizeof(float));
   if (ce != cudaSuccess) {
-    delete net;
+    caro_net_destroy(net);
     return caro_fail(CARO_E_CUDA, cudaGetErrorString(ce));
   }
   const int rc = caro_net_update(net, h_blob, n_floats);
@@ -235,6 +243,35 @@ int caro_net_create(int rows, int cols, int actions, const float* h_blob, size_t
   }
   *out = net;
   return CARO_OK;
+}
+
+static bool bad_net_shape(int rows, int cols, int actions) {
+  return rows < 2 || cols < 2 || rows > 15 || cols > 15 || actions < 1 || actions > 255;
+}
+
+int caro_net_create(int rows, int cols, int actions, const float* h_blob, size_t n_floats, caro_net** out) {
+  if (!out || !h_blob) return caro_fail(CARO_E_ARG, "null argument");
+  if (bad_net_shape(rows, cols, actions)) return caro_fail(CARO_E_ARG, "bad net shape");
+  if (caro_device_count() <= 0) return caro_fail(CARO_E_CUDA, "no CUDA device: the network has no CPU fallback");
+  // the depth of the tower is read off the blob's length: base + blocks x (64 x 64 x 9 + 64) floats
+  const size_t per_block = (size_t)kFilters * kFilters * 9 + kFilters;
+  const size_t base = blob_layout(rows, cols, actions, 1).total - per_block;
+  const size_t blocks = n_floats > base ? (n_floats - base) / per_block : 0;
+  if (blocks < 1 || blocks > (size_t)kMaxBlocks || base + blocks * per_block != n_floats)
+    return caro_fail(CARO_E_ARG, "weight blob has the wrong size");
+  return net_create(rows, cols, actions, blob_layout(rows, cols, actions, (int)blocks), h_blob, n_floats, out);
+}
+
+int caro_net_create_shape(int rows, int cols, int actions, int blocks, int filters, const float* h_blob, size_t n_floats,
+                          caro_net** out) {
+  if (!out || !h_blob) return caro_fail(CARO_E_ARG, "null argument");
+  if (bad_net_shape(rows, cols, actions)) return caro_fail(CARO_E_ARG, "bad net shape");
+  if (blocks < 1 || blocks > kMaxBlocks) return caro_fail(CARO_E_ARG, "bad tower depth: 1 .. 20 residual blocks are supported");
+  if (filters != kFilters && filters != kWideFilters) return caro_fail(CARO_E_ARG, "bad tower width: 64 or 128 filters are supported");
+  const BlobLayout layout = blob_layout(rows, cols, actions, blocks, filters);
+  if (n_floats != layout.total) return caro_fail(CARO_E_ARG, "weight blob has the wrong size for the stated shape");
+  if (caro_device_count() <= 0) return caro_fail(CARO_E_CUDA, "no CUDA device: the network has no CPU fallback");
+  return net_create(rows, cols, actions, layout, h_blob, n_floats, out);
 }
 
 int caro_net_set_grid_limit(caro_net* net, int ctas) {
@@ -256,6 +293,7 @@ void caro_net_destroy(caro_net* net) {
   caro_net_rt_free(net);
   caro_net_rx_free(net);
   caro_net_heads_free(net);
+  caro_net_wide_free(net);
   if (net->d_blob) cudaFree(net->d_blob);
   delete net;
 }
@@ -271,6 +309,12 @@ int caro_net_forward(caro_net* net, int game, int n, int k, const void* d_boards
     if (net->H != n || net->W != n || net->A != n * n) return caro_fail(CARO_E_ARG, "net shape does not match the m,n,k board");
   } else {
     return caro_fail(CARO_E_ARG, "unknown game");
+  }
+  if (net->layout.filters == kWideFilters && impl != 1) {
+    // 128 filters: impl 7 = the wide tower with fp16 operands, 0 / 3 = the same with bf16 operands
+    if (impl != 0 && impl != 3 && impl != 7)
+      return caro_fail(CARO_E_ARG, "a 128-filter network runs impl 0, 1, 3 or 7 only (no split-precision, CTA-pair or row-tiled tower)");
+    return caro_net_wide_forward(net, game, n, k, d_boards, d_who, d_count, max_count, d_probs, d_values, impl == 7, st);
   }
   if (impl == 1) {
     if (game == CARO_GAME_CONNECT4) return launch_simt<C4Rules>(C4Rules(), net, d_boards, d_who, d_count, max_count, d_probs, d_values, st);

@@ -8,9 +8,10 @@
 namespace caro {
 
 constexpr int kFilters = 64;      // lib/model.py:7
+constexpr int kWideFilters = 128; // the only other width: net_wide.cu's tower and the SIMT tower's wide instance
 constexpr int kBlocks = 5;        // conv_1 .. conv_5: the reference's depth (lib/model.py:21-45)
 constexpr int kMaxBlocks = 20;    // deepest tower the kernels accept ("deep residual net" of BASELINE configs[3]): the number of
-                                  // residual blocks is a run-time property of the weight blob, the width (64 filters) is not
+                                  // residual blocks is a run-time property of the weight blob
 constexpr float kLeaky = 0.01f;   // nn.LeakyReLU default slope
 
 // Offsets (in floats) of the folded-weight blob described in include/caro_b200.h
@@ -18,31 +19,34 @@ struct BlobLayout {
   size_t conv_in_w, conv_in_b;
   size_t conv_w[kMaxBlocks], conv_b[kMaxBlocks];
   int blocks;
+  int filters;  // kFilters or kWideFilters
   size_t val_conv_w, val_conv_b, val_fc1_w, val_fc1_b, val_fc2_w, val_fc2_b;
   size_t pol_conv_w, pol_conv_b, pol_fc_w, pol_fc_b;
   size_t total;
 };
 
-inline BlobLayout blob_layout(int H, int W, int A, int blocks = kBlocks) {
+inline BlobLayout blob_layout(int H, int W, int A, int blocks = kBlocks, int filters = kFilters) {
   BlobLayout L;
   L.blocks = blocks;
+  L.filters = filters;
+  const size_t F = (size_t)filters;
   for (int i = 0; i < kMaxBlocks; ++i) L.conv_w[i] = L.conv_b[i] = 0;
   size_t o = 0;
   const size_t hw = (size_t)H * W;
   auto take = [&](size_t n) { size_t r = o; o += n; return r; };
-  L.conv_in_w = take(kFilters * 2 * 9);
-  L.conv_in_b = take(kFilters);
+  L.conv_in_w = take(F * 2 * 9);
+  L.conv_in_b = take(F);
   for (int i = 0; i < blocks; ++i) {
-    L.conv_w[i] = take((size_t)kFilters * kFilters * 9);
-    L.conv_b[i] = take(kFilters);
+    L.conv_w[i] = take(F * F * 9);
+    L.conv_b[i] = take(F);
   }
-  L.val_conv_w = take(kFilters);
+  L.val_conv_w = take(F);
   L.val_conv_b = take(1);
   L.val_fc1_w = take(20 * hw);
   L.val_fc1_b = take(20);
   L.val_fc2_w = take(20);
   L.val_fc2_b = take(1);
-  L.pol_conv_w = take(2 * kFilters);
+  L.pol_conv_w = take(2 * F);
   L.pol_conv_b = take(2);
   L.pol_fc_w = take((size_t)A * 2 * hw);
   L.pol_fc_b = take(A);
@@ -64,8 +68,9 @@ struct caro_net {
   void* d_rt_scratch;       // CTA-pair form: head features + FC scratch of every CTA, kRtScratchSlots launches in flight
   unsigned rt_scratch_seq;  // next slot (round robin per launch)
   void* d_rx_weights;   // fp16 hi / lo UMMA B-operand blocks of the split-precision row-tiled tower -- see net_rx.cu
+  void* d_wide_weights; // 128-wide handles: fp16 then bf16 UMMA B-operand images of every (layer, tap) -- see net_wide.cu
   alignas(16) float h_rt_consts[(caro::kMaxBlocks + 1) * 64 + 3 * 64 + 4 + 1536 + 4];  // host copy of the row-tiled tower's by-value constants (RtConsts)
-  float* d_tc_bias;     // [6][64] folded conv biases
+  float* d_tc_bias;     // [1 + blocks][filters] folded conv biases
   float* d_pol_fc_t;    // policy FC transposed to [2*HW][A] (+ value FC1 [HW][20]) for coalesced reads in the TC epilogue
   void* d_headfeat;     // large boards: exported activated head features, bf16 hi + lo images in the A-operand layout of net_heads.cu
   void* d_heads_b;      // large boards: bf16 hi + lo B-operand image of the FC heads GEMM (net_heads.cu)
@@ -96,6 +101,13 @@ void caro_net_rt_free(caro_net* net);
 bool caro_net_rt_supports(const caro_net* net);
 int caro_net_rt_forward(caro_net* net, int game, int n, int k, const void* d_boards, const uint8_t* d_who,
                         const int32_t* d_count, int64_t max_count, float* d_probs, float* d_values, int mode, cudaStream_t st);
+
+// net_wide.cu (tap-per-MMA tower of 128-filter networks, N = 128 per MMA, weights streamed tap by tap)
+int caro_net_wide_pack(caro_net* net, const float* h_blob);
+int caro_net_wide_prepare();
+void caro_net_wide_free(caro_net* net);
+int caro_net_wide_forward(caro_net* net, int game, int n, int k, const void* d_boards, const uint8_t* d_who,
+                          const int32_t* d_count, int64_t max_count, float* d_probs, float* d_values, bool f16, cudaStream_t st);
 
 // net_rx.cu (split-precision row-tiled tower, fp16 hi + lo, boards up to 6 x 7)
 int caro_net_rx_pack(caro_net* net, const float* h_blob);

@@ -98,46 +98,6 @@ using TcExact = TcCfg<2, true>;
 using TcPair = TcCfg<4, false, true>;
 
 
-// Large boards (Caro 15x15: 225 actions, 450 x 225 policy FC) do not run their FC heads inside the tower: two head warps
-// re-reading 405 KB of FC weights for every 2-board group made the heads, not the convolutions, the bottleneck (1.9 ms
-// per 4,096 leaves, of which ~0.3 ms tower).  The tower only exports, per leaf, the ACTIVATED outputs of the 1x1 head
-// convolutions (bias + LeakyReLU applied here) as bf16 hi + lo pairs, already in the UMMA A-operand layout of the heads
-// GEMM (net_heads.cu): images [tile of 128 leaves][K / 8][128 rows][8], K = 3 HW padded to 64, one 16-byte store per
-// (leaf, 8 features) and image; heads_tc_kernel then evaluates both FC layers on the tensor cores.
-template <int TEAM, int BAR>
-__device__ __noinline__ void export_heads(const TcGeom& gm, int nvalid, long long leaf0, int ttid, float* headf_s, const float* headw_s,
-                                          uint8_t* __restrict__ out_hi, size_t lo_off, int kc8) {
-  const int HW = gm.H * gm.W, K = 3 * HW;
-  const float hb0 = headw_s[192], hb1 = headw_s[193], hb2 = headw_s[194];
-#pragma unroll 1
-  for (int item = ttid; item < nvalid * kc8; item += TEAM) {
-    const int b = item / kc8, c8 = item - b * kc8;
-    const long long leaf = leaf0 + b;
-    const float* f = headf_s + (size_t)b * K;
-    uint32_t hi[4], lo[4];
-#pragma unroll
-    for (int e = 0; e < 4; ++e) {
-      float v[2];
-#pragma unroll
-      for (int u = 0; u < 2; ++u) {
-        const int k = c8 * 8 + 2 * e + u;
-        v[u] = k < K ? lrelu_tc(f[k] + (k < HW ? hb0 : (k < 2 * HW ? hb1 : hb2))) : 0.0f;
-      }
-      const __nv_bfloat162 h2 = __floats2bfloat162_rn(v[0], v[1]);
-      const __nv_bfloat162 l2 = __floats2bfloat162_rn(v[0] - __low2float(h2), v[1] - __high2float(h2));
-      hi[e] = *reinterpret_cast<const uint32_t*>(&h2);
-      lo[e] = *reinterpret_cast<const uint32_t*>(&l2);
-    }
-    uint8_t* dst = out_hi + (((size_t)(leaf >> 7) * kc8 + c8) * 128 + (size_t)(leaf & 127)) * 16;
-    *reinterpret_cast<uint4*>(dst) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
-    *reinterpret_cast<uint4*>(dst + lo_off) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
-  }
-  asm volatile("bar.sync %0, %1;" ::"n"(BAR), "n"(TEAM) : "memory");
-#pragma unroll 1
-  for (int i = ttid; i < nvalid * K; i += TEAM) headf_s[i] = 0.0f;  // re-arm the accumulation slots
-  asm volatile("bar.sync %0, %1;" ::"n"(BAR), "n"(TEAM) : "memory");
-}
-
 // ------------------------------------------------------------------------------------- kernel
 // Roles: warps 0-7 = epilogue (warp w owns TMEM lanes [32(w&3), +32) = rows of every tile, channels 32(w>>2)..+32),
 //        warp 8    = TMEM allocation, elected-lane MMA issue for tiles 0 and 2,
@@ -245,8 +205,8 @@ net_tc_kernel(R rules, TcGeom gm, const typename R::Board* __restrict__ boards, 
       const long long leaf0 = group_leaf0(gi);
       const int nvalid = group_valid(leaf0);
       mbar_wait(bar_feat + 0, (uint32_t)gi & 1u);
-      if (headfeat_out != nullptr) export_heads<kHeadThreads, 2>(gm, nvalid, leaf0, htid, headf_s, headw_s, headfeat_out, headfeat_lo_off, headfeat_kc8);
-      else run_heads<kHeadThreads, 2>(gm, nb, nvalid, leaf0, htid, headf_s, fc_s, headw_s, blob, L, pol_fc_t, val_fc1_t, probs, values);
+      if (headfeat_out != nullptr) export_heads<kHeadThreads, 2>(gm, nvalid, leaf0, htid, headf_s, headw_s + 192, headfeat_out, headfeat_lo_off, headfeat_kc8);
+      else run_heads<kHeadThreads, 2>(gm, nb, nvalid, leaf0, htid, headf_s, fc_s, headw_s + 192, blob, L, pol_fc_t, val_fc1_t, probs, values);
       mbar_arrive(bar_feat + 1);  // features consumed, slots re-zeroed, scratch free
       if (htid == 0) TC_TRACE(5, gi);  // heads done
     }
@@ -519,8 +479,8 @@ net_tc_kernel(R rules, TcGeom gm, const typename R::Board* __restrict__ boards, 
         // last group of this CTA: nothing left to overlap with, so all eight epilogue warps do the heads
         asm volatile("bar.sync 1, 256;" ::: "memory");
         const int nvalid = group_valid(leaf0);
-        if (headfeat_out != nullptr) export_heads<kEpiThreads, 1>(gm, nvalid, leaf0, tid, headf_s, headw_s, headfeat_out, headfeat_lo_off, headfeat_kc8);
-        else run_heads<kEpiThreads, 1>(gm, nb, nvalid, leaf0, tid, headf_s, fc_s, headw_s, blob, L, pol_fc_t, val_fc1_t, probs, values);
+        if (headfeat_out != nullptr) export_heads<kEpiThreads, 1>(gm, nvalid, leaf0, tid, headf_s, headw_s + 192, headfeat_out, headfeat_lo_off, headfeat_kc8);
+        else run_heads<kEpiThreads, 1>(gm, nb, nvalid, leaf0, tid, headf_s, fc_s, headw_s + 192, blob, L, pol_fc_t, val_fc1_t, probs, values);
         if (tid == 0) TC_TRACE(5, gi);
       }
     }

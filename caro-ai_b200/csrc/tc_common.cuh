@@ -1,5 +1,5 @@
-// Shared device helpers of the tcgen05 towers (net_tc.cu, net_rt.cu): PTX wrappers, descriptors, TMEM
-// load/store macros, the debug timeline macro and the fully connected heads.
+// Shared device helpers of the tcgen05 towers (net_tc.cu, net_rt.cu, net_wide.cu): PTX wrappers, descriptors, TMEM
+// load/store macros, the debug timeline macro, the head-feature export and the fully connected heads.
 #pragma once
 #include <cuda_bf16.h>
 #include <cuda_runtime.h>
@@ -107,6 +107,46 @@ __device__ __forceinline__ float lrelu_tc(float x) { return fmaxf(x, kLeaky * x)
     if (trace != nullptr && blockIdx.x == 0 && (idx) < 1000) trace[(kind) * 1000 + (idx)] = clock64(); \
   } while (0)
 
+// Large boards (Caro 15x15: 225 actions, 450 x 225 policy FC) do not run their FC heads inside the tower: two head warps
+// re-reading 405 KB of FC weights for every 2-board group made the heads, not the convolutions, the bottleneck (1.9 ms
+// per 4,096 leaves, of which ~0.3 ms tower).  The tower only exports, per leaf, the ACTIVATED outputs of the 1x1 head
+// convolutions (bias + LeakyReLU applied here; `head_b` = the three head biases) as bf16 hi + lo pairs, already in the UMMA A-operand layout of the heads
+// GEMM (net_heads.cu): images [tile of 128 leaves][K / 8][128 rows][8], K = 3 HW padded to 64, one 16-byte store per
+// (leaf, 8 features) and image; heads_tc_kernel then evaluates both FC layers on the tensor cores.
+template <int TEAM, int BAR>
+__device__ __noinline__ void export_heads(const TcGeom& gm, int nvalid, long long leaf0, int ttid, float* headf_s, const float* head_b,
+                                          uint8_t* __restrict__ out_hi, size_t lo_off, int kc8) {
+  const int HW = gm.H * gm.W, K = 3 * HW;
+  const float hb0 = head_b[0], hb1 = head_b[1], hb2 = head_b[2];
+#pragma unroll 1
+  for (int item = ttid; item < nvalid * kc8; item += TEAM) {
+    const int b = item / kc8, c8 = item - b * kc8;
+    const long long leaf = leaf0 + b;
+    const float* f = headf_s + (size_t)b * K;
+    uint32_t hi[4], lo[4];
+#pragma unroll
+    for (int e = 0; e < 4; ++e) {
+      float v[2];
+#pragma unroll
+      for (int u = 0; u < 2; ++u) {
+        const int k = c8 * 8 + 2 * e + u;
+        v[u] = k < K ? lrelu_tc(f[k] + (k < HW ? hb0 : (k < 2 * HW ? hb1 : hb2))) : 0.0f;
+      }
+      const __nv_bfloat162 h2 = __floats2bfloat162_rn(v[0], v[1]);
+      const __nv_bfloat162 l2 = __floats2bfloat162_rn(v[0] - __low2float(h2), v[1] - __high2float(h2));
+      hi[e] = *reinterpret_cast<const uint32_t*>(&h2);
+      lo[e] = *reinterpret_cast<const uint32_t*>(&l2);
+    }
+    uint8_t* dst = out_hi + (((size_t)(leaf >> 7) * kc8 + c8) * 128 + (size_t)(leaf & 127)) * 16;
+    *reinterpret_cast<uint4*>(dst) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
+    *reinterpret_cast<uint4*>(dst + lo_off) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
+  }
+  asm volatile("bar.sync %0, %1;" ::"n"(BAR), "n"(TEAM) : "memory");
+#pragma unroll 1
+  for (int i = ttid; i < nvalid * K; i += TEAM) headf_s[i] = 0.0f;  // re-arm the accumulation slots
+  asm volatile("bar.sync %0, %1;" ::"n"(BAR), "n"(TEAM) : "memory");
+}
+
 // Fully connected heads of one group: value FC1 (HW -> 20) + FC2 + tanh, policy FC (2 HW -> A) + softmax over all
 // A actions (lib/model.py:56-72,90-93, lib/mcts.py:216), for all (board, output) pairs in parallel with coalesced
 // transposed weights; bias + LeakyReLU of the 1x1 head convolutions are applied on the fly.  Executed by a "team"
@@ -116,7 +156,7 @@ __device__ __forceinline__ float lrelu_tc(float x) { return fmaxf(x, kLeaky * x)
 // order, so that the result does not depend on the order in which the epilogue warps finished.
 template <int TEAM, int BAR, int NF = 1>
 __device__ __noinline__ void run_heads(const TcGeom& gm, int nb, int nvalid, long long leaf0, int ttid, float* headf_s,
-                                          float* fc_s, const float* headw_s, const float* __restrict__ blob, const BlobLayout& L,
+                                          float* fc_s, const float* head_b, const float* __restrict__ blob, const BlobLayout& L,
                                           const float* __restrict__ pol_fc_t, const float* __restrict__ val_fc1_t,
                                           float* __restrict__ probs, float* __restrict__ values, int fstride = 0) {
   const int HW = gm.H * gm.W;
@@ -137,7 +177,7 @@ __device__ __noinline__ void run_heads(const TcGeom& gm, int nb, int nvalid, lon
   const int per_board = 20 + gm.A;
   float* hid = fc_s;  // [nb][20] value hidden units, logits behind them
   float* logit = fc_s + nb * 20;
-  const float hb0 = headw_s[192], hb1 = headw_s[193], hb2 = headw_s[194];
+  const float hb0 = head_b[0], hb1 = head_b[1], hb2 = head_b[2];
 #pragma unroll 1
   for (int o = ttid; o < nvalid * per_board; o += TEAM) {
     const int b = o / per_board, i = o - b * per_board;

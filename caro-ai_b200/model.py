@@ -11,7 +11,7 @@ from __future__ import annotations
 
 import copy
 import ctypes as C
-from typing import Dict
+from typing import Dict, Tuple
 
 import numpy as np
 import torch
@@ -20,6 +20,7 @@ import torch.nn as nn
 from . import _cabi
 
 NUM_FILTERS = 64  # lib/model.py:7
+WIDTHS = (64, 128)  # filters of the towers the CUDA kernels evaluate
 BN_EPS = 1e-5
 
 
@@ -34,26 +35,34 @@ class Net(nn.Module):
     ``blocks`` (extension): number of residual blocks ``conv_1 .. conv_<blocks>``.  The reference has exactly five
     (lib/model.py:21-45) and that is the default -- same ``state_dict`` keys, same initialisation order; BASELINE.json
     configs[3] asks for a "deep residual net", which the reference does not define: here it is a deeper tower of the same
-    64-filter blocks (1..20), evaluated by the same CUDA kernels (the depth is read off the weight blob)."""
+    blocks (1..20), evaluated by the same CUDA kernels (the depth is read off the weight blob).
 
-    def __init__(self, input_shape, actions_n, blocks: int = 5):
+    ``filters`` (extension): the width of every convolution, 64 (the reference's NUM_FILTERS) or 128.  The key names are
+    the same at both widths, only the shapes scale."""
+
+    def __init__(self, input_shape, actions_n, blocks: int = 5, filters: int = NUM_FILTERS):
         super().__init__()
-        assert 1 <= blocks <= 20
+        if not 1 <= blocks <= 20:
+            raise ValueError("blocks must be 1 .. 20, got %r" % (blocks,))
+        if filters not in WIDTHS:
+            raise ValueError("filters must be one of %s, got %r" % (WIDTHS, filters))
         self.input_shape = tuple(input_shape)
         self.actions_n = int(actions_n)
         self.blocks = int(blocks)
+        self.filters = int(filters)
+        nf = self.filters
         _, h, w = self.input_shape
-        self.conv_in = _block(self.input_shape[0], NUM_FILTERS, 3)
+        self.conv_in = _block(self.input_shape[0], nf, 3)
         for i in range(1, self.blocks + 1):
-            setattr(self, "conv_%d" % i, _block(NUM_FILTERS, NUM_FILTERS, 3))
-        self.conv_val = _block(NUM_FILTERS, 1, 1)
+            setattr(self, "conv_%d" % i, _block(nf, nf, 3))
+        self.conv_val = _block(nf, 1, 1)
         # the reference sizes its heads by pushing zeros through them in train mode
         # (lib/model.py:55,69,74-80), leaving one BatchNorm running-stat update behind; kept so that
         # a fresh Net() here equals a fresh reference Net() under the same seed.
-        probe = torch.zeros(1, NUM_FILTERS, h, w)
+        probe = torch.zeros(1, nf, h, w)
         val_size = int(np.prod(self.conv_val(probe).size()))
         self.value = nn.Sequential(nn.Linear(val_size, 20), nn.LeakyReLU(), nn.Linear(20, 1), nn.Tanh())
-        self.conv_policy = _block(NUM_FILTERS, 2, 1)
+        self.conv_policy = _block(nf, 2, 1)
         pol_size = int(np.prod(self.conv_policy(probe).size()))
         self.policy = nn.Sequential(nn.Linear(pol_size, self.actions_n))
 
@@ -83,8 +92,17 @@ def _fold(conv_w, conv_b, bn_w, bn_b, mean, var):
     return conv_w * scale.view(-1, 1, 1, 1), (conv_b - mean) * scale + bn_b
 
 
+def state_dict_shape(sd: Dict[str, torch.Tensor]) -> Tuple[int, int]:
+    """(blocks, filters) of a ``Net`` state dict: the number of ``conv_N`` groups and the output channels of conv_in."""
+    blocks = 0
+    while "conv_%d.0.weight" % (blocks + 1) in sd:
+        blocks += 1
+    return blocks, int(sd["conv_in.0.weight"].shape[0])
+
+
 def fold_state_dict(sd: Dict[str, torch.Tensor], rows: int, cols: int, actions: int) -> np.ndarray:
-    """Eval-mode BN folding + flattening into the blob layout of include/caro_b200.h."""
+    """Eval-mode BN folding + flattening into the blob layout of include/caro_b200.h.  The depth and the width are read
+    off the state dict."""
     sd = {k: v.detach().double().cpu() for k, v in sd.items() if v.dtype.is_floating_point}
     parts = []
 
@@ -92,9 +110,7 @@ def fold_state_dict(sd: Dict[str, torch.Tensor], rows: int, cols: int, actions: 
         return _fold(sd[name + ".0.weight"], sd[name + ".0.bias"], sd[name + ".1.weight"], sd[name + ".1.bias"],
                      sd[name + ".1.running_mean"], sd[name + ".1.running_var"])
 
-    blocks = 0
-    while "conv_%d.0.weight" % (blocks + 1) in sd:
-        blocks += 1
+    blocks, filters = state_dict_shape(sd)
     for name in ["conv_in"] + ["conv_%d" % i for i in range(1, blocks + 1)]:
         w, b = folded(name)
         parts += [w.reshape(-1), b.reshape(-1)]
@@ -104,9 +120,10 @@ def fold_state_dict(sd: Dict[str, torch.Tensor], rows: int, cols: int, actions: 
     w, b = folded("conv_policy")
     parts += [w.reshape(-1), b.reshape(-1), sd["policy.0.weight"].reshape(-1), sd["policy.0.bias"].reshape(-1)]
     blob = torch.cat(parts).float().numpy()
-    hw = rows * cols
-    expect = 64 * 2 * 9 + 64 + blocks * (64 * 64 * 9 + 64) + 64 + 1 + 20 * hw + 20 + 20 + 1 + 2 * 64 + 2 + actions * 2 * hw + actions
-    assert blob.size == expect, (blob.size, expect)
+    expect = _cabi.lib().caro_net_blob_floats_shape(rows, cols, actions, blocks, filters)
+    if blob.size != expect:
+        raise ValueError("state dict of %d blocks x %d filters folds to %d floats, the %dx%d board's blob layout wants %d"
+                         % (blocks, filters, blob.size, rows, cols, expect))
     return np.ascontiguousarray(blob)
 
 
@@ -166,18 +183,28 @@ class DeviceNet:
         "bf16"   one bf16 tensor-core pass, fp32 accumulate (forced; the caller vouches for the tolerance),
         "bf16x3" hi/lo split of activations and weights, three MMAs per product: fp32-class accuracy (boards up to 6 x 7:
                  fp16 hi + lo, row-tiled; larger boards: bf16 hi + lo, tap-per-MMA),
-        "fp32-simt" the SIMT numerics-reference kernel."""
+        "fp32-simt" the SIMT numerics-reference kernel.
+        128-filter networks (``Net(filters=128)``) run the wide tensor-core tower (csrc/net_wide.cu) with fp16 or bf16
+        operands on every board size, or the SIMT tower; "auto" tries "fp16", then "bf16", then falls back to "fp32-simt",
+        and "bf16x3" is not available."""
         _cabi.require_cuda()
         assert precision in ("auto", "fp16", "bf16", "bf16x3", "fp32-simt")
-        self.requested = precision
         sd = net_or_state_dict.state_dict() if isinstance(net_or_state_dict, nn.Module) else net_or_state_dict
+        self.blocks, self.filters = state_dict_shape(sd)
+        if precision == "bf16x3" and self.filters != NUM_FILTERS:
+            raise ValueError("precision 'bf16x3' is not available for %d-filter networks (64 only)" % self.filters)
+        self.requested = precision
         _, self.rows, self.cols = game.obs_shape
         self.actions = game.action_space
         self.game = game
         blob = fold_state_dict(sd, self.rows, self.cols, self.actions)
         handle = C.c_void_p()
-        _cabi.check(_cabi.lib().caro_net_create(self.rows, self.cols, self.actions, blob.ctypes.data, blob.size,
-                                                C.byref(handle)))
+        if self.filters == NUM_FILTERS:
+            _cabi.check(_cabi.lib().caro_net_create(self.rows, self.cols, self.actions, blob.ctypes.data, blob.size,
+                                                    C.byref(handle)))
+        else:
+            _cabi.check(_cabi.lib().caro_net_create_shape(self.rows, self.cols, self.actions, self.blocks, self.filters,
+                                                          blob.ctypes.data, blob.size, C.byref(handle)))
         self.handle = handle
         self.calibration = None
         self._select(precision)
@@ -198,8 +225,11 @@ class DeviceNet:
         p32, v32 = self.forward_boards(d_boards, d_who, n, IMPL_SIMT)
         limit = CALIBRATION_MARGIN * PRIOR_TOLERANCE
         ok = False
-        self.calibration = {"positions": n}
-        candidates = [("fp16", IMPL_TCGEN05_F16)] if self.rows <= 6 and self.cols <= 7 else []  # the row-tiled towers' boards
+        self.calibration = {"positions": n, "filters": self.filters}
+        if self.filters != NUM_FILTERS:  # the wide tower: fp16 on every board, then bf16, then the SIMT tower (no split mode)
+            candidates = [("fp16", IMPL_TCGEN05_F16)]
+        else:
+            candidates = [("fp16", IMPL_TCGEN05_F16)] if self.rows <= 6 and self.cols <= 7 else []  # the row-tiled towers' boards
         for name, impl in candidates + [("bf16", IMPL_TCGEN05)]:  # both are measured (and recorded), the first that passes is used
             p16, v16 = self.forward_boards(d_boards, d_who, n, impl)
             dp = float((p16 - p32).abs().max().item())
@@ -211,9 +241,12 @@ class DeviceNet:
             if not ok and finite and dp <= limit and dv <= limit:
                 ok = True
                 self.calibration["selected"] = name
-        if not ok:
+        if ok:
+            return self.calibration["selected"]
+        if self.filters != NUM_FILTERS:  # no split mode for the wide tower
+            self.calibration["selected"] = "fp32-simt"
+        else:  # the split mode is checked too (fp16 hi + lo has a finite range): the SIMT tower is the last resort
             self.calibration["selected"] = "bf16x3"
-        if not ok:  # the split mode is checked too (fp16 hi + lo has a finite range): the SIMT tower is the last resort
             px, vx = self.forward_boards(d_boards, d_who, n, IMPL_TCGEN05_X3)
             dpx, dvx = float((px - p32).abs().max().item()), float((vx - v32).abs().max().item())
             self.calibration.update(split_max_abs_prior_diff=dpx, split_max_abs_value_diff=dvx)
@@ -262,9 +295,12 @@ class DeviceNet:
 
 
 def load_checkpoint(path: str, game) -> Net:
-    """play.py:29-35 / play_session.py:13-16: ``torch.load`` of a reference ``.dat`` state_dict."""
-    net = Net(game.obs_shape, game.action_space)
-    net.load_state_dict(torch.load(path, map_location=lambda storage, loc: storage))
+    """play.py:29-35 / play_session.py:13-16: ``torch.load`` of a reference ``.dat`` state_dict.  The ``Net`` is built
+    with the depth and width found in the file, so deeper and 128-filter checkpoints load as well as the reference's."""
+    sd = torch.load(path, map_location=lambda storage, loc: storage)
+    blocks, filters = state_dict_shape(sd)
+    net = Net(game.obs_shape, game.action_space, blocks=blocks, filters=filters)
+    net.load_state_dict(sd)
     return net
 
 

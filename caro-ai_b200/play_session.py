@@ -2,7 +2,6 @@
 from __future__ import annotations
 
 import numpy as np
-import torch
 
 from . import mcts, model
 
@@ -16,8 +15,7 @@ class Session:
         self.BOT_PLAYER = game.player_black
         self.USER_PLAYER = game.player_white
         self.model_file = model_file
-        self.model = model.Net(input_shape=game.obs_shape, actions_n=game.action_space)
-        self.model.load_state_dict(torch.load(model_file, map_location=lambda storage, loc: storage))
+        self.model = model.load_checkpoint(model_file, game)  # any depth and width the file holds
         self.model.eval()
         self.state = game.initial_state
         self.value = None

@@ -152,6 +152,9 @@ def parse_args(argv=None):
     p.add_argument("--compact-tree", action="store_true",
                    help="drop unreachable tree nodes after every move (bit-identical play, small arenas; for large boards)")
     p.add_argument("--evaluate-every", type=int, default=cfg.EVALUATE_EVERY_STEP, help="arena evaluation period in steps")
+    p.add_argument("--blocks", type=int, default=5, choices=range(1, 21), metavar="{1..20}",
+                   help="residual blocks of the network (reference: 5)")
+    p.add_argument("--filters", type=int, default=64, choices=[64, 128], help="filters of every convolution (reference: 64)")
     return p.parse_args(argv)
 
 
@@ -167,7 +170,7 @@ def main(argv=None):
         os.makedirs(saves_path, exist_ok=True)
     writer = make_writer(args.name) if rank == 0 else _NullWriter()
     game = get_game(args.game)
-    net = Net(game.obs_shape, game.action_space).to(device)
+    net = Net(game.obs_shape, game.action_space, blocks=args.blocks, filters=args.filters).to(device)
     D.broadcast_state_dict(net)
     best_net = NetWrapper(net)
     best_dev = DeviceNet(best_net.target_model, game)  # precision "auto", re-checked on every update()

@@ -80,24 +80,33 @@ int caro_backup_path(int32_t* d_n, float* d_w, float* d_q, const int64_t* d_edge
  * Policy/value network -- row a17 (lib/model.py:10-94) + the softmax of lib/mcts.py:216.
  * Weights are handed over ALREADY FOLDED (eval-mode BatchNorm merged into the convolutions,
  * done on the host by caro_ai_b200.model.fold_state_dict) as one float32 blob:
- *   conv_in  w[64][2][3][3] b[64] | blocks x ( w[64][64][3][3] b[64] ) |      (blocks = 5 in the reference)
- *   conv_val w[64] b[1] | value.0 w[20][HW] b[20] | value.2 w[20] b[1] |
- *   conv_policy w[2][64] b[2] | policy.0 w[A][2*HW] b[A]
+ *   conv_in  w[F][2][3][3] b[F] | blocks x ( w[F][F][3][3] b[F] ) |      (blocks = 5, F = 64 in the reference)
+ *   conv_val w[F] b[1] | value.0 w[20][HW] b[20] | value.2 w[20] b[1] |
+ *   conv_policy w[2][F] b[2] | policy.0 w[A][2*HW] b[A]
+ * F (the filters of every convolution) is 64 or 128.
  * ------------------------------------------------------------------------------------------ */
 typedef struct caro_net caro_net;
 
 size_t caro_net_blob_floats(int rows, int cols, int actions);
 /* The same for a tower of `blocks` residual blocks (1..20; the reference has 5, lib/model.py:21-45): the blob then holds
- * `blocks` x ( w[64][64][3][3] b[64] ) groups, and caro_net_create reads the depth off the blob's length.  The width
- * (64 filters) is fixed.  Returns 0 for an unsupported depth. */
+ * `blocks` x ( w[64][64][3][3] b[64] ) groups, and caro_net_create reads the depth off the blob's length.  The width is
+ * 64 filters.  Returns 0 for an unsupported depth. */
 size_t caro_net_blob_floats_deep(int rows, int cols, int actions, int blocks);
+/* The same for any supported shape: `blocks` 1..20 residual blocks of `filters` = 64 or 128 filters.  Returns 0 for an
+ * unsupported depth or width; with filters = 64 it equals caro_net_blob_floats_deep. */
+size_t caro_net_blob_floats_shape(int rows, int cols, int actions, int blocks, int filters);
 /* Copies and re-packs the blob into device memory owned by the handle (bf16 UMMA operand images
- * for the tensor-core tower + fp32 copies for the heads).  Synchronous. */
+ * for the tensor-core tower + fp32 copies for the heads).  Synchronous.  The width is 64 filters. */
 int caro_net_create(int rows, int cols, int actions, const float* h_blob, size_t n_floats,
                     caro_net** out);
+/* caro_net_create for a stated shape (`blocks` 1..20, `filters` 64 or 128).  Every argument, the blob's size included, is
+ * checked before the device is looked for: a bad shape returns CARO_E_ARG on any machine.  A 128-filter handle runs
+ * impl 7 (wide tower, fp16 operands), 0 / 3 (wide tower, bf16 operands) and 1 (SIMT); see caro_net_forward. */
+int caro_net_create_shape(int rows, int cols, int actions, int blocks, int filters, const float* h_blob, size_t n_floats,
+                          caro_net** out);
 int caro_net_update(caro_net* net, const float* h_blob, size_t n_floats);
 void caro_net_destroy(caro_net* net);
-/* Debug only: d_trace = device buffer of >= 8001 int64 (zeroed) that CTA 0 of the tensor-core kernel fills with
+/* Debug only: d_trace = device buffer of >= 8001 int64 (zeroed) that CTA 0 of the tensor-core kernels (net_tc.cu, net_wide.cu) fills with
  * (tag, clock64) pairs -- the pipeline timeline used to tune the kernel; NULL switches tracing off. */
 int caro_net_set_trace(caro_net* net, void* d_trace);
 
@@ -131,7 +140,10 @@ int caro_net_set_grid_limit(caro_net* net, int ctas);
  *             6 = the tap-per-MMA bf16 tower as CTA pairs (each CTA stores 32 of the 64 output channels of every tap; bit-identical
  *                 to impl 3; no faster stand-alone -- an M = 128, K = 16 MMA takes 48 cycles whatever N <= 64 is --, +1.5 % inside the
  *                 Caro self-play step; CARO_TC_PAIR=1 makes impl 0 / 3 use it),
- *             1 = fp32 SIMT tower (numerics reference kernel used by the tests). */
+ *             1 = fp32 SIMT tower (numerics reference kernel used by the tests).
+ *           128-filter handles (caro_net_create_shape): 7 = the wide tap-per-MMA tower (net_wide.cu: M = 128, N = 128, K = 16
+ *           MMAs, weights streamed tap by tap) with fp16 operands, 0 and 3 = the same tower with bf16 operands, 1 = the SIMT
+ *           tower; 2, 4, 5 and 6 return CARO_E_ARG. */
 int caro_net_forward(caro_net* net, int game, int n, int k, const void* d_boards,
                      const uint8_t* d_who, const int32_t* d_count, int64_t max_count,
                      float* d_probs, float* d_values, int impl, void* stream);
