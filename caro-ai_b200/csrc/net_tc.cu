@@ -20,6 +20,7 @@
 #include <math.h>
 #include <string.h>
 
+#include <algorithm>
 #include <vector>
 
 #include "../../include/caro_b200.h"
@@ -611,9 +612,10 @@ static int launch_tc(const R& rules, caro_net* net, const void* boards, const ui
   gm.A = net->A;
   gm.pitch = net->W + 1;
   gm.block = (net->H + 1) * gm.pitch;
-  gm.boards_per_group = K::kGroupRows / gm.block;
-  if (gm.boards_per_group < 1 || gm.boards_per_group > 32 || gm.pitch + 1 > kHalo ||
-      gm.boards_per_group * (20 + gm.A) > K::kFcFloats)
+  // as many boards as the group's rows hold, capped by the 32-board limit and the FC scratch (only 2 x 2 boards reach the
+  // caps: the rows past the last board are padding)
+  gm.boards_per_group = std::min(std::min(K::kGroupRows / gm.block, 32), K::kFcFloats / (20 + gm.A));
+  if (gm.boards_per_group < 1 || gm.pitch + 1 > kHalo)
     return caro_fail(CARO_E_ARG, "board does not fit the tensor-core tile geometry");
   const int lim = net->grid_limit > 0 ? net->grid_limit : net->pipeline_limit;
   const int sm_count = lim > 0 && lim < net->sm_count ? lim : net->sm_count;

@@ -24,6 +24,7 @@
 #include <cuda_runtime.h>
 #include <math.h>
 
+#include <algorithm>
 #include <vector>
 
 #include "../../include/caro_b200.h"
@@ -374,8 +375,10 @@ static int launch_wide(const R& rules, caro_net* net, const void* boards, const 
   gm.A = net->A;
   gm.pitch = net->W + 1;
   gm.block = (net->H + 1) * gm.pitch;
-  gm.boards_per_group = kGroupRows / gm.block;
-  if (gm.boards_per_group < 1 || gm.boards_per_group > 32 || gm.pitch + 1 > kHalo || gm.boards_per_group * (20 + gm.A) > kFcFloats)
+  // as many boards as the group's rows hold, capped by the 32-board limit and the FC scratch (only 2 x 2 boards reach the
+  // caps: the rows past the last board are padding)
+  gm.boards_per_group = std::min(std::min(kGroupRows / gm.block, 32), kFcFloats / (20 + gm.A));
+  if (gm.boards_per_group < 1 || gm.pitch + 1 > kHalo)
     return caro_fail(CARO_E_ARG, "board does not fit the wide tensor-core tile geometry");
   const int lim = net->grid_limit > 0 ? net->grid_limit : net->pipeline_limit;
   const int sm_count = lim > 0 && lim < net->sm_count ? lim : net->sm_count;
