@@ -311,11 +311,15 @@ int caro_net_forward(caro_net* net, int game, int n, int k, const void* d_boards
     return caro_fail(CARO_E_ARG, "unknown game");
   }
   if (net->layout.filters == kWideFilters && impl != 1) {
-    // 128 filters: impl 7 = the wide tower with fp16 operands, 0 / 3 = the same with bf16 operands
-    if (impl != 0 && impl != 3 && impl != 7)
-      return caro_fail(CARO_E_ARG, "a 128-filter network runs impl 0, 1, 3 or 7 only (no split-precision, CTA-pair or row-tiled tower)");
-    return caro_net_wide_forward(net, game, n, k, d_boards, d_who, d_count, max_count, d_probs, d_values, impl == 7, st);
+    // 128 filters: impl 7 = the wide tower with fp16 operands, 0 / 3 = the same with bf16 operands, 8 = bf16 hi + lo
+    if (impl != 0 && impl != 3 && impl != 7 && impl != 8)
+      return caro_fail(CARO_E_ARG, "a 128-filter network runs impl 0, 1, 3, 7 or 8 only (no CTA-pair or row-tiled tower; "
+                                   "its split-precision tower is impl 8)");
+    return caro_net_wide_forward(net, game, n, k, d_boards, d_who, d_count, max_count, d_probs, d_values,
+                                 impl == 7 ? 0 : impl == 8 ? 2 : 1, st);
   }
+  if (impl == 8)
+    return caro_fail(CARO_E_ARG, "impl 8 is the split-precision tower of 128 filters; a 64-filter network runs impl 2 for split precision");
   if (impl == 1) {
     if (game == CARO_GAME_CONNECT4) return launch_simt<C4Rules>(C4Rules(), net, d_boards, d_who, d_count, max_count, d_probs, d_values, st);
     return launch_simt<MnkRules>(MnkRules{n, k}, net, d_boards, d_who, d_count, max_count, d_probs, d_values, st);

@@ -68,7 +68,7 @@ struct caro_net {
   void* d_rt_scratch;       // CTA-pair form: head features + FC scratch of every CTA, kRtScratchSlots launches in flight
   unsigned rt_scratch_seq;  // next slot (round robin per launch)
   void* d_rx_weights;   // fp16 hi / lo UMMA B-operand blocks of the split-precision row-tiled tower -- see net_rx.cu
-  void* d_wide_weights; // 128-wide handles: fp16 then bf16 UMMA B-operand images of every (layer, tap) -- see net_wide.cu
+  void* d_wide_weights; // 128-wide handles: fp16, bf16 (hi) and bf16 lo UMMA B-operand images of every (layer, tap) -- see net_wide.cu
   alignas(16) float h_rt_consts[(caro::kMaxBlocks + 1) * 64 + 3 * 64 + 4 + 1536 + 4];  // host copy of the row-tiled tower's by-value constants (RtConsts)
   float* d_tc_bias;     // [1 + blocks][filters] folded conv biases
   float* d_pol_fc_t;    // policy FC transposed to [2*HW][A] (+ value FC1 [HW][20]) for coalesced reads in the TC epilogue
@@ -103,11 +103,12 @@ int caro_net_rt_forward(caro_net* net, int game, int n, int k, const void* d_boa
                         const int32_t* d_count, int64_t max_count, float* d_probs, float* d_values, int mode, cudaStream_t st);
 
 // net_wide.cu (tap-per-MMA tower of 128-filter networks, N = 128 per MMA, weights streamed tap by tap)
+// ops: 0 = fp16 operands, 1 = bf16 operands, 2 = bf16 hi + lo operands (3 MMAs per product)
 int caro_net_wide_pack(caro_net* net, const float* h_blob);
 int caro_net_wide_prepare();
 void caro_net_wide_free(caro_net* net);
 int caro_net_wide_forward(caro_net* net, int game, int n, int k, const void* d_boards, const uint8_t* d_who,
-                          const int32_t* d_count, int64_t max_count, float* d_probs, float* d_values, bool f16, cudaStream_t st);
+                          const int32_t* d_count, int64_t max_count, float* d_probs, float* d_values, int ops, cudaStream_t st);
 
 // net_rx.cu (split-precision row-tiled tower, fp16 hi + lo, boards up to 6 x 7)
 int caro_net_rx_pack(caro_net* net, const float* h_blob);

@@ -17,8 +17,11 @@
 //   * heads: the 1x1 head convolutions reduce over 128 channels in the last epilogue; boards with HW <= 64 run the FC
 //     heads and the softmax in the kernel (run_heads), larger boards export the activated head features for
 //     heads_tc_kernel (net_heads.cu), whose K = 3 HW does not depend on the width.
-// Operand format (fp16 or bf16) is a compile-time switch; the residual stream is fp32 in both.  Every sum has a fixed
-// order, so a leaf's outputs do not depend on the batch, the grid or d_count.
+// The operand mode is a compile-time switch (WideOps): fp16, bf16, or bf16 hi + lo pairs (lo = bf16(x - bf16(x))) with
+// every product evaluated as hi*hi + lo*hi + hi*lo, the arithmetic of net_tc.cu's SPLIT form, for trained networks whose
+// logits one 8-bit-mantissa pass cannot hold to 1e-3.  The split mode keeps a hi and a lo activation image (151,552 B)
+// and streams each tap's hi and lo weight images through a ring of two 32 KB slots.  The residual stream is fp32 in every
+// mode.  Every sum has a fixed order, so a leaf's outputs do not depend on the batch, the grid or d_count.
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
 #include <cuda_runtime.h>
@@ -50,7 +53,6 @@ constexpr int kTapBytes = (F / 8) * F * 16;           // 32,768: one tap of a 12
 constexpr int kTapBytesIn = 2 * F * 16;               // 4,096: one tap of conv_in (K padded to 16)
 constexpr int kLayerBytesIn = 9 * kTapBytesIn;
 constexpr int kLayerBytes = 9 * kTapBytes;
-constexpr int kSlots = 4;                             // weight ring: 4 taps in flight
 constexpr int kHeadfeatSlots = 8;                     // scratch slots for exported head features (launches in flight)
 constexpr int kHeadsInTowerMaxHW = 64;                // larger boards run their FC heads in heads_tc_kernel
 constexpr int kFcFloats = 512;                        // FC scratch: hidden[nb][20] + logits[nb][A]
@@ -62,17 +64,29 @@ constexpr int kMmaWarp = kEpiWarps;       // warp 8: TMEM owner, MMA issue
 constexpr int kLoadWarp = kEpiWarps + 1;  // warp 9: weight streaming
 constexpr int kThreads = kEpiThreads + 64;
 
-// dynamic shared memory carve-up (byte offsets)
-constexpr int kAct = 0;
-constexpr int kWgt = kAct + kActBytes;
-constexpr int kHeadW = kWgt + kSlots * kTapBytes;     // float [3][128] head conv weights + [3] biases
-constexpr int kHeadF = kHeadW + 400 * 4;              // float [rows][3] head features
-constexpr int kFc = kHeadF + kGroupRows * 3 * 4;
-constexpr int kCellTab = kFc + kFcFloats * 4;         // uint16 [rows]: (board << 9) | (cell + 1), 0 = padding
-constexpr int kBars = kCellTab + kGroupRows * 2;
-constexpr int kTotal = kBars + 128;
-static_assert(kTotal <= 232448, "exceeds the 227 KB shared memory of an sm_100 CTA");
-static_assert(kWgt % 128 == 0 && kBars % 8 == 0, "alignment");
+enum WideOps { kOpsF16 = 0, kOpsBf16 = 1, kOpsBf16x3 = 2 };
+
+// Per operand mode: the weight ring and the dynamic shared memory carve-up (byte offsets).
+template <int OPS>
+struct WideCfg {
+  static constexpr bool kF16 = OPS == kOpsF16;
+  static constexpr bool kSplit = OPS == kOpsBf16x3;
+  static constexpr int kParts = kSplit ? 2 : 1;  // images of the activations and of every weight tap: hi (+ lo)
+  // weight ring of 32 KB slots, one tap image each: one-pass 4 taps in flight, split 2 (on a B200, 2 x 32 KB slots ran the
+  // split tower 3-5 % faster than 4 x 16 KB half images: profiles/r4_wide_split_ring.jsonl)
+  static constexpr int kSlots = kSplit ? 2 : 4;
+  static constexpr int kAct = 0;
+  static constexpr int kWgt = kAct + kParts * kActBytes;
+  static constexpr int kHeadW = kWgt + kSlots * kTapBytes;         // float [3][128] head conv weights + [3] biases
+  static constexpr int kHeadF = kHeadW + 400 * 4;                  // float [rows][3] head features
+  static constexpr int kFc = kHeadF + kGroupRows * 3 * 4;
+  static constexpr int kCellTab = kFc + kFcFloats * 4;             // uint16 [rows]: (board << 9) | (cell + 1), 0 = padding
+  static constexpr int kBars = kCellTab + kGroupRows * 2;
+  static constexpr int kTotal = kBars + 128;
+  static_assert(kTotal <= 232448, "exceeds the 227 KB shared memory of an sm_100 CTA");
+  static_assert(kWgt % 128 == 0 && kBars % 8 == 0, "alignment");
+};
+static_assert(WideCfg<kOpsBf16x3>::kTotal == 224448, "split mode: 2 x 75,776 B activations + 2 x 32 KB ring + 7,360 B");
 
 template <bool F16>
 __device__ __forceinline__ uint32_t pack2(float a, float b) {
@@ -84,29 +98,40 @@ __device__ __forceinline__ uint32_t pack2(float a, float b) {
   return *reinterpret_cast<const uint32_t*>(&h);
 }
 
+// The lo halves of a bf16 hi pair (a in the low 16 bits): bf16(a - hi(a)), bf16(b - hi(b)); the differences are exact.
+__device__ __forceinline__ uint32_t pack2_lo(uint32_t hi, float a, float b) {
+  return pack2<false>(a - __uint_as_float(hi << 16), b - __uint_as_float(hi & 0xffff0000u));
+}
+
 // Roles: warps 0-7 = epilogue (warp w: TMEM lanes [32(w&3), +32) = rows of both tiles, channels 64(w>>2)..+64, read in
 //        32-column chunks), warp 8 = TMEM allocation + elected-lane MMA issue, warp 9 = elected-lane weight streaming.
 // Barriers: full[s] / empty[s] = weight slot s landed / read by its MMAs; acc = every MMA of a layer complete;
 //           act = the layer's input rows written and the accumulators drained (kEpiThreads arrivals).
+// Weight stream: per tap its image (one-pass) or its hi, then its lo image (split), one ring slot each.  Per image and
+// tile the MMAs run K-step by K-step: the hi image issues a_hi*w_hi then a_lo*w_hi, the lo image a_hi*w_lo (conv_in: its
+// 0/1 input planes have no lo part, so only a_hi*w_hi and a_hi*w_lo).
 // Timeline (caro_net_set_trace, CTA 0, slot = kind * 1000 + global layer): 0 = layer input ready (MMA warp), 1 = last
 // commit of the layer issued, 2 = accumulators complete (epilogue warp 0), 3 = epilogue done, 4 = cycles the MMA warp
 // waited for weight slots during the layer (a count, not a clock).
-template <class R, bool F16>
+template <class R, int OPS>
 __global__ void __launch_bounds__(kThreads, 1)
 net_wide_kernel(R rules, TcGeom gm, const typename R::Board* __restrict__ boards, const uint8_t* __restrict__ who,
-                const int32_t* __restrict__ d_count, long long max_count, const uint8_t* __restrict__ wimg,
+                const int32_t* __restrict__ d_count, long long max_count, const uint8_t* __restrict__ wimg, size_t wimg_lo_off,
                 const float* __restrict__ bias_g, const float* __restrict__ blob, BlobLayout L,
                 const float* __restrict__ pol_fc_t, const float* __restrict__ val_fc1_t, float* __restrict__ probs,
                 float* __restrict__ values, uint8_t* __restrict__ headfeat_out, size_t headfeat_lo_off, int headfeat_kc8,
                 long long* __restrict__ trace) {
+  using K = WideCfg<OPS>;
+  constexpr bool F16 = K::kF16;
+  constexpr int kSlots = K::kSlots;
   extern __shared__ __align__(128) uint8_t smem[];
-  uint8_t* act = smem + kAct;
-  uint8_t* wgt = smem + kWgt;
-  float* headw_s = reinterpret_cast<float*>(smem + kHeadW);
-  float* headf_s = reinterpret_cast<float*>(smem + kHeadF);
-  float* fc_s = reinterpret_cast<float*>(smem + kFc);
-  uint16_t* cell_tab = reinterpret_cast<uint16_t*>(smem + kCellTab);
-  uint64_t* bar_full = reinterpret_cast<uint64_t*>(smem + kBars);
+  uint8_t* act = smem + K::kAct;
+  uint8_t* wgt = smem + K::kWgt;
+  float* headw_s = reinterpret_cast<float*>(smem + K::kHeadW);
+  float* headf_s = reinterpret_cast<float*>(smem + K::kHeadF);
+  float* fc_s = reinterpret_cast<float*>(smem + K::kFc);
+  uint16_t* cell_tab = reinterpret_cast<uint16_t*>(smem + K::kCellTab);
+  uint64_t* bar_full = reinterpret_cast<uint64_t*>(smem + K::kBars);
   uint64_t* bar_empty = bar_full + kSlots;
   uint64_t* bar_acc = bar_empty + kSlots;
   uint64_t* bar_act = bar_acc + 1;
@@ -123,7 +148,7 @@ net_wide_kernel(R rules, TcGeom gm, const typename R::Board* __restrict__ boards
   const int n_layers = 1 + L.blocks;
 
   // ---- one-time setup ---------------------------------------------------------------------
-  for (int i = tid; i < kActBytes / 16; i += kThreads) reinterpret_cast<uint4*>(act)[i] = make_uint4(0, 0, 0, 0);
+  for (int i = tid; i < K::kParts * kActBytes / 16; i += kThreads) reinterpret_cast<uint4*>(act)[i] = make_uint4(0, 0, 0, 0);
   for (int p = tid; p < kGroupRows; p += kThreads) {
     const int b = p / gm.block, within = p - b * gm.block;
     const int r = within / gm.pitch, c = within - r * gm.pitch;
@@ -161,28 +186,31 @@ net_wide_kernel(R rules, TcGeom gm, const typename R::Board* __restrict__ boards
   const int total_layers = my_groups * n_layers;
 
   if (warp == kLoadWarp) {
-    // ===================== weight producer: taps in issue order, kSlots ahead of the MMAs ==========================
+    // ===================== weight producer: tap images in issue order, kSlots ahead of the MMAs =====================
     if ((tid & 31) == 0) {
       int g = 0;
       for (int gl = 0; gl < total_layers; ++gl) {
         const int l = gl % n_layers;
         const int tap_bytes = l == 0 ? kTapBytesIn : kTapBytes;
         const uint8_t* src = l == 0 ? wimg : wimg + kLayerBytesIn + (size_t)(l - 1) * kLayerBytes;
-        for (int tap = 0; tap < 9; ++tap, ++g) {
-          const int s = g % kSlots;
-          if (g >= kSlots) mbar_wait(bar_empty + s, (uint32_t)(g / kSlots - 1) & 1u);
-          mbar_expect_tx(bar_full + s, (uint32_t)tap_bytes);
-          bulk_g2s(wgt + s * kTapBytes, src + (size_t)tap * tap_bytes, (uint32_t)tap_bytes, bar_full + s);
+        for (int tap = 0; tap < 9; ++tap) {
+          for (int part = 0; part < K::kParts; ++part, ++g) {
+            const int s = g % kSlots;
+            if (g >= kSlots) mbar_wait(bar_empty + s, (uint32_t)(g / kSlots - 1) & 1u);
+            mbar_expect_tx(bar_full + s, (uint32_t)tap_bytes);
+            bulk_g2s(wgt + s * kTapBytes, src + part * wimg_lo_off + (size_t)tap * tap_bytes, (uint32_t)tap_bytes, bar_full + s);
+          }
         }
       }
     }
     __syncwarp();
   } else if (warp == kMmaWarp) {
-    // ===================== MMA issue: tap-major, both tiles per tap ================================================
+    // ===================== MMA issue: tap-major, both tiles per tap image ==========================================
     uint32_t elected;
     asm volatile("{\n\t.reg .pred P;\n\telect.sync _|P, 0xffffffff;\n\tselp.u32 %0, 1, 0, P;\n\t}" : "=r"(elected));
     const uint64_t a_desc0 = make_desc(smem_u32(act) + (uint32_t)kHalo * 16u, kChunkBytes, 128u);
     const uint64_t b_desc0 = make_desc(smem_u32(wgt), (uint32_t)F * 16u, 128u);
+    constexpr uint64_t kALo = (uint64_t)(kActBytes / 16);  // lo activation image
     constexpr uint32_t idesc = rt_idesc_fmt<F16>((uint32_t)F);
     const int pitch = gm.pitch;
     int g = 0;
@@ -193,35 +221,47 @@ net_wide_kernel(R rules, TcGeom gm, const typename R::Board* __restrict__ boards
       if (elected) TC_TRACE(0, gl);
       long long wait_cycles = 0;
 #pragma unroll 1
-      for (int tap = 0; tap < 9; ++tap, ++g) {
-        const int s = g % kSlots;
-        if (trace != nullptr) {
-          const long long t0 = clock64();
-          mbar_wait(bar_full + s, (uint32_t)(g / kSlots) & 1u);
-          wait_cycles += clock64() - t0;
-        } else {
-          mbar_wait(bar_full + s, (uint32_t)(g / kSlots) & 1u);
-        }
-        tc_fence_after();
+      for (int tap = 0; tap < 9; ++tap) {
         const int sh = (tap / 3 - 1) * pitch + (tap % 3 - 1);
-        const uint64_t bd = b_desc0 + (uint64_t)(uint32_t)(s * (kTapBytes / 16));
-        if (elected) {
-#pragma unroll
-          for (int t = 0; t < kTiles; ++t) {
-            const uint32_t d = tmem_base + (uint32_t)(t * F);
-            const uint64_t ad = a_desc0 + (uint64_t)(int64_t)(t * kTileRows + sh);
-            if (first) {  // conv_in: K = 2 input planes padded to 16
-              umma_bf16(d, ad, bd, idesc, tap > 0 ? 1u : 0u);
-            } else {
-#pragma unroll
-              for (int kk = 0; kk < F / 16; ++kk)
-                umma_bf16(d, ad + (uint64_t)(kk * 2 * kActRows), bd + (uint64_t)(kk * 2 * F), idesc, (tap | kk) ? 1u : 0u);
-            }
+#pragma unroll 1
+        for (int part = 0; part < K::kParts; ++part, ++g) {
+          const int s = g % kSlots;
+          if (trace != nullptr) {
+            const long long t0 = clock64();
+            mbar_wait(bar_full + s, (uint32_t)(g / kSlots) & 1u);
+            wait_cycles += clock64() - t0;
+          } else {
+            mbar_wait(bar_full + s, (uint32_t)(g / kSlots) & 1u);
           }
-          umma_commit(bar_empty + s);  // the slot is free once these MMAs have read it
-          if (tap == 8) umma_commit(bar_acc);
+          tc_fence_after();
+          const bool w_lo = part == 1;
+          const uint64_t bd = b_desc0 + (uint64_t)(uint32_t)(s * (kTapBytes / 16));
+          if (elected) {
+#pragma unroll
+            for (int t = 0; t < kTiles; ++t) {
+              const uint32_t d = tmem_base + (uint32_t)(t * F);
+              const uint64_t ad = a_desc0 + (uint64_t)(int64_t)(t * kTileRows + sh);
+              if (first) {  // conv_in: K = 2 input planes padded to 16 (split: a_hi * w_hi, then a_hi * w_lo)
+                umma_bf16(d, ad, bd, idesc, (tap > 0 || w_lo) ? 1u : 0u);
+              } else {
+#pragma unroll
+                for (int kk = 0; kk < F / 16; ++kk) {
+                  const uint64_t a = ad + (uint64_t)(kk * 2 * kActRows);
+                  const uint64_t b = bd + (uint64_t)(kk * 2 * F);
+                  if (w_lo) {
+                    umma_bf16(d, a, b, idesc, 1u);  // hi(a) * lo(w)
+                  } else {
+                    umma_bf16(d, a, b, idesc, (tap | kk) ? 1u : 0u);
+                    if (K::kSplit) umma_bf16(d, a + kALo, b, idesc, 1u);  // lo(a) * hi(w)
+                  }
+                }
+              }
+            }
+            umma_commit(bar_empty + s);  // the slot is free once these MMAs have read it
+            if (tap == 8 && part == K::kParts - 1) umma_commit(bar_acc);
+          }
+          __syncwarp();
         }
-        __syncwarp();
       }
       if (elected) {
         TC_TRACE(1, gl);
@@ -312,12 +352,16 @@ net_wide_kernel(R rules, TcGeom gm, const typename R::Board* __restrict__ boards
               TMEM_ST16(a_res + 16u, (rr + 16));
 #pragma unroll
               for (int c8 = 0; c8 < 4; ++c8) {
-                uint32_t packed[4];
+                uint32_t packed[4], packed_lo[4];
 #pragma unroll
-                for (int j = 0; j < 4; ++j)
-                  packed[j] = real ? pack2<F16>(__uint_as_float(rr[c8 * 8 + 2 * j]), __uint_as_float(rr[c8 * 8 + 2 * j + 1])) : 0u;
+                for (int j = 0; j < 4; ++j) {
+                  const float v0 = __uint_as_float(rr[c8 * 8 + 2 * j]), v1 = __uint_as_float(rr[c8 * 8 + 2 * j + 1]);
+                  packed[j] = real ? pack2<F16>(v0, v1) : 0u;
+                  if (K::kSplit) packed_lo[j] = real ? pack2_lo(packed[j], v0, v1) : 0u;
+                }
                 uint8_t* dst = act + (size_t)((ch0 / 8 + c8) * kActRows + kHalo + p) * 16;
                 *reinterpret_cast<uint4*>(dst) = make_uint4(packed[0], packed[1], packed[2], packed[3]);
+                if (K::kSplit) *reinterpret_cast<uint4*>(dst + kActBytes) = make_uint4(packed_lo[0], packed_lo[1], packed_lo[2], packed_lo[3]);
               }
             } else {  // 1x1 head convolutions over this chunk's 32 channels, in channel order
               const float4* hw4 = reinterpret_cast<const float4*>(headw_s + ch0);
@@ -366,7 +410,7 @@ net_wide_kernel(R rules, TcGeom gm, const typename R::Board* __restrict__ boards
   }
 }
 
-template <class R, bool F16>
+template <class R, int OPS>
 static int launch_wide(const R& rules, caro_net* net, const void* boards, const uint8_t* who, const int32_t* d_count,
                        int64_t max_count, float* probs, float* values, cudaStream_t st) {
   TcGeom gm;
@@ -393,11 +437,11 @@ static int launch_wide(const R& rules, caro_net* net, const void* boards, const 
   if (net->d_headfeat != nullptr && max_count <= net->headfeat_leaves)
     headfeat = (uint8_t*)net->d_headfeat + (size_t)(net->headfeat_seq++ % kHeadfeatSlots) * 2 * image;
   const size_t img_bytes = (size_t)kLayerBytesIn + (size_t)net->layout.blocks * kLayerBytes;
-  const uint8_t* wimg = (const uint8_t*)net->d_wide_weights + (F16 ? 0 : img_bytes);
-  net_wide_kernel<R, F16><<<grid, kThreads, kTotal, st>>>(rules, gm, (const typename R::Board*)boards, who, d_count, (long long)max_count,
-                                                          wimg, net->d_tc_bias, net->d_blob, net->layout, net->d_pol_fc_t,
-                                                          net->d_pol_fc_t + (size_t)2 * HW * net->A, probs, values, headfeat, image,
-                                                          kc64 * 8, (long long*)net->d_trace);
+  const uint8_t* wimg = (const uint8_t*)net->d_wide_weights + (OPS == kOpsF16 ? 0 : img_bytes);  // bf16 (hi), then lo
+  net_wide_kernel<R, OPS><<<grid, kThreads, WideCfg<OPS>::kTotal, st>>>(
+      rules, gm, (const typename R::Board*)boards, who, d_count, (long long)max_count, wimg, img_bytes, net->d_tc_bias, net->d_blob,
+      net->layout, net->d_pol_fc_t, net->d_pol_fc_t + (size_t)2 * HW * net->A, probs, values, headfeat, image, kc64 * 8,
+      (long long*)net->d_trace);
   int rc = caro_check_launch("net_wide_kernel");
   if (rc == CARO_OK && headfeat != nullptr) rc = caro_net_heads_forward(net, headfeat, image, d_count, max_count, probs, values, st);
   return rc;
@@ -409,21 +453,25 @@ static int launch_wide(const R& rules, caro_net* net, const void* boards, const 
 using namespace caro;
 using namespace caro::wide;
 
-// Weight images: fp16 first, then bf16; each is conv_in (9 taps of kTapBytesIn) followed by 9 taps of kTapBytes per residual
-// block, every tap in the UMMA B-operand layout [8-channel chunk of ci][co = 0..127][ci % 8] (no-swizzle K-major).
+// Weight images: fp16, bf16 (= the hi image of the split mode), then the split mode's lo image bf16(w - bf16(w)); each is
+// conv_in (9 taps of kTapBytesIn) followed by 9 taps of kTapBytes per residual block, every tap in the UMMA B-operand
+// layout [8-channel chunk of ci][co = 0..127][ci % 8] (no-swizzle K-major).
 // Also the conv biases [1 + blocks][128], the transposed FC weights of the in-kernel heads and, for boards with
 // HW > 64, the head-feature slots + B image of heads_tc_kernel -- the same buffers the 64-wide towers use.
 int caro_net_wide_pack(caro_net* net, const float* h) {
   const BlobLayout& L = net->layout;
   const int blocks = L.blocks;
   const size_t img_bytes = (size_t)kLayerBytesIn + (size_t)blocks * kLayerBytes;
-  std::vector<uint16_t> img(img_bytes, 0);  // two images of img_bytes / 2 halves each
+  std::vector<uint16_t> img(3 * img_bytes / 2, 0);  // three images of img_bytes / 2 halves each
   auto put = [&](size_t tap_base, int co, int ci, float w) {
     const size_t off = (tap_base + (size_t)((ci / 8) * F + co) * 16) / 2 + (ci % 8);
     const __half_raw hr = __float2half_rn(w);
-    const __nv_bfloat16_raw br = __float2bfloat16_rn(w);
+    const __nv_bfloat16 hi = __float2bfloat16_rn(w);
+    const __nv_bfloat16_raw br = hi;
+    const __nv_bfloat16_raw lr = __float2bfloat16_rn(w - __bfloat162float(hi));
     img[off] = hr.x;
     img[img_bytes / 2 + off] = br.x;
+    img[img_bytes + off] = lr.x;
   };
   for (int tap = 0; tap < 9; ++tap)
     for (int co = 0; co < F; ++co)
@@ -455,10 +503,10 @@ int caro_net_wide_pack(caro_net* net, const float* h) {
     const int hrc = caro_net_heads_pack(net, h);
     if (hrc != CARO_OK) return hrc;
   }
-  if (!net->d_wide_weights) ce = cudaMalloc(&net->d_wide_weights, 2 * img_bytes);
+  if (!net->d_wide_weights) ce = cudaMalloc(&net->d_wide_weights, 3 * img_bytes);
   if (ce == cudaSuccess && !net->d_tc_bias) ce = cudaMalloc(&net->d_tc_bias, bias.size() * sizeof(float));
   if (ce == cudaSuccess && !net->d_pol_fc_t) ce = cudaMalloc(&net->d_pol_fc_t, polt.size() * sizeof(float));
-  if (ce == cudaSuccess) ce = cudaMemcpy(net->d_wide_weights, img.data(), 2 * img_bytes, cudaMemcpyHostToDevice);
+  if (ce == cudaSuccess) ce = cudaMemcpy(net->d_wide_weights, img.data(), 3 * img_bytes, cudaMemcpyHostToDevice);
   if (ce == cudaSuccess) ce = cudaMemcpy(net->d_tc_bias, bias.data(), bias.size() * sizeof(float), cudaMemcpyHostToDevice);
   if (ce == cudaSuccess) ce = cudaMemcpy(net->d_pol_fc_t, polt.data(), polt.size() * sizeof(float), cudaMemcpyHostToDevice);
   if (ce != cudaSuccess) return caro_fail(CARO_E_CUDA, cudaGetErrorString(ce));
@@ -473,21 +521,31 @@ void caro_net_wide_free(caro_net* net) {
 
 // Sets the dynamic shared memory attribute of every instantiation up front (caro_net_create), so that no attribute call
 // can fall inside a CUDA-graph capture of the search loop.
+template <class R>
+static cudaError_t prepare_ops() {
+  cudaError_t ce = cudaFuncSetAttribute(net_wide_kernel<R, kOpsF16>, cudaFuncAttributeMaxDynamicSharedMemorySize, WideCfg<kOpsF16>::kTotal);
+  if (ce == cudaSuccess) ce = cudaFuncSetAttribute(net_wide_kernel<R, kOpsBf16>, cudaFuncAttributeMaxDynamicSharedMemorySize, WideCfg<kOpsBf16>::kTotal);
+  if (ce == cudaSuccess) ce = cudaFuncSetAttribute(net_wide_kernel<R, kOpsBf16x3>, cudaFuncAttributeMaxDynamicSharedMemorySize, WideCfg<kOpsBf16x3>::kTotal);
+  return ce;
+}
+
 int caro_net_wide_prepare() {
-  cudaError_t ce = cudaFuncSetAttribute(net_wide_kernel<C4Rules, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kTotal);
-  if (ce == cudaSuccess) ce = cudaFuncSetAttribute(net_wide_kernel<C4Rules, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kTotal);
-  if (ce == cudaSuccess) ce = cudaFuncSetAttribute(net_wide_kernel<MnkRules, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kTotal);
-  if (ce == cudaSuccess) ce = cudaFuncSetAttribute(net_wide_kernel<MnkRules, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kTotal);
+  cudaError_t ce = prepare_ops<C4Rules>();
+  if (ce == cudaSuccess) ce = prepare_ops<MnkRules>();
   if (ce != cudaSuccess) return caro_fail(CARO_E_CUDA, cudaGetErrorString(ce));
   return CARO_OK;
 }
 
+template <class R>
+static int forward_ops(const R& rules, caro_net* net, const void* d_boards, const uint8_t* d_who, const int32_t* d_count, int64_t max_count,
+                       float* d_probs, float* d_values, int ops, cudaStream_t st) {
+  if (ops == kOpsF16) return launch_wide<R, kOpsF16>(rules, net, d_boards, d_who, d_count, max_count, d_probs, d_values, st);
+  if (ops == kOpsBf16x3) return launch_wide<R, kOpsBf16x3>(rules, net, d_boards, d_who, d_count, max_count, d_probs, d_values, st);
+  return launch_wide<R, kOpsBf16>(rules, net, d_boards, d_who, d_count, max_count, d_probs, d_values, st);
+}
+
 int caro_net_wide_forward(caro_net* net, int game, int n, int k, const void* d_boards, const uint8_t* d_who,
-                          const int32_t* d_count, int64_t max_count, float* d_probs, float* d_values, bool f16, cudaStream_t st) {
-  if (game == CARO_GAME_CONNECT4) {
-    if (f16) return launch_wide<C4Rules, true>(C4Rules(), net, d_boards, d_who, d_count, max_count, d_probs, d_values, st);
-    return launch_wide<C4Rules, false>(C4Rules(), net, d_boards, d_who, d_count, max_count, d_probs, d_values, st);
-  }
-  if (f16) return launch_wide<MnkRules, true>(MnkRules{n, k}, net, d_boards, d_who, d_count, max_count, d_probs, d_values, st);
-  return launch_wide<MnkRules, false>(MnkRules{n, k}, net, d_boards, d_who, d_count, max_count, d_probs, d_values, st);
+                          const int32_t* d_count, int64_t max_count, float* d_probs, float* d_values, int ops, cudaStream_t st) {
+  if (game == CARO_GAME_CONNECT4) return forward_ops(C4Rules(), net, d_boards, d_who, d_count, max_count, d_probs, d_values, ops, st);
+  return forward_ops(MnkRules{n, k}, net, d_boards, d_who, d_count, max_count, d_probs, d_values, ops, st);
 }

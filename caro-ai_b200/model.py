@@ -127,7 +127,7 @@ def fold_state_dict(sd: Dict[str, torch.Tensor], rows: int, cols: int, actions: 
     return np.ascontiguousarray(blob)
 
 
-IMPL_TCGEN05, IMPL_SIMT, IMPL_TCGEN05_X3, IMPL_TCGEN05_F16 = 0, 1, 2, 7
+IMPL_TCGEN05, IMPL_SIMT, IMPL_TCGEN05_X3, IMPL_TCGEN05_F16, IMPL_WIDE_X3 = 0, 1, 2, 7, 8
 PRIOR_TOLERANCE = 1e-3      # BASELINE.json north_star: priors / values within 1e-3 of the fp32 reference
 CALIBRATION_MARGIN = 0.8    # the probe set is a sample: switch to the split mode at 0.8 x the tolerance
 _PROBE_BOARDS: Dict[tuple, tuple] = {}
@@ -183,16 +183,23 @@ class DeviceNet:
         "bf16"   one bf16 tensor-core pass, fp32 accumulate (forced; the caller vouches for the tolerance),
         "bf16x3" hi/lo split of activations and weights, three MMAs per product: fp32-class accuracy (boards up to 6 x 7:
                  fp16 hi + lo, row-tiled; larger boards: bf16 hi + lo, tap-per-MMA),
+        "bf16x3-wide" the split-precision form of the wide tower (128 filters only): bf16 hi + lo activations and weights,
+                 three MMAs per product, fp32 residual stream,
         "fp32-simt" the SIMT numerics-reference kernel.
-        128-filter networks (``Net(filters=128)``) run the wide tensor-core tower (csrc/net_wide.cu) with fp16 or bf16
-        operands on every board size, or the SIMT tower; "auto" tries "fp16", then "bf16", then falls back to "fp32-simt",
-        and "bf16x3" is not available."""
+        128-filter networks (``Net(filters=128)``) run the wide tensor-core tower (csrc/net_wide.cu) with fp16, bf16 or bf16
+        hi + lo operands on every board size, or the SIMT tower; "auto" tries "fp16", then "bf16", then "bf16x3-wide", and
+        falls back to "fp32-simt" only when all three miss the check.  "bf16x3" (the 64-filter split towers) is not
+        available for them."""
         _cabi.require_cuda()
-        assert precision in ("auto", "fp16", "bf16", "bf16x3", "fp32-simt")
+        assert precision in ("auto", "fp16", "bf16", "bf16x3", "bf16x3-wide", "fp32-simt")
         sd = net_or_state_dict.state_dict() if isinstance(net_or_state_dict, nn.Module) else net_or_state_dict
         self.blocks, self.filters = state_dict_shape(sd)
         if precision == "bf16x3" and self.filters != NUM_FILTERS:
-            raise ValueError("precision 'bf16x3' is not available for %d-filter networks (64 only)" % self.filters)
+            raise ValueError("precision 'bf16x3' is not available for %d-filter networks (64 only); their split-precision "
+                             "tower is 'bf16x3-wide'" % self.filters)
+        if precision == "bf16x3-wide" and self.filters != WIDTHS[1]:
+            raise ValueError("precision 'bf16x3-wide' is the split tower of 128-filter networks, not of %d-filter ones "
+                             "(use 'bf16x3')" % self.filters)
         self.requested = precision
         _, self.rows, self.cols = game.obs_shape
         self.actions = game.action_space
@@ -213,12 +220,16 @@ class DeviceNet:
         if precision == "auto":
             precision = self.calibrate()
         self.precision = precision
-        self.impl = {"fp16": IMPL_TCGEN05_F16, "bf16": IMPL_TCGEN05, "bf16x3": IMPL_TCGEN05_X3, "fp32-simt": IMPL_SIMT}[precision]
+        self.impl = {"fp16": IMPL_TCGEN05_F16, "bf16": IMPL_TCGEN05, "bf16x3": IMPL_TCGEN05_X3, "bf16x3-wide": IMPL_WIDE_X3,
+                     "fp32-simt": IMPL_SIMT}[precision]
 
     def calibrate(self, d_boards=None, d_who=None) -> str:
-        """Max |prior| / |value| deviation of the one-pass bf16 tower from the fp32 SIMT tower on probe positions
-        (``d_boards`` / ``d_who``: caller-supplied device boards, e.g. replay positions; default: cached random play-outs).
-        Returns the precision that keeps the 1e-3 contract and records the measurement in ``self.calibration``."""
+        """Max |prior| / |value| deviation of the one-pass towers (fp16 where it applies, then bf16) from the fp32 SIMT
+        tower on probe positions (``d_boards`` / ``d_who``: caller-supplied device boards, e.g. replay positions; default:
+        cached random play-outs).  If neither keeps the margin, the split-precision tower of the width ("bf16x3" at 64
+        filters, "bf16x3-wide" at 128) is measured too (``split_max_abs_*``) and selected if it keeps it; "fp32-simt" is
+        the last resort.  Returns the precision that keeps the 1e-3 contract and records the measurement in
+        ``self.calibration``."""
         if d_boards is None:
             d_boards, d_who = probe_positions(self.game)
         n = int(d_who.numel())
@@ -226,7 +237,7 @@ class DeviceNet:
         limit = CALIBRATION_MARGIN * PRIOR_TOLERANCE
         ok = False
         self.calibration = {"positions": n, "filters": self.filters}
-        if self.filters != NUM_FILTERS:  # the wide tower: fp16 on every board, then bf16, then the SIMT tower (no split mode)
+        if self.filters != NUM_FILTERS:  # the wide tower: fp16 on every board, then bf16, then its split mode
             candidates = [("fp16", IMPL_TCGEN05_F16)]
         else:
             candidates = [("fp16", IMPL_TCGEN05_F16)] if self.rows <= 6 and self.cols <= 7 else []  # the row-tiled towers' boards
@@ -243,15 +254,15 @@ class DeviceNet:
                 self.calibration["selected"] = name
         if ok:
             return self.calibration["selected"]
-        if self.filters != NUM_FILTERS:  # no split mode for the wide tower
+        # the split mode is checked too (the 64-filter row-tiled one is fp16 hi + lo, of a finite range): the SIMT tower is
+        # the last resort
+        split, split_impl = ("bf16x3", IMPL_TCGEN05_X3) if self.filters == NUM_FILTERS else ("bf16x3-wide", IMPL_WIDE_X3)
+        self.calibration["selected"] = split
+        px, vx = self.forward_boards(d_boards, d_who, n, split_impl)
+        dpx, dvx = float((px - p32).abs().max().item()), float((vx - v32).abs().max().item())
+        self.calibration.update(split_max_abs_prior_diff=dpx, split_max_abs_value_diff=dvx)
+        if not (dpx <= limit and dvx <= limit):
             self.calibration["selected"] = "fp32-simt"
-        else:  # the split mode is checked too (fp16 hi + lo has a finite range): the SIMT tower is the last resort
-            self.calibration["selected"] = "bf16x3"
-            px, vx = self.forward_boards(d_boards, d_who, n, IMPL_TCGEN05_X3)
-            dpx, dvx = float((px - p32).abs().max().item()), float((vx - v32).abs().max().item())
-            self.calibration.update(split_max_abs_prior_diff=dpx, split_max_abs_value_diff=dvx)
-            if not (dpx <= CALIBRATION_MARGIN * PRIOR_TOLERANCE and dvx <= CALIBRATION_MARGIN * PRIOR_TOLERANCE):
-                self.calibration["selected"] = "fp32-simt"
         return self.calibration["selected"]
 
     def update(self, net_or_state_dict):

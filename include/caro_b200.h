@@ -101,7 +101,8 @@ int caro_net_create(int rows, int cols, int actions, const float* h_blob, size_t
                     caro_net** out);
 /* caro_net_create for a stated shape (`blocks` 1..20, `filters` 64 or 128).  Every argument, the blob's size included, is
  * checked before the device is looked for: a bad shape returns CARO_E_ARG on any machine.  A 128-filter handle runs
- * impl 7 (wide tower, fp16 operands), 0 / 3 (wide tower, bf16 operands) and 1 (SIMT); see caro_net_forward. */
+ * impl 7 (wide tower, fp16 operands), 0 / 3 (wide tower, bf16 operands), 8 (wide tower, bf16 hi + lo split precision)
+ * and 1 (SIMT); see caro_net_forward. */
 int caro_net_create_shape(int rows, int cols, int actions, int blocks, int filters, const float* h_blob, size_t n_floats,
                           caro_net** out);
 int caro_net_update(caro_net* net, const float* h_blob, size_t n_floats);
@@ -142,8 +143,10 @@ int caro_net_set_grid_limit(caro_net* net, int ctas);
  *                 Caro self-play step; CARO_TC_PAIR=1 makes impl 0 / 3 use it),
  *             1 = fp32 SIMT tower (numerics reference kernel used by the tests).
  *           128-filter handles (caro_net_create_shape): 7 = the wide tap-per-MMA tower (net_wide.cu: M = 128, N = 128, K = 16
- *           MMAs, weights streamed tap by tap) with fp16 operands, 0 and 3 = the same tower with bf16 operands, 1 = the SIMT
- *           tower; 2, 4, 5 and 6 return CARO_E_ARG. */
+ *           MMAs, weights streamed tap by tap) with fp16 operands, 0 and 3 = the same tower with bf16 operands, 8 = the same
+ *           tower in split precision (bf16 hi + lo activations and weights, hi*hi + lo*hi + hi*lo per product, fp32
+ *           residual stream: fp32-class accuracy for trained wide networks), 1 = the SIMT tower; 2, 4, 5 and 6 return
+ *           CARO_E_ARG.  Impl 8 runs on 128-filter handles only: a 64-filter handle returns CARO_E_ARG (its split tower is 2). */
 int caro_net_forward(caro_net* net, int game, int n, int k, const void* d_boards,
                      const uint8_t* d_who, const int32_t* d_count, int64_t max_count,
                      float* d_probs, float* d_values, int impl, void* stream);

@@ -3,13 +3,18 @@
     python tools/wide_bench.py [--seconds S] [--out FILE]
 
 1. Stand-alone tower time (CUDA events, after warm-up): 5x128 Connect4 at 9,472 and 33,152 leaves, 10x128 Caro 15x15 at
-   4,096 and 16,384 leaves; the wide tower with fp16 (impl 7) and bf16 (impl 0) operands and, on the same boards, the
-   64-wide tap-per-MMA tower (impl 3, a 64-filter net of the same depth), alternated in rounds.  Useful TFLOP/s =
-   leaves x FLOP per leaf / time, with FLOP per leaf from the formula below.
+   4,096 and 16,384 leaves; the wide tower with fp16 (impl 7), bf16 (impl 0) and bf16 hi + lo (impl 8, split precision)
+   operands and, on the same boards, the 64-wide tap-per-MMA tower (impl 3, a 64-filter net of the same depth),
+   alternated in rounds; the SIMT tower (impl 1, the fallback of precision "auto") at the smaller size of each board.
+   Useful TFLOP/s = leaves x FLOP per leaf / time, with FLOP per leaf from the formula below (the split tower's three
+   products per multiply-add are not counted as useful).
 2. The phases of one layer (clock64 timeline of CTA 0): MMA phase, weight waits, epilogue, hand-off, against the tensor
-   floor, for 10x128 Caro at 16,384 leaves and 5x128 Connect4 at 33,152 leaves.
-3. Self-play leaf evaluations/s with precision "auto": Caro 15,15,5 at search_batch(200, 8), 2 parts x 1,024 games,
-   10x128 net, compact tree; Connect4 at search_batch(100, 8), 2 x 8,192 games, 5x128 net.
+   floor, for 10x128 Caro at 16,384 leaves and 5x128 Connect4 at 33,152 leaves, for impls 7, 0 and 8.
+3. Self-play leaf evaluations/s: Caro 15,15,5 at search_batch(200, 8), 2 parts x 1,024 games, 10x128 net, compact tree;
+   Connect4 at search_batch(100, 8), 2 x 8,192 games, 5x128 net -- both random-init, precision "auto".  Then the
+   "trained-like" 10x128 Caro net of tests/wide_split_net.py (policy FC x 100, residual stream x 2^17), which "auto" sends
+   to the split tower: at the configuration above, and at a small one (2 x 256 games, search_batch(10, 8)) both on the
+   split tower and on the SIMT tower, whose self-play rate the small configuration makes measurable.
 The card's name, power limit and SM clock under load are read with a read-only nvidia-smi query in the same run.
 """
 import argparse
@@ -100,21 +105,24 @@ def tower_bench(torch, seconds, out):
         torch.manual_seed(0)
         narrow = DeviceNet(Net(game.obs_shape, a, blocks=blocks).eval(), game, precision="fp32-simt")
         base_b, base_w = probe_positions(game, 1024)
-        towers = [("wide_fp16", wide, 7, 128), ("wide_bf16", wide, 0, 128), ("tap_per_mma_64", narrow, 3, 64)]
         for leaves in sizes:
+            towers = [("wide_fp16", wide, 7, 128), ("wide_bf16", wide, 0, 128), ("wide_bf16x3", wide, 8, 128),
+                      ("tap_per_mma_64", narrow, 3, 64)]
+            if leaves == sizes[0]:  # the SIMT tower at one size per board: a launch takes up to about a second
+                towers.append(("simt_128", wide, 1, 128))
             idx = torch.arange(leaves, device="cuda") % base_b.shape[0]
             d_boards, d_who = base_b[idx].contiguous(), base_w[idx].contiguous()
             times = {name: [] for name, *_ in towers}
             iters = {}
             for name, dn, impl, _ in towers:  # warm-up and sizing: each timed window lasts about `seconds`
-                for _ in range(3):
+                for _ in range(2):
                     dn.forward_boards(d_boards, d_who, leaves, impl)
                 torch.cuda.synchronize()
                 t0 = time.time()
-                for _ in range(5):
+                for _ in range(3):
                     dn.forward_boards(d_boards, d_who, leaves, impl)
                 torch.cuda.synchronize()
-                iters[name] = max(10, int(seconds / max(1e-6, (time.time() - t0) / 5)))
+                iters[name] = max(10 if impl != 1 else 2, int(seconds / max(1e-6, (time.time() - t0) / 3)))
             for _ in range(2):  # rounds, the towers alternate
                 for name, dn, impl, _ in towers:
                     s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -139,12 +147,12 @@ def timeline_bench(torch, out):
     """Splits one layer of the wide tower into its phases with the kernel's clock64 timeline (CTA 0, caro_net_set_trace):
     MMA phase (layer input ready -> every MMA complete; of it, the cycles the MMA warp waited for weight slots), epilogue
     (accumulators complete -> epilogue done) and hand-off (epilogue done -> next layer's input seen by the MMA warp), as
-    medians over the residual layers of CTA 0, against the tensor floor of 2 tiles x 72 MMAs x 64 cycles."""
+    medians over the residual layers of CTA 0, against the tensor floor of 2 tiles x 72 MMAs x 64 cycles (split
+    precision: 3 x 72 MMAs per tile)."""
     import ctypes as C
     from caro_ai_b200 import _cabi
     from caro_ai_b200.game import ConnectFour, TicTacToe
     from caro_ai_b200.model import DeviceNet, Net, probe_positions
-    floor = 2 * 72 * 64
     for game, blocks, leaves in ((TicTacToe(15, 5), 10, 16384), (ConnectFour(), 5, 33152)):
         torch.manual_seed(0)
         dn = DeviceNet(Net(game.obs_shape, game.action_space, blocks=blocks, filters=128).eval(), game, precision="fp32-simt")
@@ -153,7 +161,8 @@ def timeline_bench(torch, out):
         d_boards, d_who = base_b[idx].contiguous(), base_w[idx].contiguous()
         trace = torch.zeros(8001, dtype=torch.int64, device="cuda")
         n_layers = blocks + 1
-        for name, impl in (("wide_fp16", 7), ("wide_bf16", 0)):
+        for name, impl in (("wide_fp16", 7), ("wide_bf16", 0), ("wide_bf16x3", 8)):
+            floor = 2 * 72 * 64 * (3 if impl == 8 else 1)
             for _ in range(3):
                 dn.forward_boards(d_boards, d_who, leaves, impl)
             trace.zero_()
@@ -180,12 +189,26 @@ def selfplay_bench(torch, out):
     from caro_ai_b200.engine import SelfPlayEngine
     from caro_ai_b200.game import ConnectFour, TicTacToe
     from caro_ai_b200.model import DeviceNet, Net
-    # (game, blocks, parts, games per part, searches, batch, node capacity, warm-up plies, timed plies, flags)
-    cases = [(TicTacToe(15, 5), 10, 2, 1024, 200, 8, 8192, 1, 3, {"compact_tree": True}),
-             (ConnectFour(), 5, 2, 8192, 100, 8, 8192, 2, 6, {})]
-    for game, blocks, parts, gpp, count, batch, cap, warm, plies, flags in cases:
+    sys.path.insert(0, os.path.join(ROOT, "tests"))
+    import wide_split_net
+
+    def random_init(game, blocks):
         torch.manual_seed(0)
-        dn = DeviceNet(Net(game.obs_shape, game.action_space, blocks=blocks, filters=128).eval(), game)
+        return Net(game.obs_shape, game.action_space, blocks=blocks, filters=128).eval().state_dict()
+
+    def trained_like(game, blocks):
+        return wide_split_net.trained_like_net(game, blocks)[1]
+
+    caro, c4, compact = TicTacToe(15, 5), ConnectFour(), {"compact_tree": True}
+    # (net, game, blocks, precision, parts, games per part, searches, batch, node capacity, warm-up plies, timed plies, flags)
+    cases = [("random_init", caro, 10, "auto", 2, 1024, 200, 8, 8192, 1, 3, compact),
+             ("random_init", c4, 5, "auto", 2, 8192, 100, 8, 8192, 2, 6, {}),
+             ("trained_like", caro, 10, "auto", 2, 1024, 200, 8, 8192, 1, 3, compact),
+             ("trained_like", caro, 10, "auto", 2, 256, 10, 8, 2048, 1, 1, compact),
+             ("trained_like", caro, 10, "fp32-simt", 2, 256, 10, 8, 2048, 1, 1, compact)]
+    for kind, game, blocks, precision, parts, gpp, count, batch, cap, warm, plies, flags in cases:
+        sd = random_init(game, blocks) if kind == "random_init" else trained_like(game, blocks)
+        dn = DeviceNet(sd, game, precision=precision)
         engs = [SelfPlayEngine(game, gpp, max_batch=batch, node_capacity=cap, seed=11 + 7 * h, **flags) for h in range(parts)]
         SelfPlayEngine.play_multi(engs, dn, moves=warm, count=count, batch=batch, tau_plies=30, auto_restart=True)
         torch.cuda.synchronize()
@@ -198,10 +221,11 @@ def selfplay_bench(torch, out):
         sec = s.elapsed_time(e) / 1e3
         c1 = [x.counters() for x in engs]
         d = {k: sum(b[k] - a[k] for a, b in zip(c0, c1)) for k in c1[0]}
-        emit({"kind": "selfplay", "game": type(game).__name__, "board": list(game.obs_shape[1:]), "blocks": blocks, "filters": 128,
-              "games": parts * gpp, "parts": parts, "search_batch": [count, batch], "compact_tree": bool(flags.get("compact_tree")),
-              "timed_plies": plies, "ms_per_ply": 1e3 * sec / plies, "leaf_evals_per_sec": d["leaf_evals"] / sec,
-              "errors": sum(c["errors"] for c in c1), "precision": dn.precision, "calibration": dn.calibration}, out)
+        emit({"kind": "selfplay", "net": kind, "game": type(game).__name__, "board": list(game.obs_shape[1:]), "blocks": blocks,
+              "filters": 128, "games": parts * gpp, "parts": parts, "search_batch": [count, batch],
+              "compact_tree": bool(flags.get("compact_tree")), "timed_plies": plies, "ms_per_ply": 1e3 * sec / plies,
+              "leaf_evals_per_sec": d["leaf_evals"] / sec, "errors": sum(c["errors"] for c in c1), "precision": dn.precision,
+              "impl": dn.impl, "calibration": dn.calibration}, out)
         for x in engs:
             x.close()
         dn.close()
