@@ -18,12 +18,14 @@ def oracle_for(game):
 
 class StubOracleTree(OracleMCTS):
     """OracleMCTS whose network is the integer stub and whose Dirichlet draws are replayed from
-    `noise[minibatch][descent]`."""
+    `noise[minibatch][descent]`.  `stub` is the network: stub_priors, or any other pure function of the planes with
+    the same signature (oracle.stubs.chain_priors)."""
 
-    def __init__(self, game, c_puct=1.0, alpha=0.3, explore=0.25):
+    def __init__(self, game, c_puct=1.0, alpha=0.3, explore=0.25, stub=stub_priors):
         super().__init__(game, c_puct, alpha, explore, dirichlet=self._next_noise)
         self._noise = None
         self._j = 0
+        self._stub = stub
 
     def _next_noise(self, alpha):
         z = self._noise[self._j]
@@ -32,7 +34,7 @@ class StubOracleTree(OracleMCTS):
 
     def evaluate(self, states, players, net, device="cpu"):
         planes = self.game.states_to_training_batch(states, players)
-        return stub_priors(planes, self.game.action_space)
+        return self._stub(planes, self.game.action_space)
 
     def minibatch(self, batch, state, player, noise_bj):
         self._noise, self._j = noise_bj, 0
