@@ -6,7 +6,7 @@ import os
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "libcaro_b200.so")
 
-GAME_CONNECT4, GAME_MNK = 0, 1
+GAME_CONNECT4, GAME_MNK, GAME_CARO = 0, 1, 2
 
 
 class CaroError(RuntimeError):

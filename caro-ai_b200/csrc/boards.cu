@@ -103,9 +103,12 @@ static inline cudaStream_t S(void* s) { return reinterpret_cast<cudaStream_t>(s)
 
 static int check_game(int game, int n, int k) {
   if (game == CARO_GAME_CONNECT4) return CARO_OK;
-  if (game == CARO_GAME_MNK && n >= 2 && n <= 15 && k >= 2 && k <= n) return CARO_OK;
+  if ((game == CARO_GAME_MNK || game == CARO_GAME_CARO) && n >= 2 && n <= 15 && k >= 2 && k <= n) return CARO_OK;
   return caro_fail(CARO_E_ARG, "unknown game or bad (n,k)");
 }
+
+// freestyle m,n,k or Caro (the same board; a run blocked at both ends does not win)
+static MnkRules mnk_rules(int game, int n, int k) { return MnkRules{n, k, game == CARO_GAME_CARO ? 1 : 0}; }
 
 extern "C" {
 
@@ -120,7 +123,7 @@ int caro_boards_apply(int game, int n, int k, const void* d_boards, const int32_
     apply_kernel<C4Rules><<<grid, 256, 0, S(stream)>>>(C4Rules(), (const C4Board*)d_boards, d_actions, d_players, count,
                                                        (C4Board*)d_out, d_won, d_draw);
   else
-    apply_kernel<MnkRules><<<grid, 256, 0, S(stream)>>>(MnkRules{n, k}, (const MnkBoard*)d_boards, d_actions, d_players, count,
+    apply_kernel<MnkRules><<<grid, 256, 0, S(stream)>>>(mnk_rules(game, n, k), (const MnkBoard*)d_boards, d_actions, d_players, count,
                                                         (MnkBoard*)d_out, d_won, d_draw);
   return caro_check_launch("apply_kernel");
 }
@@ -134,7 +137,7 @@ int caro_boards_legal_mask(int game, int n, int k, const void* d_boards, int64_t
   if (game == CARO_GAME_CONNECT4)
     legal_kernel<C4Rules><<<grid, 256, 0, S(stream)>>>(C4Rules(), (const C4Board*)d_boards, count, 1, d_mask);
   else
-    legal_kernel<MnkRules><<<grid, 256, 0, S(stream)>>>(MnkRules{n, k}, (const MnkBoard*)d_boards, count, (n * n + 31) / 32, d_mask);
+    legal_kernel<MnkRules><<<grid, 256, 0, S(stream)>>>(mnk_rules(game, n, k), (const MnkBoard*)d_boards, count, (n * n + 31) / 32, d_mask);
   return caro_check_launch("legal_kernel");
 }
 
@@ -159,16 +162,16 @@ int caro_boards_encode_planes(int game, int n, int k, const void* d_boards, cons
     planes_vec_kernel<C4Rules, 4><<<grid, 256, 0, S(stream)>>>(C4Rules(), (const C4Board*)d_boards, d_who, count, d_planes);
   } else if (game != CARO_GAME_CONNECT4 && aligned && per % 4 == 0) {
     const unsigned grid = (unsigned)((count * (per / 4) + 255) / 256);
-    planes_vec_kernel<MnkRules, 4><<<grid, 256, 0, S(stream)>>>(MnkRules{n, k}, (const MnkBoard*)d_boards, d_who, count, d_planes);
+    planes_vec_kernel<MnkRules, 4><<<grid, 256, 0, S(stream)>>>(mnk_rules(game, n, k), (const MnkBoard*)d_boards, d_who, count, d_planes);
   } else if (game != CARO_GAME_CONNECT4 && aligned) {
     const unsigned grid = (unsigned)((count * (per / 2) + 255) / 256);
-    planes_vec_kernel<MnkRules, 2><<<grid, 256, 0, S(stream)>>>(MnkRules{n, k}, (const MnkBoard*)d_boards, d_who, count, d_planes);
+    planes_vec_kernel<MnkRules, 2><<<grid, 256, 0, S(stream)>>>(mnk_rules(game, n, k), (const MnkBoard*)d_boards, d_who, count, d_planes);
   } else {
     const unsigned grid = (unsigned)((count * per + 255) / 256);
     if (game == CARO_GAME_CONNECT4)
       planes_kernel<C4Rules><<<grid, 256, 0, S(stream)>>>(C4Rules(), (const C4Board*)d_boards, d_who, count, d_planes);
     else
-      planes_kernel<MnkRules><<<grid, 256, 0, S(stream)>>>(MnkRules{n, k}, (const MnkBoard*)d_boards, d_who, count, d_planes);
+      planes_kernel<MnkRules><<<grid, 256, 0, S(stream)>>>(mnk_rules(game, n, k), (const MnkBoard*)d_boards, d_who, count, d_planes);
   }
   return caro_check_launch("planes_kernel");
 }

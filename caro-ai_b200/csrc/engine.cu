@@ -156,7 +156,7 @@ int fill_dims(const caro_engine_config* cfg, Dims* dm, int* max_plies) {
   if (cfg->game == CARO_GAME_CONNECT4) {
     A = 7;
     plies = 42;
-  } else if (cfg->game == CARO_GAME_MNK) {
+  } else if (cfg->game == CARO_GAME_MNK || cfg->game == CARO_GAME_CARO) {
     if (cfg->n < 2 || cfg->n > 15 || cfg->k < 2 || cfg->k > cfg->n) return caro_fail(CARO_E_ARG, "m,n,k needs 2 <= k <= n <= 15");
     A = cfg->n * cfg->n;
     plies = A;
@@ -279,6 +279,7 @@ int caro_engine_create(const caro_engine_config* cfg, void* d_workspace, size_t 
   e->ws_bytes = need;
   e->mnk.n = cfg->n;
   e->mnk.k = cfg->k;
+  e->mnk.blocked_ends = cfg->game == CARO_GAME_CARO ? 1 : 0;
   if (cfg->game == CARO_GAME_CONNECT4) {
     build_view<C4Board>(e->carve, dm, e->ws, &e->v_c4);
     e->board_bytes = sizeof(C4Board);

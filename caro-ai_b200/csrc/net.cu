@@ -305,7 +305,7 @@ int caro_net_forward(caro_net* net, int game, int n, int k, const void* d_boards
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   if (game == CARO_GAME_CONNECT4) {
     if (net->H != 6 || net->W != 7 || net->A != 7) return caro_fail(CARO_E_ARG, "net shape does not match Connect4");
-  } else if (game == CARO_GAME_MNK) {
+  } else if (game == CARO_GAME_MNK || game == CARO_GAME_CARO) {  // the network does not depend on the win rule
     if (net->H != n || net->W != n || net->A != n * n) return caro_fail(CARO_E_ARG, "net shape does not match the m,n,k board");
   } else {
     return caro_fail(CARO_E_ARG, "unknown game");

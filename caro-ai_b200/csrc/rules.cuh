@@ -107,6 +107,9 @@ struct MnkRules {
   using Board = MnkBoard;
   int n;  // board side (<= 15)
   int k;  // run length to win
+  // 0: freestyle (any run >= k wins).  1: Caro -- a run >= k with an opponent stone just past BOTH of its ends does
+  // not win (the board edge never blocks).  Read only once a direction already reaches k.
+  int blocked_ends;
 
   CARO_HD int actions() const { return n * n; }
   CARO_HD int rows() const { return n; }
@@ -151,11 +154,30 @@ struct MnkRules {
     return cnt;
   }
 
+  // Caro: is the cell just past the END of the maximal run of `mine` from (r, c) along (dr, dc) an opponent stone?
+  // The walk runs to the real end of the run (up to n - 1 cells), not ray's k - 1: overlines and dense boards have
+  // runs longer than k.  Off the board is not a block.
+  CARO_HD bool flank_blocked(const uint64_t* mine, const uint64_t* other, int r, int c, int dr, int dc) const {
+    int rr = r + dr, cc = c + dc;
+    while (rr >= 0 && rr < n && cc >= 0 && cc < n && test(mine, rr * n + cc)) {
+      rr += dr;
+      cc += dc;
+    }
+    return rr >= 0 && rr < n && cc >= 0 && cc < n && test(other, rr * n + cc);
+  }
+
+  // The line through (r, c) along +-(dr, dc) wins: a run >= k and, under Caro, not blocked at both ends.
+  CARO_HD bool line_wins(const uint64_t* mine, const uint64_t* other, int r, int c, int dr, int dc) const {
+    if (1 + ray(mine, r, c, dr, dc) + ray(mine, r, c, -dr, -dc) < k) return false;
+    return !blocked_ends || !(flank_blocked(mine, other, r, c, dr, dc) && flank_blocked(mine, other, r, c, -dr, -dc));
+  }
+
   // tictactoe.py:210-235 + tictactoe_helpers.py:7-56.  The reference scans the whole row /
   // column / diagonal / anti-diagonal through the move for ANY run >= k; in every position
   // reachable by legal play (the game stops at the first win) that equals "the run through the
   // new cell is >= k", which is what is evaluated here.  Like the reference the target cell is
-  // overwritten without an emptiness check.
+  // overwritten without an emptiness check.  With blocked_ends set (Caro) a direction whose run
+  // has an opponent stone past both ends does not win; another direction still may.
   CARO_HD bool apply(Board& s, int a, int player) const {
     const uint64_t bit = 1ULL << (a & 63);
     uint64_t* mine = player ? s.b : s.w;
@@ -164,10 +186,10 @@ struct MnkRules {
     other[a >> 6] &= ~bit;
     const int r = a / n, c = a - r * n;
     bool won = false;
-    won = won || (1 + ray(mine, r, c, 0, 1) + ray(mine, r, c, 0, -1) >= k);
-    won = won || (1 + ray(mine, r, c, 1, 0) + ray(mine, r, c, -1, 0) >= k);
-    won = won || (1 + ray(mine, r, c, 1, 1) + ray(mine, r, c, -1, -1) >= k);
-    won = won || (1 + ray(mine, r, c, -1, 1) + ray(mine, r, c, 1, -1) >= k);
+    won = won || line_wins(mine, other, r, c, 0, 1);
+    won = won || line_wins(mine, other, r, c, 1, 0);
+    won = won || line_wins(mine, other, r, c, 1, 1);
+    won = won || line_wins(mine, other, r, c, -1, 1);
     return won;
   }
 

@@ -306,6 +306,24 @@ class TicTacToe(_DeviceGame):
         return "\n".join(rows)
 
 
+class Caro(TicTacToe):
+    """Caro (Vietnamese gomoku) on an n x n board: k in a row wins unless the run is blocked at both ends.
+
+    Everything but the win test is TicTacToe(n, k)'s: state integers, planes, actions, render and the draw rule.  A
+    move wins when, in one of the four directions, the maximal run of the mover's stones through it reaches k
+    (overlines count) and does not have an opponent stone just past both of its ends; the board edge never blocks.
+    A blocked run stays on the board and the game goes on (rule in csrc/rules.cuh, MnkRules::blocked_ends)."""
+
+    game_kind = _cabi.GAME_CARO
+
+    def __init__(self, n: int = 15, k_to_win: int = 5):
+        super().__init__(n, k_to_win)
+
+
 def get_game(game_type: str):
-    """lib/game/game_provider.py:15-22: '0' -> ConnectFour, anything else -> TicTacToe()."""
-    return ConnectFour() if game_type == "0" else TicTacToe()
+    """lib/game/game_provider.py:15-22: '0' -> ConnectFour, '2' -> Caro(15, 5), anything else -> TicTacToe()."""
+    if game_type == "0":
+        return ConnectFour()
+    if game_type == "2":
+        return Caro()
+    return TicTacToe()

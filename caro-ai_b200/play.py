@@ -22,7 +22,8 @@ def main(argv=None):
     parser.add_argument("models", nargs="+", help="The list of models (at least 2) to play against each other")
     parser.add_argument("-r", "--rounds", type=int, default=2, help="Count of rounds to perform for every pair")
     parser.add_argument("--cuda", default=False, action="store_true", help="accepted for compatibility (always CUDA)")
-    parser.add_argument("-g", "--game", required=True, choices=["0", "1"], help="The type of game. 0: Connect4, 1: TicTacToe")
+    parser.add_argument("-g", "--game", required=True, choices=["0", "1", "2"],
+                        help="The type of game. 0: Connect4, 1: TicTacToe, 2: Caro 15x15")
     parser.add_argument("--precision", default="auto", choices=["auto", "bf16", "bf16x3"],
                         help="tensor-core precision: auto (default) keeps the one-pass bf16 tower only while it reproduces the fp32 priors to 1e-3 on probe positions")
     args = parser.parse_args(argv)

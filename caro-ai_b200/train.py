@@ -142,7 +142,7 @@ def parse_args(argv=None):
     p = argparse.ArgumentParser()
     p.add_argument("-n", "--name", required=True, help="Name of the run")
     p.add_argument("--cuda", default=False, action="store_true", help="accepted for compatibility (always CUDA)")
-    p.add_argument("-g", "--game", required=True, choices=["0", "1"], help="0: Connect4, 1: TicTacToe")
+    p.add_argument("-g", "--game", required=True, choices=["0", "1", "2"], help="0: Connect4, 1: TicTacToe, 2: Caro 15x15")
     p.add_argument("--games", type=int, default=256, help="self-play games per step and per rank (reference: PLAY_EPISODES=1)")
     p.add_argument("--max-steps", type=int, default=0, help="stop after this many steps (0 = run forever, like the reference)")
     p.add_argument("--replay-steps", type=int, default=4, help="device replay ring = this many steps of --games games (>= REPLAY_BUFFER)")

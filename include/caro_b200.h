@@ -21,6 +21,12 @@
  *   Connect4 : caro_c4_board  {mask, black}, bit = 7*col + row (row 0 = bottom, bit 6 of each
  *              column is an always-empty sentinel).
  *   m,n,k    : caro_mnk_board {w[4], b[4]}, bit = row*n + col (= the action index), n <= 15.
+ *   Caro     : the m,n,k board, (n, k) bounds, actions, planes and draw rule; only the win test
+ *              differs.  A move wins iff in at least one of the four directions the maximal run
+ *              of the mover's stones through the new cell is >= k (overlines count) AND that run
+ *              is not blocked at both ends, an end being blocked when the cell just past it is on
+ *              the board and holds an opponent stone.  The board edge never blocks.  A blocked run
+ *              stays on the board and the game goes on.
  */
 #ifndef CARO_B200_H_
 #define CARO_B200_H_
@@ -36,7 +42,7 @@ extern "C" {
 
 enum { CARO_OK = 0, CARO_E_ARG = -1, CARO_E_CUDA = -2, CARO_E_STATE = -3, CARO_E_CAPACITY = -4 };
 
-enum { CARO_GAME_CONNECT4 = 0, CARO_GAME_MNK = 1 };
+enum { CARO_GAME_CONNECT4 = 0, CARO_GAME_MNK = 1, CARO_GAME_CARO = 2 };
 
 typedef struct { uint64_t mask, black; } caro_c4_board;
 typedef struct { uint64_t w[4], b[4]; } caro_mnk_board;
@@ -48,7 +54,7 @@ int caro_device_count(void);
 
 /* ------------------------------------------------------------------------------------------
  * Stand-alone board kernels -- rows a11..a16 of SURVEY.md section 8.
- * `d_boards` is an array of `count` caro_c4_board (game = CONNECT4) or caro_mnk_board (MNK).
+ * `d_boards` is an array of `count` caro_c4_board (game = CONNECT4) or caro_mnk_board (MNK, CARO).
  * ------------------------------------------------------------------------------------------ */
 
 /* game.move for a batch: lib/game/connect_four/connect_four.py:241-265 (+ _check_won :206-239),
@@ -160,7 +166,7 @@ typedef struct caro_engine caro_engine;
 
 typedef struct {
   int32_t game;            /* CARO_GAME_* */
-  int32_t n, k;            /* m,n,k only */
+  int32_t n, k;            /* m,n,k and Caro only */
   int32_t games;           /* G */
   int32_t trees_per_game;  /* 1 or 2 */
   int32_t max_batch;       /* largest batch_size (descents per minibatch) that will be used, 1..32 */
