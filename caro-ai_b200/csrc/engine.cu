@@ -144,6 +144,12 @@ void build_view(Carver& c, const Dims& dm, char* base, View<Board>* v) {
   CARVE(rp_z, "replay_z", float, rc);
   CARVE(rp_cursor, "replay_cursor", unsigned long long, 1);
   CARVE(ctr, "counters", unsigned long long, CTR_COUNT);
+  // resignation (extension): carved after every other region so that no earlier offset moves; zero (= off) at create
+  CARVE(resign_params, "resign_params", ResignParams, 1);
+  CARVE(resign_playthrough, "resign_playthrough", uint8_t, dm.G);
+  CARVE(resign_min, "resign_min", double, dm.G, 2);
+  CARVE(resign_log, "resign_log", ResignRecord, dm.G);
+  CARVE(resign_ctr, "resign_counters", unsigned long long, RCTR_COUNT);
 #undef CARVE
 }
 
@@ -747,6 +753,19 @@ int caro_engine_replay_gather(caro_engine* e, const int64_t* d_entries, const in
   else
     replay_gather_kernel<MnkRules><<<(unsigned)count, 64, 0, S(stream)>>>(e->v_mnk, e->mnk, e->dm, ent, d_symmetry, (long long)count, d_planes, d_pi, d_z);
   return caro_check_launch("replay_gather_kernel");
+}
+
+int caro_engine_set_resign(caro_engine* e, int enable, double threshold, double playthrough, void* stream) {
+  if (!e) return caro_fail(CARO_E_ARG, "null engine");
+  if (!(threshold >= -1.0 && threshold <= 1.0)) return caro_fail(CARO_E_ARG, "resign threshold must be in [-1, 1]");
+  if (!(playthrough >= 0.0 && playthrough <= 1.0)) return caro_fail(CARO_E_ARG, "resign playthrough must be in [0, 1]");
+  ResignParams p{};
+  p.enabled = enable ? 1 : 0;
+  p.threshold = threshold;
+  p.playthrough = playthrough;
+  ResignParams* dst = e->cfg.game == CARO_GAME_CONNECT4 ? e->v_c4.resign_params : e->v_mnk.resign_params;
+  set_resign_kernel<<<1, 1, 0, S(stream)>>>(dst, p);
+  return caro_check_launch("set_resign_kernel");
 }
 
 int caro_engine_counters(caro_engine* e, uint64_t h_out[8], void* stream) {

@@ -67,6 +67,23 @@ struct Dims {
 };
 enum : unsigned { FLAG_VIRTUAL_LOSS = 1u, FLAG_MASK_PRIORS = 2u, FLAG_FRESH_TREE = 4u, FLAG_RECYCLE_TREE = 8u, FLAG_COMPACT_TREE = 16u };
 
+// Resignation (extension, off by default; include/caro_b200.h caro_engine_set_resign).  The parameters live in device memory
+// and are read by advance_kernel / reset_kernel at run time, so a captured ply graph never holds stale values.
+struct alignas(8) ResignParams {
+  int32_t enabled;     // 0 = off: no statistic, no resignation, no log
+  int32_t pad_;
+  double threshold;    // the side to move resigns when its root statistic is < threshold
+  double playthrough;  // share of games (drawn per game at its start) that never resign and are logged instead
+};
+// One finished playthrough game: the smallest root statistic each player saw, the result from player 0's point of view
+struct alignas(8) ResignRecord {
+  double min_stat[2];
+  int32_t result;
+  int32_t plies;
+};
+static_assert(sizeof(ResignRecord) == 24, "resign log records are 24 bytes");
+enum { RCTR_RESIGNED = 0, RCTR_LOGGED, RCTR_COUNT };
+
 struct SearchParams {
   double c_puct, alpha, explore;
   uint32_t seed_lo, seed_hi;
@@ -123,6 +140,12 @@ struct View {
   unsigned long long* rp_cursor;  // [1] total entries ever written
   // ---- counters ------------------------------------------------------------------------------
   unsigned long long* ctr;  // [CTR_COUNT]
+  // ---- resignation (extension) -----------------------------------------------------------------
+  ResignParams* resign_params;   // [1]
+  uint8_t* resign_playthrough;   // [G] the current game is a playthrough game
+  double* resign_min;            // [G][2] smallest statistic per player of the current playthrough game
+  ResignRecord* resign_log;      // [G] ring of finished playthrough games (slot = cursor % G)
+  unsigned long long* resign_ctr;  // [RCTR_COUNT] games resigned, playthrough games logged (= log cursor)
 };
 
 }  // namespace caro

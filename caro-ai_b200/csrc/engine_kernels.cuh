@@ -1102,6 +1102,22 @@ compact_kernel(View<typename R::Board> e, R rules, Dims dm, int chunk_nodes) {
   for (int i = tid; i < kept; i += 256) ht_insert_cas(ht, dm.hash_cap, gen, rules.key(e.node_board[nb + i]).lo, i);
 }
 
+// ----------------------------------------------------------------------------------- resignation
+// Extension (caro_engine_set_resign, off by default).  A game that starts while resignation is on is a playthrough game
+// with probability `playthrough` (a Philox draw of its uid): it never resigns and logs its per-player minima instead.
+template <class Board>
+__device__ __forceinline__ void resign_game_start(const View<Board>& e, const SearchParams& sp, int g, uint64_t uid) {
+  const ResignParams rp = *e.resign_params;
+  uint8_t play = 0;
+  if (rp.enabled) {
+    const Philox4 r = philox4x32_10((uint32_t)uid, (uint32_t)(uid >> 32), 0u, 0u, sp.seed_lo ^ kStreamResign, sp.seed_hi);
+    play = u01d(r.v[0], r.v[1]) < rp.playthrough ? 1 : 0;
+    e.resign_min[2 * g] = INFINITY;
+    e.resign_min[2 * g + 1] = INFINITY;
+  }
+  e.resign_playthrough[g] = play;
+}
+
 // ----------------------------------------------------------------------------------- advance
 // One ply of lib/utils.py:76-106 for every active game.  One thread per game.
 template <class R>
@@ -1120,18 +1136,34 @@ __global__ void advance_kernel(View<typename R::Board> e, R rules, Dims dm, Sear
   const int who = e.root_player[g];
   const int ply = e.ply[g];
   const int tau = ply < tau_plies ? 1 : 0;  // lib/utils.py:68,97-99
+  const ResignParams rp = *e.resign_params;
   // visit counts -> pi
   long long total = 0;
   int best_n = -1, best_a = 0;
+  double sum_w = 0.0;  // resignation statistic: sum of W over the root's edges, in action order
   const size_t row = (nb + (size_t)(node < 0 ? 0 : node)) * dm.RS;
   if (node >= 0) {
     for (int a = 0; a < A; ++a) {
       const int n = e.N[row + a] & kCountMask;
       total += n;
+      if (rp.enabled) sum_w = __dadd_rn(sum_w, (double)e.W[row + a]);
       if (n > best_n) {
         best_n = n;
         best_a = a;
       }
+    }
+  }
+  // stat = max(mean root value, Q of the most visited edge), from the mover's point of view
+  bool resign = false;
+  if (rp.enabled && total > 0) {
+    const double v_root = __ddiv_rn(sum_w, (double)total);
+    const double v_best = (double)__fdiv_rn(e.W[row + best_a], (float)best_n);
+    const double stat = v_root > v_best ? v_root : v_best;
+    if (e.resign_playthrough[g]) {
+      double* m = e.resign_min + 2 * g + who;
+      if (stat < *m) *m = stat;
+    } else {
+      resign = stat < rp.threshold;
     }
   }
   // np.random.choice(A, p=pi): cdf = cumsum(p) / cumsum(p)[-1]; first index with cdf > u
@@ -1158,7 +1190,7 @@ __global__ void advance_kernel(View<typename R::Board> e, R rules, Dims dm, Sear
       }
     }
   }
-  if (action_out) action_out[g] = action;
+  if (action_out) action_out[g] = resign ? -1 : action;
   // history (lib/utils.py:81)
   const int hidx = ply < dm.max_plies ? ply : dm.max_plies - 1;
   const size_t h = (size_t)g * dm.max_plies + hidx;
@@ -1170,11 +1202,17 @@ __global__ void advance_kernel(View<typename R::Board> e, R rules, Dims dm, Sear
     else p = (float)__ddiv_rn((double)(e.N[row + a] & kCountMask), (double)total);
     e.hist_pi[h * A + a] = p;
   }
-  if (!rules.legal(s, action)) atomicOr(e.ctr + CTR_ERRORS, ERR_ILLEGAL_ACTION);  // "Impossible action selected"
-  const bool won = rules.apply(s, action, who);
+  bool won = false;
+  if (!resign) {
+    if (!rules.legal(s, action)) atomicOr(e.ctr + CTR_ERRORS, ERR_ILLEGAL_ACTION);  // "Impossible action selected"
+    won = rules.apply(s, action, who);
+  }
   atomicAdd(e.ctr + CTR_PLIES, 1ull);
   int finished = 0, res = 0;  // res from the last mover's point of view (lib/utils.py:88,94)
-  if (won) {
+  if (resign) {
+    finished = 1;
+    res = -1;
+  } else if (won) {
     finished = 1;
     res = 1;
   } else if (!rules.any_legal(s)) {
@@ -1200,9 +1238,20 @@ __global__ void advance_kernel(View<typename R::Board> e, R rules, Dims dm, Sear
   }
   // ---- game over -------------------------------------------------------------------------
   const int n_hist = hidx + 1;
-  e.result[g] = won ? (who == 0 ? 1 : -1) : 0;  // net1 == player 0 (lib/utils.py:89)
+  const int result = who == 0 ? res : -res;  // net1 == player 0 (lib/utils.py:89)
+  e.result[g] = result;
   atomicAdd(e.ctr + CTR_GAMES, 1ull);
-  atomicAdd(e.ctr + (won ? (who == 0 ? CTR_WIN0 : CTR_WIN1) : CTR_DRAW), 1ull);
+  atomicAdd(e.ctr + (result == 0 ? CTR_DRAW : (result > 0 ? CTR_WIN0 : CTR_WIN1)), 1ull);
+  if (resign) atomicAdd(e.resign_ctr + RCTR_RESIGNED, 1ull);
+  if (rp.enabled && e.resign_playthrough[g]) {
+    const unsigned long long k = atomicAdd(e.resign_ctr + RCTR_LOGGED, 1ull);
+    ResignRecord rec;
+    rec.min_stat[0] = e.resign_min[2 * g];
+    rec.min_stat[1] = e.resign_min[2 * g + 1];
+    rec.result = result;
+    rec.plies = ply + 1;
+    e.resign_log[k % (unsigned long long)dm.G] = rec;
+  }
   if (dm.replay_cap > 0) {
     // lib/utils.py:101-106: z = result for the last entry, sign flips walking back
     const unsigned long long base = atomicAdd(e.rp_cursor, (unsigned long long)n_hist);
@@ -1234,6 +1283,7 @@ __global__ void advance_kernel(View<typename R::Board> e, R rules, Dims dm, Sear
     e.root_player[g] = (uint8_t)fp;
     e.ply[g] = 0;
     e.status[g] = ST_ACTIVE;
+    resign_game_start(e, sp, g, uid);
     for (int t = 0; t < dm.tpg; ++t) {  // MCTS.clear(): bump the generation, no memset
       e.node_count[g * dm.tpg + t] = 0;
       e.tree_gen[g * dm.tpg + t] += 1u;
@@ -1285,6 +1335,10 @@ replay_gather_kernel(View<typename R::Board> e, R rules, Dims dm, const long lon
   if (threadIdx.x == 0) z[i] = e.rp_z[slot];
 }
 
+// ----------------------------------------------------------------------------- resignation parameters
+// One thread: the parameters arrive by value and are stored on the stream, behind every earlier ply.
+__global__ void set_resign_kernel(ResignParams* __restrict__ dst, ResignParams p) { *dst = p; }
+
 // ------------------------------------------------------------------------------------- reset
 template <class R>
 __global__ void reset_kernel(View<typename R::Board> e, Dims dm, SearchParams sp, const uint8_t* __restrict__ mask,
@@ -1309,6 +1363,7 @@ __global__ void reset_kernel(View<typename R::Board> e, Dims dm, SearchParams sp
   e.ply[g] = 0;
   e.status[g] = ST_ACTIVE;
   e.result[g] = 0;
+  resign_game_start(e, sp, g, uid);
   for (int t = 0; t < dm.tpg; ++t) {
     e.node_count[g * dm.tpg + t] = 0;
     e.tree_gen[g * dm.tpg + t] += 1u;

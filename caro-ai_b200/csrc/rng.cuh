@@ -41,7 +41,8 @@ CARO_HD double u01d(uint32_t hi, uint32_t lo) {
 }
 
 // Stream tags
-enum : uint32_t { kStreamDirichlet = 0x44495243u, kStreamChoice = 0x43484F49u, kStreamFirst = 0x46495253u };
+enum : uint32_t { kStreamDirichlet = 0x44495243u, kStreamChoice = 0x43484F49u, kStreamFirst = 0x46495253u,
+                  kStreamResign = 0x52455347u };
 
 // Device code uses the fast-math intrinsics: the noise only has to be distributed correctly, and whatever is
 // generated is what both the engine and (through noise_out) the oracle consume.

@@ -115,3 +115,16 @@ def reduce_tallies(wins: int, losses: int, draws: int, device=None) -> Tuple[int
     t = torch.tensor([wins, losses, draws], dtype=torch.int64, device=device)
     dist.all_reduce(t, op=dist.ReduceOp.SUM)
     return int(t[0]), int(t[1]), int(t[2])
+
+
+def sum_counts(counts, device=None):
+    """Element-wise sum over the ranks of an integer array (the resignation calibration's per-threshold tallies): one
+    all-reduce, so every rank derives the same decision from the same numbers."""
+    import numpy as np
+    counts = np.asarray(counts, dtype=np.int64)
+    _, ws = world()
+    if ws == 1:
+        return counts
+    t = torch.from_numpy(counts.copy()).to(device if device is not None else "cpu")
+    dist.all_reduce(t, op=dist.ReduceOp.SUM)
+    return t.cpu().numpy()

@@ -266,6 +266,34 @@ class SelfPlayEngine:
         _cabi.check(_cabi.lib().caro_engine_play_multi(arr, len(engines), net.handle, moves, count, batch, tau_plies,
                                                        1 if auto_restart else 0, first_player, impl, engines[0]._stream()))
 
+    # ------------------------------------------------------------------ resignation (extension)
+    def set_resign(self, threshold: Optional[float] = None, playthrough: float = 0.0):
+        """Resignation (extension, off by default; include/caro_b200.h caro_engine_set_resign): from the next ply on, the
+        side to move resigns when max(mean root value, Q of its most visited move) < ``threshold``.  ``threshold=None``
+        switches it off; -1.0 never fires ("log only").  ``playthrough``: share of the games starting after this call that
+        never resign and are logged instead (``resign_log``).  Enqueued on the current stream."""
+        enable = threshold is not None
+        _cabi.check(_cabi.lib().caro_engine_set_resign(self.handle, 1 if enable else 0, float(threshold) if enable else -1.0,
+                                                       float(playthrough), self._stream()))
+
+    RESIGN_RECORD_DTYPE = np.dtype([("min_stat", np.float64, (2,)), ("result", np.int32), ("plies", np.int32)])
+
+    def resign_log(self, start: int = 0) -> Tuple[np.ndarray, int]:
+        """Records [start, cursor) of the playthrough-game log (the ring keeps the last G), oldest first, as a structured
+        array of ``RESIGN_RECORD_DTYPE`` (min_stat per player, result from player 0's point of view, plies).  Returns
+        (records, cursor)."""
+        cursor = self.resign_counters()["logged"]
+        start = max(start, cursor - self.G)
+        if cursor <= start:
+            return np.zeros(0, dtype=self.RESIGN_RECORD_DTYPE), cursor
+        raw = self.region("resign_log").cpu().numpy().view(self.RESIGN_RECORD_DTYPE).reshape(-1)
+        return raw[np.arange(start, cursor) % self.G].copy(), cursor
+
+    def resign_counters(self) -> Dict[str, int]:
+        """{"resigned": games that ended by resignation, "logged": playthrough games logged (= the log cursor)}."""
+        c = self.region("resign_counters").cpu().numpy()
+        return {"resigned": int(c[0]), "logged": int(c[1])}
+
     # ------------------------------------------------------------------ read-back
     COUNTER_NAMES = ("leaf_evals", "games", "plies", "wins_p0", "wins_p1", "draws", "descents", "errors")
 

@@ -9,7 +9,8 @@ Same pieces as the reference: a replay buffer (here the self-play engine's DEVIC
 never smaller than REPLAY_BUFFER), 10 SGD rounds of 256 samples (MSE + soft-target cross-entropy, lr 0.1, momentum 0.9),
 an arena of EVALUATION_ROUNDS games every EVALUATE_EVERY_STEP steps with 20 x 16 searches at tau = 0, promotion above
 0.60, checkpoints ``saves/<name>/best_%03d_%05d.dat`` written with ``torch.save(net.state_dict())``, TensorBoard tags
-speed_steps / speed_nodes / loss_total / loss_value / loss_policy / eval_win_ratio.
+speed_steps / speed_nodes / loss_total / loss_value / loss_policy / eval_win_ratio (plus plies_per_game, and with the
+resignation extension resign_threshold / resign_fp_rate / resigned_share).
 The SGD step itself is plain PyTorch autograd (out of scope for hand kernels).  The batch never visits the host: the
 reference's ``random.sample`` draws entry numbers, a CUDA kernel turns the ring rows into the planes / pi / z tensors.
 With several ranks every rank contributes BATCH_SIZE / world rows of its own ring to the step's batch (one NCCL
@@ -59,7 +60,36 @@ def self_play(worker: SelfPlayWorker, best: DeviceNet, tb, step_idx: int):
     dt = time.time() - t
     tb.track("speed_steps", stats["plies"] / dt, step_idx)
     tb.track("speed_nodes", stats["leaf_evals"] / dt, step_idx)
+    if stats["games"]:
+        tb.track("plies_per_game", stats["plies"] / stats["games"], step_idx)
+    rs = worker.resign_stats()
+    if rs:
+        tb.track("resigned_share", rs["resigned_share"], step_idx)
+        if rs["threshold"] is not None:
+            tb.track("resign_threshold", rs["threshold"], step_idx)
+        if rs["fp_rate"] is not None:
+            tb.track("resign_fp_rate", rs["fp_rate"], step_idx)
     return stats, dt
+
+
+def resign_option(text: str):
+    """--resign: "off" -> None, "auto" -> "auto", else a threshold in [-1, 1]."""
+    if text in ("off", "auto"):
+        return None if text == "off" else "auto"
+    try:
+        t = float(text)
+    except ValueError:
+        raise argparse.ArgumentTypeError("expected off, auto or a threshold in [-1, 1], got %r" % text)
+    if not -1.0 <= t <= 1.0:
+        raise argparse.ArgumentTypeError("resign threshold must be in [-1, 1], got %r" % text)
+    return t
+
+
+def share_option(text: str) -> float:
+    v = float(text)
+    if not 0.0 <= v <= 1.0:
+        raise argparse.ArgumentTypeError("share must be in [0, 1], got %r" % text)
+    return v
 
 
 def sgd_losses(net: Net, planes: torch.Tensor, probs: torch.Tensor, values: torch.Tensor):
@@ -151,6 +181,11 @@ def parse_args(argv=None):
     p.add_argument("--augment", action="store_true", help="extension: random board symmetries on the sampled replay rows")
     p.add_argument("--compact-tree", action="store_true",
                    help="drop unreachable tree nodes after every move (bit-identical play, small arenas; for large boards)")
+    p.add_argument("--resign", type=resign_option, default=None, metavar="{off,auto,<threshold>}",
+                   help="extension: resign self-play games whose search says they are lost (default off; auto = calibrated "
+                        "from played-through games to keep wrong resignations under 5 %%)")
+    p.add_argument("--resign-playthrough", type=share_option, default=0.1,
+                   help="share of self-play games played through with resignation off to measure wrong resignations")
     p.add_argument("--evaluate-every", type=int, default=cfg.EVALUATE_EVERY_STEP, help="arena evaluation period in steps")
     p.add_argument("--blocks", type=int, default=5, choices=range(1, 21), metavar="{1..20}",
                    help="residual blocks of the network (reference: 5)")
@@ -180,7 +215,7 @@ def main(argv=None):
     bucket = D.FlatGradients(net.parameters())
     worker = SelfPlayWorker(game, args.games, cfg.MCTS_SEARCHES, cfg.MCTS_BATCH_SIZE, cfg.STEPS_BEFORE_TAU_0,
                             replay_steps=args.replay_steps, min_replay=cfg.REPLAY_BUFFER, seed=1000003 * rank + 17,
-                            compact_tree=args.compact_tree)
+                            compact_tree=args.compact_tree, resign=args.resign, resign_playthrough=args.resign_playthrough)
     step_idx = best_idx = 0
     with TBMeanTracker(writer, batch_size=10) as tb:
         while args.max_steps == 0 or step_idx < args.max_steps:
@@ -190,7 +225,11 @@ def main(argv=None):
             if rank == 0:
                 print("Step %d, steps %3d, leaves %4d, steps/s %5.2f, leaves/s %6.2f, best_idx %d, replay %d" % (
                     step_idx, stats["plies"], stats["leaf_evals"], stats["plies"] / dt, stats["leaf_evals"] / dt, best_idx,
-                    replay_len), end="\r")
+                    replay_len), end="")
+                if args.resign is not None:
+                    t = worker.resign_stats()["threshold"]
+                    print(", resign %s" % ("-" if t is None else "%.2f" % t), end="")
+                print(end="\r")
                 sys.stdout.flush()
             # train.py:199 -- decided on the SMALLEST ring of all ranks, so that every rank enters (or skips) the
             # collectives of the SGD rounds together

@@ -10,7 +10,7 @@ from typing import Dict, List, Optional, Tuple, Union
 import numpy as np
 import torch
 
-from . import mcts, model
+from . import distributed, mcts, model
 from .engine import SelfPlayEngine
 
 
@@ -140,6 +140,64 @@ def play_games_batched(game, n_games: int, net1, net2, steps_before_tau_0: int, 
     return totals
 
 
+# ------------------------------------------------------------------ resignation calibration (extension)
+# Thresholds the calibration can choose: -0.99, -0.98, ..., -0.50.
+RESIGN_GRID = tuple(round(-0.99 + 0.01 * i, 2) for i in range(50))
+RESIGN_WINDOW = 2000  # logged playthrough games per rank the "auto" calibration looks at
+
+
+def resign_tallies(records) -> np.ndarray:
+    """int64 [len(RESIGN_GRID), 2]: for every threshold t of the grid, (false positives, records) over the playthrough
+    games ``records`` (``SelfPlayEngine.resign_log``).  A game is a false positive at t when some player whose smallest
+    statistic was < t did not lose (won or drew): resigning there would have been wrong.  Tallies of several ranks or
+    windows add element-wise."""
+    out = np.zeros((len(RESIGN_GRID), 2), dtype=np.int64)
+    for i, t in enumerate(RESIGN_GRID):
+        out[i] = _false_positives(records, t), len(records)
+    return out
+
+
+def _false_positives(records, t: float) -> int:
+    if len(records) == 0:
+        return 0
+    mins = np.asarray(records["min_stat"], dtype=np.float64).reshape(-1, 2)
+    result = np.asarray(records["result"], dtype=np.int64).reshape(-1)
+    not_lost = np.stack([result != -1, result != 1], axis=1)  # player 0 lost iff result == -1, player 1 iff +1
+    return int(((mins < t) & not_lost).any(axis=1).sum())
+
+
+def choose_resign_threshold(tallies, target: float = 0.05, min_records: int = 200) -> Optional[float]:
+    """The largest threshold of RESIGN_GRID whose false-positive rate is <= ``target``; None while the tallies hold fewer
+    than ``min_records`` games, or when no threshold qualifies."""
+    tallies = np.asarray(tallies, dtype=np.int64)
+    n = int(tallies[0, 1])
+    if n < min_records:
+        return None
+    best = None
+    for i, t in enumerate(RESIGN_GRID):
+        if tallies[i, 0] <= target * n:
+            best = t
+    return best
+
+
+def resign_threshold_over_ranks(records, target: float = 0.05, min_records: int = 200,
+                                device=None) -> Tuple[Optional[float], np.ndarray]:
+    """``choose_resign_threshold`` on the tallies of ``records`` summed over all ranks (one all-reduce, entered by every
+    rank whether or not it holds records): every rank gets the same threshold.  Returns (threshold, summed tallies)."""
+    tallies = distributed.sum_counts(resign_tallies(records), device=device)
+    return choose_resign_threshold(tallies, target, min_records), tallies
+
+
+def _fp_rate(records, tallies, threshold: Optional[float]) -> Optional[float]:
+    """False-positive rate at ``threshold``: from the (rank-summed) tallies on the grid, from ``records`` off it."""
+    if threshold is None or tallies[0, 1] == 0:
+        return None
+    if threshold in RESIGN_GRID:
+        i = RESIGN_GRID.index(threshold)
+        return float(tallies[i, 0]) / float(tallies[i, 1])
+    return _false_positives(records, threshold) / len(records)
+
+
 class SelfPlayWorker:
     """The trainer's self-play side (train.py:25-59 for ``games`` games at once): ONE engine that lives as long as the
     training run -- its arenas are re-seated every step, not re-allocated -- and whose device replay ring is the
@@ -148,9 +206,14 @@ class SelfPlayWorker:
 
     def __init__(self, game, games: int, mcts_searches: int, mcts_batch_size: int, steps_before_tau_0: int,
                  replay_steps: int = 4, min_replay: int = 5000, seed: int = 0, node_capacity: Optional[int] = None,
-                 compact_tree: bool = False):
+                 compact_tree: bool = False, resign: Union[None, float, str] = None, resign_playthrough: float = 0.1):
         """``compact_tree``: drop unreachable nodes after every move (CARO_FLAG_COMPACT_TREE: bit-identical play, arenas of a
-        few moves' searches instead of a whole game's -- what large boards need)."""
+        few moves' searches instead of a whole game's -- what large boards need).
+        ``resign`` (extension, default off): None plays every game to its end; a float is a fixed resignation threshold
+        with ``resign_playthrough`` of the games played through and logged; "auto" logs every game and never resigns
+        until the log (the last RESIGN_WINDOW games of every rank, summed over ranks) yields a threshold whose
+        false-positive rate is <= 5 %, then resigns at that threshold with ``resign_playthrough`` played through.  The
+        calibration runs after every step on every rank (one all-reduce)."""
         self.game, self.games = game, int(games)
         self.searches, self.batch, self.tau_plies = mcts_searches, mcts_batch_size, steps_before_tau_0
         max_plies = _max_plies(game)
@@ -162,6 +225,20 @@ class SelfPlayWorker:
         self.engine = SelfPlayEngine(game, self.games, trees_per_game=1, max_batch=mcts_batch_size, node_capacity=cap,
                                      replay_capacity=self.replay_capacity, seed=seed, compact_tree=compact_tree)
         self._last = self.engine.counters()
+        if not (resign is None or resign == "auto" or isinstance(resign, (int, float))):
+            raise ValueError("resign must be None, a threshold or 'auto'")
+        self.resign = resign
+        self.resign_playthrough = float(resign_playthrough)
+        self.resign_threshold: Optional[float] = None
+        self._resign_window = collections.deque(maxlen=RESIGN_WINDOW)
+        self._resign_cursor = 0
+        self._resign_last = {"resigned": 0, "logged": 0}
+        self._resign_stats: Dict[str, Optional[float]] = {}
+        if resign == "auto":
+            self.engine.set_resign(-1.0, 1.0)  # log only until calibrated
+        elif resign is not None:
+            self.resign_threshold = float(resign)
+            self.engine.set_resign(self.resign_threshold, self.resign_playthrough)
 
     def play_step(self, net: "model.DeviceNet") -> Dict[str, int]:
         """Every game slot plays one fresh game to its end with ``net`` on both sides; the finished games' positions go
@@ -174,8 +251,41 @@ class SelfPlayWorker:
             raise RuntimeError("self-play engine reported error bits %d" % c["errors"])
         d = {k: c[k] - self._last[k] for k in c}
         self._last = c
+        if self.resign is not None:
+            self._resign_update(d)
         return {"wins": d["wins_p0"], "losses": d["wins_p1"], "draws": d["draws"], "games": d["games"], "plies": d["plies"],
                 "leaf_evals": d["leaf_evals"]}
+
+    def _resign_update(self, d: Dict[str, int]) -> None:
+        eng = self.engine
+        records, self._resign_cursor = eng.resign_log(self._resign_cursor)
+        self._resign_window.extend(records.tolist())
+        rc = eng.resign_counters()
+        resigned = rc["resigned"] - self._resign_last["resigned"]
+        logged = rc["logged"] - self._resign_last["logged"]
+        self._resign_last = rc
+        window = np.array(list(self._resign_window), dtype=SelfPlayEngine.RESIGN_RECORD_DTYPE)
+        if self.resign == "auto":
+            t, tallies = resign_threshold_over_ranks(window, device=eng.device)
+            if t != self.resign_threshold:
+                self.resign_threshold = t
+                if t is None:
+                    eng.set_resign(-1.0, 1.0)
+                else:
+                    eng.set_resign(t, self.resign_playthrough)
+        else:
+            tallies = resign_tallies(window)
+        self._resign_stats = {"threshold": self.resign_threshold, "fp_rate": _fp_rate(window, tallies, self.resign_threshold),
+                              "resigned": resigned, "logged": logged, "window": int(tallies[0, 1]),
+                              "resigned_share": resigned / d["games"] if d["games"] else 0.0,
+                              "plies_per_game": d["plies"] / d["games"] if d["games"] else 0.0}
+
+    def resign_stats(self) -> Dict[str, Optional[float]]:
+        """Resignation statistics of the last step (empty while resignation is off): the threshold in force for the next
+        step (None = not calibrated yet), its false-positive rate over the logged window (over all ranks in "auto"
+        mode), games resigned and playthrough games logged in the step, the window size, the resigned share of the
+        step's games and its plies per game."""
+        return dict(self._resign_stats)
 
     def replay_len(self) -> int:
         return self.engine.replay_live()

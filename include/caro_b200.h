@@ -205,6 +205,29 @@ typedef struct {
 enum { CARO_FLAG_VIRTUAL_LOSS = 1, CARO_FLAG_MASK_PRIORS = 2, CARO_FLAG_FRESH_TREE = 4, CARO_FLAG_RECYCLE_TREE = 8,
        CARO_FLAG_COMPACT_TREE = 16 };
 
+/* Resignation (extension, off by default; the reference plays every game to its end).  Not a flag: it is switched and
+ * tuned at run time by caro_engine_set_resign, whose parameters live in device memory (region "resign_params"), so a
+ * ply graph captured by caro_engine_play_multi reads the current values on every replay.
+ *   The rule, decided in caro_engine_advance from the root row of the mover's tree: with total = sum N[a] > 0,
+ *     v_root = (sum over a, in action order, of (double)W[a]) / total          (double adds, one double division)
+ *     v_best = (double)f32(W[best] / N[best]), best = the most visited action (lowest index on ties)
+ *     stat   = max(v_root, v_best)                                              (mover's point of view)
+ *   A game that is not a playthrough game resigns when stat < threshold: its history entry for the ply is written, the
+ *   ply is counted, no move is played (d_action_out = -1) and the game ends lost for the mover (result, win counters and
+ *   replay z as for any finished game; auto_restart re-seats the slot).  total == 0: no statistic, no resignation.
+ *   A game is a playthrough game when, at its start (caro_engine_reset, or an auto-restart), resignation is enabled and
+ *   u01d(Philox(uid, 0, 0; seed ^ 'RESG')) < playthrough.  It never resigns; it keeps each player's smallest stat
+ *   (+inf until that player has one) and, when it ends, appends one record to the log ring.
+ *   threshold = -1.0 never fires (stat >= -1 exactly): "log only".
+ *   A false positive at threshold t is a logged game in which some player with min_stat < t did not lose (won or drew).
+ * Regions: "resign_params" {int32 enabled, int32 pad, double threshold, double playthrough},
+ *          "resign_playthrough" uint8 [G] (1 = the current game is a playthrough game),
+ *          "resign_min" double [G][2] (the current playthrough game's minima per player),
+ *          "resign_log" [G] records of 24 bytes {double min_stat[2]; int32 result (player 0's view); int32 plies},
+ *                       record k in slot k % G,
+ *          "resign_counters" uint64 [2]: [0] games resigned, [1] playthrough games logged (= the log cursor).
+ * They follow every other region, so no other offset depends on them. */
+
 /* Bytes of device workspace the engine needs; the caller allocates it (e.g. a torch uint8 CUDA
  * tensor) and keeps it alive for the life of the handle. */
 size_t caro_engine_workspace_bytes(const caro_engine_config* cfg);
@@ -305,6 +328,12 @@ int caro_engine_replay_gather(caro_engine* e, const int64_t* d_entries, const in
 /* enable: 0 = off, 1 = network kernel only (2 events per minibatch), 2 = all four phases. */
 int caro_engine_profile(caro_engine* e, int enable);
 int caro_engine_profile_read(caro_engine* e, double h_ms[5], uint64_t* h_launches, void* stream);
+
+/* Resignation parameters (the rule beside CARO_FLAG_*), enqueued on `stream` and read by every later
+ * advance; the playthrough share applies to games that start after the call.  enable = 0 switches resignation off.
+ * Returns CARO_E_ARG (before touching the device) for a null handle, a threshold that is NaN or outside [-1, 1], or a
+ * playthrough share that is NaN or outside [0, 1]. */
+int caro_engine_set_resign(caro_engine* e, int enable, double threshold, double playthrough, void* stream);
 
 /* Host copies of the 64-bit counters (synchronises `stream`): [0] leaf evaluations, [1] finished
  * games, [2] plies played, [3] wins of player 0, [4] wins of player 1, [5] draws, [6] descents,
