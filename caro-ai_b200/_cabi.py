@@ -62,6 +62,7 @@ _SIGNATURES = {
     "caro_engine_replay_gather": (C.c_int, [_P, _P, _P, C.c_int64, _P, _P, _P, _P]),
     "caro_engine_counters": (C.c_int, [_P, C.POINTER(C.c_uint64 * 8), _P]),
     "caro_engine_set_resign": (C.c_int, [_P, C.c_int, C.c_double, C.c_double, _P]),
+    "caro_engine_set_solver": (C.c_int, [_P, C.c_int, _P]),
 }
 
 _lib = None

@@ -77,6 +77,7 @@ struct caro_engine {
   cudaEvent_t sync_a = nullptr, sync_b = nullptr;  // cross-stream hand-offs (pair pipeline)
   bool lean_tree = false;  // set while the parts pipeline issues launches: prefer tree kernels with few warps
   unsigned long long serial = 0;  // unique per created engine (keys the cached ply graph; heap addresses are reused)
+  int solver_players = 0;  // the mask last enqueued by caro_engine_set_solver: picks the select / back-up instances
   size_t next_event() {
     if (events_used == events.size()) {
       cudaEvent_t ev;
@@ -150,6 +151,9 @@ void build_view(Carver& c, const Dims& dm, char* base, View<Board>* v) {
   CARVE(resign_min, "resign_min", double, dm.G, 2);
   CARVE(resign_log, "resign_log", ResignRecord, dm.G);
   CARVE(resign_ctr, "resign_counters", unsigned long long, RCTR_COUNT);
+  // MCTS solver (extension): after the resignation regions, for the same reason
+  CARVE(solver_params, "solver_params", SolverParams, 1);
+  CARVE(solver_ctr, "solver_counters", unsigned long long, SCTR_COUNT);
 #undef CARVE
 }
 
@@ -190,10 +194,33 @@ int fill_dims(const caro_engine_config* cfg, Dims* dm, int* max_plies) {
 
 inline cudaStream_t S(void* s) { return reinterpret_cast<cudaStream_t>(s); }
 
+// the select instance for the action count and the number of descents
+template <class R, bool SOLVER, class Board>
+void launch_select_kernel(const View<Board>& v, const R& rules, const Dims& dm, const SearchParams& sp, int batch,
+                          const double* src, cudaStream_t st) {
+  const long long groups = (long long)dm.G * batch;
+  auto grid = [&](int gw) { return (unsigned)((groups * gw + 255) / 256); };
+  const int A = dm.A;
+#define SELECT(GW, APL) select_kernel<R, GW, APL, SOLVER><<<grid(GW), 256, 0, st>>>(v, rules, dm, sp, batch, src)
+  // more descents than the GPU holds at once (5 blocks of 90-register threads per SM): the 72-register build keeps 7 blocks
+  // per SM resident (-20 % at 16 k games, -12 % at 64 k; a few spilled words; CARO_SELECT_DENSE=0 switches it off)
+  static const bool dense = !(getenv("CARO_SELECT_DENSE") && atoi(getenv("CARO_SELECT_DENSE")) == 0);
+  if (A <= 8 && dense && groups > 128ll * 5 * 148) select_thread_dense_kernel<R, 2, 7, SOLVER><<<(unsigned)((groups + 127) / 128), 128, 0, st>>>(v, rules, dm, sp, batch, src);
+  else if (A <= 8) select_thread_kernel<R, 2, SOLVER><<<(unsigned)((groups + 127) / 128), 128, 0, st>>>(v, rules, dm, sp, batch, src);
+  else if constexpr (!std::is_same<R, C4Rules>::value) {  // lane-group kernels: m,n,k boards only (Connect4 has 7 actions)
+    if (A <= 16) select_thread_kernel<R, 4, SOLVER><<<(unsigned)((groups + 127) / 128), 128, 0, st>>>(v, rules, dm, sp, batch, src);
+    else if (A <= 32) SELECT(32, 1);
+    else if (A <= 64) SELECT(32, 2);
+    else if (A <= 128) SELECT(32, 4);
+    else SELECT(32, 8);
+  }
+#undef SELECT
+}
+
 // group width / actions per lane for the select and noise kernels
 template <class R, class Board>
 int launch_select(const View<Board>& v, const R& rules, const Dims& dm, const SearchParams& sp, int batch, int mb,
-                  const double* noise, double* noise_out, cudaStream_t st, int phase = 0) {
+                  const double* noise, double* noise_out, cudaStream_t st, int phase, bool solver) {
   // phase 0: noise (unless injected) + select; 1: only generate the Philox noise of minibatch `mb` into v.noise;
   // 2: only select, reading v.noise as generated by an earlier phase-1 call (the self-play pipeline issues the
   // noise of minibatch i+1 underneath the network pass of minibatch i: it depends on (uid, ply, i) alone)
@@ -222,20 +249,8 @@ int launch_select(const View<Board>& v, const R& rules, const Dims& dm, const Se
     else select_vl_kernel<R><<<(unsigned)((dm.G + 63) / 64), 64, 0, st>>>(v, rules, dm, sp, batch, src);
     return caro_check_launch("select_vl_kernel");
   }
-#define SELECT(GW, APL) select_kernel<R, GW, APL><<<grid(GW), 256, 0, st>>>(v, rules, dm, sp, batch, src)
-  // more descents than the GPU holds at once (5 blocks of 90-register threads per SM): the 72-register build keeps 7 blocks
-  // per SM resident (-20 % at 16 k games, -12 % at 64 k; a few spilled words; CARO_SELECT_DENSE=0 switches it off)
-  static const bool dense = !(getenv("CARO_SELECT_DENSE") && atoi(getenv("CARO_SELECT_DENSE")) == 0);
-  if (A <= 8 && dense && groups > 128ll * 5 * 148) select_thread_dense_kernel<R, 2, 7><<<(unsigned)((groups + 127) / 128), 128, 0, st>>>(v, rules, dm, sp, batch, src);
-  else if (A <= 8) select_thread_kernel<R, 2><<<(unsigned)((groups + 127) / 128), 128, 0, st>>>(v, rules, dm, sp, batch, src);
-  else if constexpr (!std::is_same<R, C4Rules>::value) {  // lane-group kernels: m,n,k boards only (Connect4 has 7 actions)
-    if (A <= 16) select_thread_kernel<R, 4><<<(unsigned)((groups + 127) / 128), 128, 0, st>>>(v, rules, dm, sp, batch, src);
-    else if (A <= 32) SELECT(32, 1);
-    else if (A <= 64) SELECT(32, 2);
-    else if (A <= 128) SELECT(32, 4);
-    else SELECT(32, 8);
-  }
-#undef SELECT
+  if (solver) launch_select_kernel<R, true>(v, rules, dm, sp, batch, src, st);
+  else launch_select_kernel<R, false>(v, rules, dm, sp, batch, src, st);
   return caro_check_launch("select_kernel");
 }
 
@@ -407,8 +422,10 @@ int caro_engine_select(caro_engine* e, int batch, int minibatch_index, const dou
   if (!e) return caro_fail(CARO_E_ARG, "null engine");
   if (batch <= 0 || batch > e->dm.B) return caro_fail(CARO_E_ARG, "batch exceeds max_batch");
   if (e->cfg.game == CARO_GAME_CONNECT4)
-    return launch_select<C4Rules>(e->v_c4, C4Rules(), e->dm, e->sp, batch, minibatch_index, d_noise, d_noise_out, S(stream));
-  return launch_select<MnkRules>(e->v_mnk, e->mnk, e->dm, e->sp, batch, minibatch_index, d_noise, d_noise_out, S(stream));
+    return launch_select<C4Rules>(e->v_c4, C4Rules(), e->dm, e->sp, batch, minibatch_index, d_noise, d_noise_out, S(stream), 0,
+                                  e->solver_players != 0);
+  return launch_select<MnkRules>(e->v_mnk, e->mnk, e->dm, e->sp, batch, minibatch_index, d_noise, d_noise_out, S(stream), 0,
+                                 e->solver_players != 0);
 }
 
 int caro_engine_plan(caro_engine* e, int batch, void* stream) {
@@ -433,10 +450,13 @@ int caro_engine_expand_backup(caro_engine* e, int batch, const float* d_probs, c
   if (!e || !d_probs || !d_values) return caro_fail(CARO_E_ARG, "null argument");
   const unsigned grid = (unsigned)(((long long)e->dm.G * 32 + 127) / 128);
   const bool c4 = e->cfg.game == CARO_GAME_CONNECT4;
-#define LAUNCH_EB(BK)                                                                                               \
-  do {                                                                                                              \
-    if (c4) expand_backup_kernel<C4Rules, BK><<<grid, 128, 0, S(stream)>>>(e->v_c4, e->dm, batch, d_probs, d_values); \
-    else expand_backup_kernel<MnkRules, BK><<<grid, 128, 0, S(stream)>>>(e->v_mnk, e->dm, batch, d_probs, d_values);  \
+  const bool sol = e->solver_players != 0;  // the proof pass lives in the SOLVER instances only
+#define LAUNCH_EB(BK)                                                                                                       \
+  do {                                                                                                                      \
+    if (c4 && sol) expand_backup_kernel<C4Rules, BK, true><<<grid, 128, 0, S(stream)>>>(e->v_c4, e->dm, batch, d_probs, d_values); \
+    else if (c4) expand_backup_kernel<C4Rules, BK, false><<<grid, 128, 0, S(stream)>>>(e->v_c4, e->dm, batch, d_probs, d_values); \
+    else if (sol) expand_backup_kernel<MnkRules, BK, true><<<grid, 128, 0, S(stream)>>>(e->v_mnk, e->dm, batch, d_probs, d_values); \
+    else expand_backup_kernel<MnkRules, BK, false><<<grid, 128, 0, S(stream)>>>(e->v_mnk, e->dm, batch, d_probs, d_values);  \
   } while (0)
   // eight lanes per game inside the parts pipeline (a quarter of the warps: +2.5 % there, where the tree kernels live in
   // the warp slots next to tower CTAs), one warp per game otherwise (20 us instead of 36 us stand-alone at 4,096 games)
@@ -444,7 +464,8 @@ int caro_engine_expand_backup(caro_engine* e, int batch, const float* d_probs, c
   // (and stand-alone from 32 k games per launch: 138 us instead of 194 us at 65,536 games -- a quarter of the warps, one wave less)
   if (batch <= 8 && e->dm.Apad <= 8 && c4 && group8 && (e->lean_tree || group8 == 2 || e->dm.G >= 32768)) {
     const unsigned g8 = (unsigned)(((long long)e->dm.G * 8 + 127) / 128);
-    expand_backup_group8_kernel<C4Rules><<<g8, 128, 0, S(stream)>>>(e->v_c4, e->dm, batch, d_probs, d_values);
+    if (sol) expand_backup_group8_kernel<C4Rules, true><<<g8, 128, 0, S(stream)>>>(e->v_c4, e->dm, batch, d_probs, d_values);
+    else expand_backup_group8_kernel<C4Rules, false><<<g8, 128, 0, S(stream)>>>(e->v_c4, e->dm, batch, d_probs, d_values);
   } else if (batch <= 8) LAUNCH_EB(8);
   else if (batch <= 16) LAUNCH_EB(16);
   else LAUNCH_EB(32);
@@ -458,8 +479,8 @@ int caro_engine_expand_backup(caro_engine* e, int batch, const float* d_probs, c
 // hand-offs are CUDA events, so that another engine's tree kernels can run underneath this engine's network pass.
 static int select_phase(caro_engine* e, int batch, int mb, int phase, cudaStream_t st) {
   if (e->cfg.game == CARO_GAME_CONNECT4)
-    return launch_select<C4Rules>(e->v_c4, C4Rules(), e->dm, e->sp, batch, mb, nullptr, nullptr, st, phase);
-  return launch_select<MnkRules>(e->v_mnk, e->mnk, e->dm, e->sp, batch, mb, nullptr, nullptr, st, phase);
+    return launch_select<C4Rules>(e->v_c4, C4Rules(), e->dm, e->sp, batch, mb, nullptr, nullptr, st, phase, e->solver_players != 0);
+  return launch_select<MnkRules>(e->v_mnk, e->mnk, e->dm, e->sp, batch, mb, nullptr, nullptr, st, phase, e->solver_players != 0);
 }
 
 // `prefetch`: 0 = noise + select as one step, 1 = minibatch i's noise was issued by the previous step, and this
@@ -766,6 +787,24 @@ int caro_engine_set_resign(caro_engine* e, int enable, double threshold, double 
   ResignParams* dst = e->cfg.game == CARO_GAME_CONNECT4 ? e->v_c4.resign_params : e->v_mnk.resign_params;
   set_resign_kernel<<<1, 1, 0, S(stream)>>>(dst, p);
   return caro_check_launch("set_resign_kernel");
+}
+
+int caro_engine_set_solver(caro_engine* e, int players, void* stream) {
+  if (!e) return caro_fail(CARO_E_ARG, "null engine");
+  if (players < 0 || players > 3) return caro_fail(CARO_E_ARG, "solver players must be a mask in 0..3");
+  if (players != 0 && (e->dm.flags & FLAG_VIRTUAL_LOSS))
+    return caro_fail(CARO_E_ARG, "the solver does not run with virtual loss");
+  if ((players == 1 || players == 2) && e->dm.tpg == 1)
+    return caro_fail(CARO_E_ARG, "a per-player solver mask needs two trees per game (one tree serves both players)");
+  SolverParams p{};
+  p.players = players;
+  SolverParams* dst = e->cfg.game == CARO_GAME_CONNECT4 ? e->v_c4.solver_params : e->v_mnk.solver_params;
+  set_solver_kernel<<<1, 1, 0, S(stream)>>>(dst, p);
+  const int rc = caro_check_launch("set_solver_kernel");
+  if (rc == CARO_OK && (players != 0) != (e->solver_players != 0))
+    caro_pipeline_forget(e->serial, 0);  // a captured ply graph holds the other select / back-up instances
+  if (rc == CARO_OK) e->solver_players = players;
+  return rc;
 }
 
 int caro_engine_counters(caro_engine* e, uint64_t h_out[8], void* stream) {

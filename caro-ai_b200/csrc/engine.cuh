@@ -14,7 +14,11 @@ enum : uint8_t { KIND_SKIP = 0, KIND_TERMINAL = 1, KIND_EXPAND = 2 };
 enum : uint8_t { ST_ACTIVE = 0, ST_FINISHED = 1 };
 enum { CTR_LEAVES = 0, CTR_GAMES, CTR_PLIES, CTR_WIN0, CTR_WIN1, CTR_DRAW, CTR_DESCENTS, CTR_ERRORS, CTR_COUNT };
 constexpr int kNetBit = (int)0x80000000u;   // flag bit inside an N word
-constexpr int kCountMask = 0x7fffffff;
+constexpr int kCountMask = 0x1fffffff;      // visit count: bits 0..28 (counts stay far below 2^29)
+// Solver (extension): bits 29-30 of an N word hold the edge's proof for the side to move at the node
+constexpr int kProofShift = 29;
+constexpr int kProofMask = 3 << kProofShift;
+enum : int { PROOF_UNKNOWN = 0, PROOF_WIN = 1, PROOF_LOSS = 2, PROOF_DRAW = 3 };
 enum : unsigned long long { ERR_ARENA_FULL = 1ull, ERR_REPLAY_OVERRUN = 2ull, ERR_ILLEGAL_ACTION = 4ull };
 
 struct alignas(16) HashSlot {
@@ -84,6 +88,14 @@ struct alignas(8) ResignRecord {
 static_assert(sizeof(ResignRecord) == 24, "resign log records are 24 bytes");
 enum { RCTR_RESIGNED = 0, RCTR_LOGGED, RCTR_COUNT };
 
+// MCTS solver (extension, off by default; include/caro_b200.h caro_engine_set_solver).  Read by the select, expand +
+// back-up, root policy and advance kernels at run time, like the resignation parameters.
+struct alignas(8) SolverParams {
+  int32_t players;  // bit p: searches whose root player is p use the solver
+  int32_t pad_;
+};
+enum { SCTR_STOPPED = 0, SCTR_PROVEN, SCTR_COUNT };
+
 struct SearchParams {
   double c_puct, alpha, explore;
   uint32_t seed_lo, seed_hi;
@@ -95,7 +107,7 @@ struct View {
   // One record of RS = 4 * Apad words per node, rows [N | W | P | C]; the four pointers below address row 0 / 1 / 2 / 3
   // of record 0, so X[(nb + node) * RS + a] is entry a of row X.  A Connect4 record is one aligned 128-byte line: a
   // descent step reads exactly that line, a back-up touches its first 64 bytes, an expansion writes it whole.
-  int32_t* N;          // visit counts (lib/mcts.py:30) in bits 0..30; bit 31 (kNetBit): W(s,a) has absorbed a float32
+  int32_t* N;          // visit counts (lib/mcts.py:30) in bits 0..28; bits 29-30: solver proof; bit 31 (kNetBit): W(s,a) has absorbed a float32
                        // network value (numpy promotion state of the reference's python-float / np.float32 sums)
   float* W;            // total value (lib/mcts.py:32).  The mean value Q (lib/mcts.py:34) is not stored: it always
                        // equals f32(W / N) (0 while N == 0) and is recomputed where it is read
@@ -146,6 +158,9 @@ struct View {
   double* resign_min;            // [G][2] smallest statistic per player of the current playthrough game
   ResignRecord* resign_log;      // [G] ring of finished playthrough games (slot = cursor % G)
   unsigned long long* resign_ctr;  // [RCTR_COUNT] games resigned, playthrough games logged (= log cursor)
+  // ---- MCTS solver (extension) ------------------------------------------------------------------
+  SolverParams* solver_params;     // [1]
+  unsigned long long* solver_ctr;  // [SCTR_COUNT] descents stopped at a proven node, edges proven
 };
 
 }  // namespace caro

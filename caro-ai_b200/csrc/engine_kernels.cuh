@@ -108,6 +108,19 @@ struct RulesTraits<C4Rules> {
   static constexpr bool kHasKeyHi = false;
 };
 
+// ---------------------------------------------------------------------------------- MCTS solver (extension)
+// A node's status from its legal edges' proofs: WIN if one is WIN, LOSS if all are LOSS, DRAW if all are proven, none is
+// WIN and one is DRAW.  A node always has a legal edge (terminal positions never become nodes).
+__device__ __forceinline__ int proof_status(bool any_win, bool all_loss, bool all_proven, bool any_draw) {
+  return any_win ? PROOF_WIN : (all_loss ? PROOF_LOSS : ((all_proven && any_draw) ? PROOF_DRAW : PROOF_UNKNOWN));
+}
+// value of a proven node for its mover, and the proof of the edge into a node of status `st` for the mover above
+__device__ __forceinline__ float proof_value(int st) { return st == PROOF_WIN ? 1.0f : (st == PROOF_LOSS ? -1.0f : 0.0f); }
+__device__ __forceinline__ int proof_negate(int st) { return st == PROOF_WIN ? PROOF_LOSS : (st == PROOF_LOSS ? PROOF_WIN : st); }
+// is the solver on for searches of game g (root player `who`)?
+template <class Board>
+__device__ __forceinline__ bool solver_on(const View<Board>& e, int who) { return (e.solver_params->players >> who) & 1; }
+
 // ------------------------------------------------------------------------------- Dirichlet noise
 // np.random.dirichlet([alpha] * A) for every descent of the coming minibatch (lib/mcts.py:56), Philox-addressed by
 // (seed, game uid, ply, side to move, minibatch, descent, action).  Kept out of select_kernel: the sampler's
@@ -149,15 +162,15 @@ noise_kernel(const uint64_t* __restrict__ uid_g, const int32_t* __restrict__ ply
 
 // ---------------------------------------------------------------------------------- select
 // One group of GW lanes per descent, APL actions per lane (action = lane + i*GW).
-template <class R, int GW, int APL>
-__global__ void __launch_bounds__(256, (APL == 1 && sizeof(typename R::Board) <= 16) ? 7 : (APL == 8 ? 2 : 1))
-select_kernel(View<typename R::Board> e, R rules, Dims dm, SearchParams sp, int batch,
-              const double* __restrict__ noise_in) {
+// SOLVER (extension): the body reads the proofs of the N words when the solver is on for the game's root player.  A
+// descent that reaches a proven node below the root stops there as a terminal (value +1 / -1 / 0 for the node's mover),
+// a proven root makes no descent at all, and LOSS edges are left out of the argmax.  (The lowest WIN edge of a node with
+// a WIN edge, and the argmax over LOSS edges when all legal edges are LOSS, are never taken here: such a node is proven.)
+template <class R, int GW, int APL, bool SOLVER>
+__device__ __forceinline__ void select_group_body(const View<typename R::Board>& e, const R& rules, const Dims& dm,
+                                                  const SearchParams& sp, int batch, const double* __restrict__ noise_in,
+                                                  long long gthread) {
   using Board = typename R::Board;
-  const long long gthread = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  if (gthread == 0) {
-    *e.leaf_count = 0;  // plan_kernel (next launch on the stream) accumulates into it
-  }
   const long long grp = gthread / GW;
   if (grp >= (long long)dm.G * batch) return;
   const int gl = threadIdx.x & (GW - 1);
@@ -171,6 +184,7 @@ select_kernel(View<typename R::Board> e, R rules, Dims dm, SearchParams sp, int 
   const int A = dm.A;
   Board s = e.root_board[g];
   int who = e.root_player[g];
+  const bool sol = SOLVER && solver_on(e, who);
   const int tree = g * dm.tpg + (dm.tpg == 2 ? who : 0);
   const uint32_t gen = e.tree_gen[tree];
   const HashSlot* ht = e.ht + (size_t)tree * dm.hash_cap;
@@ -213,6 +227,34 @@ select_kernel(View<typename R::Board> e, R rules, Dims dm, SearchParams sp, int 
     }
 #pragma unroll
     for (int off = GW / 2; off > 0; off >>= 1) sum_n += __shfl_xor_sync(gmask, sum_n, off);
+    unsigned loss_m = 0u;  // bit i: my action gl + i * GW is a LOSS edge (solver)
+    if (sol) {
+      bool win = false, all_loss = true, all_proven = true, draw = false;
+#pragma unroll
+      for (int i = 0; i < APL; ++i) {
+        const int a = gl + i * GW;
+        if (a < A && rules.legal(s, a)) {
+          const int pf = (e.N[row + a] >> kProofShift) & 3;
+          win = win || pf == PROOF_WIN;
+          draw = draw || pf == PROOF_DRAW;
+          all_loss = all_loss && pf == PROOF_LOSS;
+          all_proven = all_proven && pf != PROOF_UNKNOWN;
+          loss_m |= (pf == PROOF_LOSS ? 1u : 0u) << i;
+        }
+      }
+      const int st = proof_status(__any_sync(gmask, win), __all_sync(gmask, all_loss), __all_sync(gmask, all_proven),
+                                  __any_sync(gmask, draw));
+      if (st != PROOF_UNKNOWN) {
+        if (depth == 0) {  // proven root: no descent
+          if (gl == 0) store_desc_skip(e.desc + di);
+          return;
+        }
+        kind = KIND_TERMINAL;
+        term_value = proof_value(st);
+        if (gl == 0) atomicAdd(e.solver_ctr + SCTR_STOPPED, 1ull);
+        break;
+      }
+    }
 
     double best = -INFINITY;
     int best_a = 0x7fffffff;
@@ -228,7 +270,7 @@ select_kernel(View<typename R::Board> e, R rules, Dims dm, SearchParams sp, int 
 #pragma unroll
       for (int i = 0; i < APL; ++i) {
         const int a = gl + i * GW;
-        if (a < A && rules.legal(s, a)) {
+        if (a < A && rules.legal(s, a) && !((loss_m >> i) & 1u)) {
           const double pn = __dadd_rn((double)__fmul_rn(keep_f, p_loc[i]), __dmul_rn(sp.explore, z[i]));
           const double u = __ddiv_rn(__dmul_rn(__dmul_rn(sp.c_puct, pn), sq), (double)(1 + n_loc[i]));
           // Q keeps python-float (float64) precision until a float32 value touched W(s,a)
@@ -250,7 +292,7 @@ select_kernel(View<typename R::Board> e, R rules, Dims dm, SearchParams sp, int 
 #pragma unroll
       for (int i = 0; i < APL; ++i) {
         const int a = gl + i * GW;
-        if (a < A && rules.legal(s, a)) {
+        if (a < A && rules.legal(s, a) && !((loss_m >> i) & 1u)) {
           const float t = __fdiv_rn(__fmul_rn(__fmul_rn(c_f, p_loc[i]), sq), (float)(1 + n_loc[i]));
           const float q = n_loc[i] > 0 ? __fdiv_rn(w_loc[i], (float)n_loc[i]) : 0.0f;  // value_avg, lib/mcts.py:244
           const double sc = (double)__fadd_rn(q, t);
@@ -303,11 +345,24 @@ select_kernel(View<typename R::Board> e, R rules, Dims dm, SearchParams sp, int 
   if (gl == 0) store_desc(e.desc + di, kind, who, depth, term_value, key, s);
 }
 
+// SOLVER = false is the reference's search.  The host launches the SOLVER instance while the engine's solver mask is
+// non-zero (a run-time branch on the mask would cost the plain instances registers); it then checks the mask per game.
+template <class R, int GW, int APL, bool SOLVER>
+__global__ void __launch_bounds__(256, (APL == 1 && sizeof(typename R::Board) <= 16) ? 7 : (APL == 8 ? 2 : 1))
+select_kernel(View<typename R::Board> e, R rules, Dims dm, SearchParams sp, int batch,
+              const double* __restrict__ noise_in) {
+  const long long gthread = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (gthread == 0) {
+    *e.leaf_count = 0;  // plan_kernel (next launch on the stream) accumulates into it
+  }
+  select_group_body<R, GW, APL, SOLVER>(e, rules, dm, sp, batch, noise_in, gthread);
+}
+
 // Thread-per-descent variant for small action spaces (A <= 16: Connect4, 3x3 / 4x4 boards).  The board update,
 // key and transposition probe are scalar work; with one lane-group per descent they are replicated on every
 // lane and the kernel becomes issue-bound (ncu: 12.7 M warp instructions per launch).  Here each lane owns a whole
 // descent and loops over the <= 16 actions; the arithmetic and its order are identical to select_kernel.
-template <class R, int ROWV>  // ROWV = Apad / 4 = number of 16-byte vectors per row
+template <class R, int ROWV, bool SOLVER>  // ROWV = Apad / 4 = number of 16-byte vectors per row; SOLVER: as select_group_body
 __device__ __forceinline__ void select_thread_body(const View<typename R::Board>& e, const R& rules, const Dims& dm,
                                                    const SearchParams& sp, int batch, const double* __restrict__ noise_in,
                                                    long long grp) {
@@ -322,6 +377,7 @@ __device__ __forceinline__ void select_thread_body(const View<typename R::Board>
   const int A = dm.A;
   Board s = e.root_board[g];
   int who = e.root_player[g];
+  const bool sol = SOLVER && solver_on(e, who);
   const int tree = g * dm.tpg + (dm.tpg == 2 ? who : 0);
   const uint32_t gen = e.tree_gen[tree];
   const HashSlot* ht = e.ht + (size_t)tree * dm.hash_cap;
@@ -350,7 +406,33 @@ __device__ __forceinline__ void select_thread_body(const View<typename R::Board>
       c_loc[4 * v] = cv.x; c_loc[4 * v + 1] = cv.y; c_loc[4 * v + 2] = cv.z; c_loc[4 * v + 3] = cv.w;
     }
     unsigned net_bits = 0u;  // bit a: W(s,a) has absorbed a float32 value (bit 31 of the N word)
+    unsigned loss_m = 0u;    // bit a: a LOSS edge (solver)
     int sum_n = 0;
+    if (sol) {
+      bool win = false, all_loss = true, all_proven = true, draw = false;
+#pragma unroll
+      for (int a = 0; a < ROWV * 4; ++a) {
+        if (a < A && rules.legal(s, a)) {
+          const int pf = (n_loc[a] >> kProofShift) & 3;
+          win = win || pf == PROOF_WIN;
+          draw = draw || pf == PROOF_DRAW;
+          all_loss = all_loss && pf == PROOF_LOSS;
+          all_proven = all_proven && pf != PROOF_UNKNOWN;
+          loss_m |= (pf == PROOF_LOSS ? 1u : 0u) << a;
+        }
+      }
+      const int st = proof_status(win, all_loss, all_proven, draw);
+      if (st != PROOF_UNKNOWN) {
+        if (depth == 0) {  // proven root: no descent
+          store_desc_skip(e.desc + di);
+          return;
+        }
+        kind = KIND_TERMINAL;
+        term_value = proof_value(st);
+        atomicAdd(e.solver_ctr + SCTR_STOPPED, 1ull);
+        break;
+      }
+    }
 #pragma unroll
     for (int a = 0; a < ROWV * 4; ++a) {
       net_bits |= (n_loc[a] < 0 ? 1u : 0u) << a;
@@ -364,7 +446,7 @@ __device__ __forceinline__ void select_thread_body(const View<typename R::Board>
       const double* z = noise_in + ((size_t)g * batch + j) * A;
 #pragma unroll
       for (int a = 0; a < ROWV * 4; ++a) {
-        if (a < A && rules.legal(s, a)) {
+        if (a < A && rules.legal(s, a) && !((loss_m >> a) & 1u)) {
           const double pn = __dadd_rn((double)__fmul_rn(keep_f, p_loc[a]), __dmul_rn(sp.explore, z[a]));
           const double u = __ddiv_rn(__dmul_rn(__dmul_rn(sp.c_puct, pn), sq), (double)(1 + n_loc[a]));
           // Q keeps python-float (float64) precision until a float32 value touched W(s,a)
@@ -385,7 +467,7 @@ __device__ __forceinline__ void select_thread_body(const View<typename R::Board>
       float bestf = -INFINITY;
 #pragma unroll
       for (int a = 0; a < ROWV * 4; ++a) {
-        if (a < A && rules.legal(s, a)) {
+        if (a < A && rules.legal(s, a) && !((loss_m >> a) & 1u)) {
           const float t = __fdiv_rn(__fmul_rn(__fmul_rn(c_f, p_loc[a]), sq), (float)(1 + n_loc[a]));
           const float q = n_loc[a] > 0 ? __fdiv_rn(w_loc[a], (float)n_loc[a]) : 0.0f;  // value_avg, lib/mcts.py:244
           const float sc = __fadd_rn(q, t);
@@ -423,24 +505,24 @@ __device__ __forceinline__ void select_thread_body(const View<typename R::Board>
   store_desc(e.desc + di, kind, who, depth, term_value, key, s);
 }
 
-template <class R, int ROWV>
+template <class R, int ROWV, bool SOLVER>
 __global__ void __launch_bounds__(128)
 select_thread_kernel(View<typename R::Board> e, R rules, Dims dm, SearchParams sp, int batch,
                      const double* __restrict__ noise_in) {
   const long long grp = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (grp == 0) *e.leaf_count = 0;  // plan_kernel (next launch on the stream) accumulates into it
-  select_thread_body<R, ROWV>(e, rules, dm, sp, batch, noise_in, grp);
+  select_thread_body<R, ROWV, SOLVER>(e, rules, dm, sp, batch, noise_in, grp);
 }
 
 // The same descent with at most 64 registers (8 blocks per SM instead of 5): for launches of more descents than fit the
 // GPU at once, where the number of resident warps, not the latency of one descent, sets the kernel's duration.
-template <class R, int ROWV, int BPS>
+template <class R, int ROWV, int BPS, bool SOLVER>
 __global__ void __launch_bounds__(128, BPS)
 select_thread_dense_kernel(View<typename R::Board> e, R rules, Dims dm, SearchParams sp, int batch,
                            const double* __restrict__ noise_in) {
   const long long grp = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (grp == 0) *e.leaf_count = 0;
-  select_thread_body<R, ROWV>(e, rules, dm, sp, batch, noise_in, grp);
+  select_thread_body<R, ROWV, SOLVER>(e, rules, dm, sp, batch, noise_in, grp);
 }
 
 // ------------------------------------------------------------- select with virtual loss (extension)
@@ -791,7 +873,11 @@ __device__ __forceinline__ void ht_insert_cas(HashSlot* __restrict__ ht, int cap
 //            N/W of its edge in EVERY queued path up front, then replays the queue IN ORDER in registers
 //            (float32 W sums are order dependent), forwarding values between entries that hit the same edge,
 //            and stores each distinct edge once.
-template <class R, int BK, int GW = 32>  // GW lanes per game (BK <= GW): 32 = one warp per game, 8 = four games per warp
+//   solver (SOLVER and the solver on for the root player): after phase 2, in queue order, every terminal entry proves its
+//            last edge (leaf value -1: WIN, 0: DRAW, +1: LOSS, for the edge's mover) and walks up its own path while the
+//            node above is proven, setting the next edge to the negated status.  The order decides which parent of a
+//            transposition learns first.
+template <class R, int BK, int GW = 32, bool SOLVER = false>  // GW lanes per game (BK <= GW): 32 = one warp per game, 8 = four games per warp
 __device__ __forceinline__ void expand_backup_body(const View<typename R::Board>& e, const Dims& dm, int batch,
                                                    const float* __restrict__ probs, const float* __restrict__ values, int g,
                                                    int lane32) {
@@ -922,24 +1008,61 @@ __device__ __forceinline__ void expand_backup_body(const View<typename R::Board>
       }
     }
   }
+  if (SOLVER && solver_on(e, who0)) {
+    __syncwarp(gmask);  // phase 2's N words are visible to the whole group
+    unsigned long long proven = 0ull;
+    for (int q = 0; q < qn; ++q) {
+      if (__shfl_sync(gmask, my_kind, gbase + q) != KIND_TERMINAL) continue;
+      const int di = __shfl_sync(gmask, my_di, gbase + q);
+      const int len = __shfl_sync(gmask, my_len, gbase + q);
+      const float v = __shfl_sync(gmask, my_val, gbase + q);
+      int st = v < 0.0f ? PROOF_WIN : (v > 0.0f ? PROOF_LOSS : PROOF_DRAW);
+      for (int i = len - 1; i >= 0; --i) {
+        const uint32_t pe = e.d_path[(d0 + di) * dm.max_depth + i];
+        const size_t row = (nb + (size_t)(pe >> 8)) * dm.RS;
+        if (lane == 0) {
+          const int old = e.N[row + (pe & 0xffu)];
+          proven += (old & kProofMask) ? 0ull : 1ull;
+          e.N[row + (pe & 0xffu)] = (old & ~kProofMask) | (st << kProofShift);
+        }
+        __syncwarp(gmask);
+        const typename R::Board b = e.node_board[nb + (pe >> 8)];
+        bool win = false, all_loss = true, all_proven = true, draw = false;
+        for (int a = lane; a < dm.A; a += GW) {
+          if (R{}.legal(b, a)) {
+            const int pf = (e.N[row + a] >> kProofShift) & 3;
+            win = win || pf == PROOF_WIN;
+            draw = draw || pf == PROOF_DRAW;
+            all_loss = all_loss && pf == PROOF_LOSS;
+            all_proven = all_proven && pf != PROOF_UNKNOWN;
+          }
+        }
+        const int ns = proof_status(__any_sync(gmask, win), __all_sync(gmask, all_loss), __all_sync(gmask, all_proven),
+                                    __any_sync(gmask, draw));
+        if (ns == PROOF_UNKNOWN) break;
+        st = proof_negate(ns);
+      }
+    }
+    if (lane == 0 && proven) atomicAdd(e.solver_ctr + SCTR_PROVEN, proven);
+  }
 }
 
-template <class R, int BK>
+template <class R, int BK, bool SOLVER>
 __global__ void __launch_bounds__(128)
 expand_backup_kernel(View<typename R::Board> e, Dims dm, int batch, const float* __restrict__ probs,
                      const float* __restrict__ values) {
-  expand_backup_body<R, BK>(e, dm, batch, probs, values, (blockIdx.x * blockDim.x + threadIdx.x) >> 5, threadIdx.x & 31);
+  expand_backup_body<R, BK, 32, SOLVER>(e, dm, batch, probs, values, (blockIdx.x * blockDim.x + threadIdx.x) >> 5, threadIdx.x & 31);
 }
 
 // Eight lanes per game (action rows of <= 8 entries, batch <= 8: Connect4): four games per warp, a quarter of the warps of
 // the warp-per-game kernel for the same work.  The tree kernels of the self-play pipeline run in the few warp slots
 // a tower CTA leaves free (+ 16 SMs of their own), where the number of warps, not the work, sets their time.
-template <class R>
+template <class R, bool SOLVER>
 __global__ void __launch_bounds__(128)
 expand_backup_group8_kernel(View<typename R::Board> e, Dims dm, int batch, const float* __restrict__ probs,
                             const float* __restrict__ values) {
   const int t = blockIdx.x * blockDim.x + threadIdx.x;
-  expand_backup_body<R, 8, 8>(e, dm, batch, probs, values, t >> 3, threadIdx.x & 31);
+  expand_backup_body<R, 8, 8, SOLVER>(e, dm, batch, probs, values, t >> 3, threadIdx.x & 31);
 }
 
 // ------------------------------------------------------------------------------ root policy
@@ -954,6 +1077,33 @@ __device__ __forceinline__ int root_node_of(const View<typename R::Board>& e, co
   const Key128 key = rules.key(e.root_board[g]);
   return ht_lookup1(e.ht + (size_t)tree * dm.hash_cap, dm.hash_cap, e.tree_gen[tree], key,
                     RulesTraits<R>::kHasKeyHi ? (e.key_hi + nb) : nullptr);
+}
+
+// Solver at the root (extension): the lowest WIN edge of a proven-WIN root (-1 = none), and whether LOSS edges are left
+// out of pi and the move (they are, unless that leaves no visit).  Without the solver for the root player: (-1, false).
+struct RootProof {
+  int win_a;
+  bool drop_loss;
+};
+template <class R>
+__device__ __forceinline__ RootProof root_proof(const View<typename R::Board>& e, const R& rules, const Dims& dm, int g,
+                                                size_t row) {
+  RootProof rp{-1, false};
+  if (!solver_on(e, e.root_player[g])) return rp;
+  const typename R::Board s = e.root_board[g];
+  long long kept = 0;
+  for (int a = dm.A - 1; a >= 0; --a) {
+    const int raw = e.N[row + a];
+    const int pf = (raw >> kProofShift) & 3;
+    if (pf == PROOF_WIN && rules.legal(s, a)) rp.win_a = a;
+    if (pf != PROOF_LOSS) kept += raw & kCountMask;
+  }
+  rp.drop_loss = kept > 0;
+  return rp;
+}
+// visit count of edge a as pi and the move see it
+__device__ __forceinline__ int pi_count(int raw, const RootProof& rp) {
+  return (rp.drop_loss && ((raw >> kProofShift) & 3) == PROOF_LOSS) ? 0 : (raw & kCountMask);
 }
 
 template <class R>
@@ -974,19 +1124,22 @@ __global__ void root_policy_kernel(View<typename R::Board> e, R rules, Dims dm, 
   }
   const size_t row = (nb + (size_t)node) * dm.RS;
   const int tau = tau_mode == 2 ? (e.ply[g] < tau_plies ? 1 : 0) : tau_mode;
+  const RootProof rp = root_proof<R>(e, rules, dm, g, row);
   long long total = 0;
   int best_n = -1, best_a = 0;
   for (int a = 0; a < A; ++a) {
-    const int n = e.N[row + a] & kCountMask;
+    const int n = pi_count(e.N[row + a], rp);
     total += n;
     if (n > best_n) {
       best_n = n;
       best_a = a;
     }
   }
+  const bool one_hot = tau == 0 || rp.win_a >= 0;
+  if (rp.win_a >= 0) best_a = rp.win_a;
   for (int a = 0; a < A; ++a) {
     const int n = e.N[row + a] & kCountMask;
-    if (pi) pi[(size_t)g * A + a] = tau == 0 ? (a == best_a ? 1.0 : 0.0) : __ddiv_rn((double)n, (double)total);
+    if (pi) pi[(size_t)g * A + a] = one_hot ? (a == best_a ? 1.0 : 0.0) : __ddiv_rn((double)pi_count(e.N[row + a], rp), (double)total);
     if (qout) qout[(size_t)g * A + a] = n > 0 ? __fdiv_rn(e.W[row + a], (float)n) : 0.0f;  // value_avg, lib/mcts.py:244
     if (nout) nout[(size_t)g * A + a] = n;
   }
@@ -1176,14 +1329,30 @@ __global__ void advance_kernel(View<typename R::Board> e, R rules, Dims dm, Sear
                                     sp.seed_lo ^ kStreamChoice, sp.seed_hi);
     u = u01d(r.v[0], r.v[1]);
   }
+  // solver (extension): a proven-WIN root plays its lowest WIN edge, otherwise LOSS edges leave pi and the move
+  const RootProof pf = node >= 0 ? root_proof<R>(e, rules, dm, g, row) : RootProof{-1, false};
+  if (pf.drop_loss) {
+    total = 0;
+    best_n = -1;
+    for (int a = 0; a < A; ++a) {
+      const int n = pi_count(e.N[row + a], pf);
+      total += n;
+      if (n > best_n) {
+        best_n = n;
+        best_a = a;
+      }
+    }
+  }
+  const bool one_hot = tau == 0 || total <= 0 || pf.win_a >= 0;
+  if (pf.win_a >= 0) best_a = pf.win_a;
   int action = best_a;
-  if (tau != 0 && total > 0) {
+  if (!one_hot) {
     double last = 0.0;
-    for (int a = 0; a < A; ++a) last = __dadd_rn(last, __ddiv_rn((double)(e.N[row + a] & kCountMask), (double)total));
+    for (int a = 0; a < A; ++a) last = __dadd_rn(last, __ddiv_rn((double)pi_count(e.N[row + a], pf), (double)total));
     double c = 0.0;
     action = A - 1;
     for (int a = 0; a < A; ++a) {
-      c = __dadd_rn(c, __ddiv_rn((double)(e.N[row + a] & kCountMask), (double)total));
+      c = __dadd_rn(c, __ddiv_rn((double)pi_count(e.N[row + a], pf), (double)total));
       if (__ddiv_rn(c, last) > u) {
         action = a;
         break;
@@ -1198,8 +1367,8 @@ __global__ void advance_kernel(View<typename R::Board> e, R rules, Dims dm, Sear
   e.hist_player[h] = (uint8_t)who;
   for (int a = 0; a < A; ++a) {
     float p;
-    if (tau == 0 || total <= 0) p = (a == best_a) ? 1.0f : 0.0f;
-    else p = (float)__ddiv_rn((double)(e.N[row + a] & kCountMask), (double)total);
+    if (one_hot) p = (a == best_a) ? 1.0f : 0.0f;
+    else p = (float)__ddiv_rn((double)pi_count(e.N[row + a], pf), (double)total);
     e.hist_pi[h * A + a] = p;
   }
   bool won = false;
@@ -1338,6 +1507,7 @@ replay_gather_kernel(View<typename R::Board> e, R rules, Dims dm, const long lon
 // ----------------------------------------------------------------------------- resignation parameters
 // One thread: the parameters arrive by value and are stored on the stream, behind every earlier ply.
 __global__ void set_resign_kernel(ResignParams* __restrict__ dst, ResignParams p) { *dst = p; }
+__global__ void set_solver_kernel(SolverParams* __restrict__ dst, SolverParams p) { *dst = p; }
 
 // ------------------------------------------------------------------------------------- reset
 template <class R>

@@ -103,15 +103,18 @@ class SelfPlayEngine:
     def pool(self, name: str, lo: int = 0, hi: Optional[int] = None) -> torch.Tensor:
         """Rows [lo, hi) of one statistic of the node records (region "nodes": int32 [nodes, 4, Apad], rows N | W | P | C,
         csrc/engine.cuh): "N" visit counts, "W" total values, "P" priors, "C" cached child links, "f32" (bool: bit 31 of
-        the N word, W has absorbed a float32 network value) and "Q" = f32(W / N) (0 where N == 0), which the engine does
-        not store but recomputes with exactly this division wherever lib/mcts.py reads value_avg."""
+        the N word, W has absorbed a float32 network value), "proof" (the solver's edge status, bits 29-30 of the N word:
+        0 unknown, 1 win, 2 loss, 3 draw for the side to move at the node) and "Q" = f32(W / N) (0 where N == 0), which
+        the engine does not store but recomputes with exactly this division wherever lib/mcts.py reads value_avg."""
         rec = self.region("nodes")
         rows = rec[lo:rec.shape[0] if hi is None else hi]
         raw = rows[:, 0, :]
         if name == "N":
-            return raw & 0x7FFFFFFF
+            return raw & 0x1FFFFFFF
         if name == "f32":
             return raw < 0
+        if name == "proof":
+            return (raw >> 29) & 3
         if name == "W":
             return rows[:, 1, :].contiguous().view(torch.float32)
         if name == "P":
@@ -119,7 +122,7 @@ class SelfPlayEngine:
         if name == "C":
             return rows[:, 3, :]
         if name == "Q":  # IEEE float32 division on the host (numpy), the same rounding as __fdiv_rn
-            n = (raw & 0x7FFFFFFF).cpu().numpy()
+            n = (raw & 0x1FFFFFFF).cpu().numpy()
             w = rows[:, 1, :].contiguous().view(torch.float32).cpu().numpy()
             q = np.zeros_like(w)
             np.divide(w, n.astype(np.float32), out=q, where=n > 0)
@@ -276,6 +279,19 @@ class SelfPlayEngine:
         _cabi.check(_cabi.lib().caro_engine_set_resign(self.handle, 1 if enable else 0, float(threshold) if enable else -1.0,
                                                        float(playthrough), self._stream()))
 
+    # ------------------------------------------------------------------ MCTS solver (extension)
+    def set_solver(self, players: int):
+        """MCTS solver (extension, off by default; include/caro_b200.h caro_engine_set_solver): bit p of ``players`` makes
+        the searches whose root player is p prove wins, losses and draws in the tree, stop descents at proven nodes and
+        keep proven-losing moves out of pi and the move.  0 switches it off; 1 and 2 need two trees per game.  Enqueued on
+        the current stream."""
+        _cabi.check(_cabi.lib().caro_engine_set_solver(self.handle, int(players), self._stream()))
+
+    def solver_counters(self) -> Dict[str, int]:
+        """{"stopped": descents stopped at a proven node, "proven": edges proven}."""
+        c = self.region("solver_counters").cpu().numpy()
+        return {"stopped": int(c[0]), "proven": int(c[1])}
+
     RESIGN_RECORD_DTYPE = np.dtype([("min_stat", np.float64, (2,)), ("result", np.int32), ("plies", np.int32)])
 
     def resign_log(self, start: int = 0) -> Tuple[np.ndarray, int]:
@@ -307,7 +323,8 @@ class SelfPlayEngine:
         return self.game.states_from_boards(boards), [int(p) for p in self.region("root_player").cpu().numpy()]
 
     def export_tree(self, tree: int) -> Dict[int, dict]:
-        """{state_int: {"N","W","Q","P","f32"}} of one arena -- the dict view of lib/mcts.py:29-36."""
+        """{state_int: {"N","W","Q","P","f32","proof"}} of one arena -- the dict view of lib/mcts.py:29-36, plus the
+        solver's edge status ("proof", see ``pool``)."""
         n_nodes = int(self.region("node_count")[tree].item())
         cap = self.cfg.node_capacity
         lo, hi = tree * cap, tree * cap + n_nodes
@@ -317,12 +334,14 @@ class SelfPlayEngine:
         Q = self.pool("Q", lo, hi)[:, :A].numpy()
         P = self.pool("P", lo, hi)[:, :A].cpu().numpy()
         F = self.pool("f32", lo, hi)[:, :A].cpu().numpy()
+        PF = self.pool("proof", lo, hi)[:, :A].cpu().numpy()
         boards = self.region("node_board")[lo:hi].cpu().numpy().view(np.uint64)
         states = self.game.states_from_boards(boards)
         out = {}
         for i, s in enumerate(states):
             f32 = [bool(F[i, a]) for a in range(A)]
-            out[s] = {"N": N[i].tolist(), "W": W[i].copy(), "Q": Q[i].copy(), "P": P[i].copy(), "f32": f32}
+            out[s] = {"N": N[i].tolist(), "W": W[i].copy(), "Q": Q[i].copy(), "P": P[i].copy(), "f32": f32,
+                      "proof": PF[i].tolist()}
         return out
 
     def replay_cursor(self) -> int:

@@ -36,8 +36,11 @@ EXPLORE = 0.25
 
 class MCTS:
     def __init__(self, game, node_capacity: int = 1 << 16, max_batch: int = 32, seed: int = 0,
-                 noise_fn: Optional[Callable[[int, int], np.ndarray]] = None):
-        """``noise_fn(batch, actions) -> float64 [batch, actions]`` injects the Dirichlet draws (tests)."""
+                 noise_fn: Optional[Callable[[int, int], np.ndarray]] = None, solver: bool = False):
+        """``noise_fn(batch, actions) -> float64 [batch, actions]`` injects the Dirichlet draws (tests).
+        ``solver`` (extension, default off): the MCTS solver (``SelfPlayEngine.set_solver``) for both players of the
+        shared tree; ``proof`` then shows which edges it proved."""
+        self.solver = bool(solver)
         self.c_puct = C_PUCT
         self.precision = "auto"  # nn.Module nets: one-pass bf16 tower while it holds 1e-3 on probe positions, else bf16x3
         self.game = game
@@ -56,6 +59,8 @@ class MCTS:
             self._engine = SelfPlayEngine(self.game, 1, trees_per_game=1, max_batch=self._cfg["max_batch"],
                                           node_capacity=self._cfg["node_capacity"], c_puct=self.c_puct, alpha=ALPHA,
                                           explore=EXPLORE, seed=self._cfg["seed"])
+            if self.solver:
+                self._engine.set_solver(3)
         return self._engine
 
     @staticmethod
@@ -197,13 +202,14 @@ class MCTS:
     def _export(self) -> Dict[str, dict]:
         if self._overlay is not None:
             return self._overlay
-        out = {"visit_count": {}, "value": {}, "value_avg": {}, "probs": {}}
+        out = {"visit_count": {}, "value": {}, "value_avg": {}, "probs": {}, "proof": {}}
         if self._engine is not None:
             for s, n in self._engine.export_tree(0).items():
                 out["visit_count"][s] = [int(x) for x in n["N"]]
                 out["value"][s] = [float(x) for x in n["W"]]
                 out["value_avg"][s] = [float(x) for x in n["Q"]]
                 out["probs"][s] = [float(x) for x in n["P"]]
+                out["proof"][s] = [int(x) for x in n["proof"]]
         return out
 
     def _set(self, name: str, value: dict) -> None:
@@ -215,6 +221,8 @@ class MCTS:
     value = property(lambda self: self._export()["value"], lambda self, v: self._set("value", v))
     value_avg = property(lambda self: self._export()["value_avg"], lambda self, v: self._set("value_avg", v))
     probs = property(lambda self: self._export()["probs"], lambda self, v: self._set("probs", v))
+    # solver extension: {state: [edge status]} with 0 unknown, 1 win, 2 loss, 3 draw for the side to move at the state
+    proof = property(lambda self: self._export().get("proof", {}))
 
     def _backup(self, value: float, states: List[int], actions: List[int]) -> None:
         """lib/mcts.py:225-246 on host-assigned statistics (the reference's own unit test drives it this way):

@@ -10,7 +10,9 @@ BOT_MCTS_BATCH_SIZE = 8  # config.py:23
 
 
 class Session:
-    def __init__(self, game, model_file, player_moves_first):
+    def __init__(self, game, model_file, player_moves_first, solver: bool = False):
+        """``solver`` (extension, default off): the bot's search proves wins, losses and draws and never plays a move it
+        has proven to lose while another is left."""
         self.game = game
         self.BOT_PLAYER = game.player_black
         self.USER_PLAYER = game.player_white
@@ -21,7 +23,7 @@ class Session:
         self.value = None
         self.player_moves_first = player_moves_first
         self.moves = []
-        self.mcts_store = mcts.MCTS(game)  # one tree for the whole session (play_session.py:20)
+        self.mcts_store = mcts.MCTS(game, solver=solver)  # one tree for the whole session (play_session.py:20)
 
     def move_player(self, move: int) -> bool:
         self.moves.append(move)

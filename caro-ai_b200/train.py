@@ -186,6 +186,9 @@ def parse_args(argv=None):
                         "from played-through games to keep wrong resignations under 5 %%)")
     p.add_argument("--resign-playthrough", type=share_option, default=0.1,
                    help="share of self-play games played through with resignation off to measure wrong resignations")
+    p.add_argument("--solver", action="store_true",
+                   help="extension: MCTS solver in the self-play searches (proven wins, losses and draws); the arena keeps "
+                        "the reference's search")
     p.add_argument("--evaluate-every", type=int, default=cfg.EVALUATE_EVERY_STEP, help="arena evaluation period in steps")
     p.add_argument("--blocks", type=int, default=5, choices=range(1, 21), metavar="{1..20}",
                    help="residual blocks of the network (reference: 5)")
@@ -215,7 +218,8 @@ def main(argv=None):
     bucket = D.FlatGradients(net.parameters())
     worker = SelfPlayWorker(game, args.games, cfg.MCTS_SEARCHES, cfg.MCTS_BATCH_SIZE, cfg.STEPS_BEFORE_TAU_0,
                             replay_steps=args.replay_steps, min_replay=cfg.REPLAY_BUFFER, seed=1000003 * rank + 17,
-                            compact_tree=args.compact_tree, resign=args.resign, resign_playthrough=args.resign_playthrough)
+                            compact_tree=args.compact_tree, resign=args.resign, resign_playthrough=args.resign_playthrough,
+                            solver=args.solver)
     step_idx = best_idx = 0
     with TBMeanTracker(writer, batch_size=10) as tb:
         while args.max_steps == 0 or step_idx < args.max_steps:

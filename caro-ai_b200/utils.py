@@ -93,7 +93,7 @@ def run_to_completion(eng: SelfPlayEngine, dn1, dn2, steps_before_tau_0: int, mc
 def play_games_batched(game, n_games: int, net1, net2, steps_before_tau_0: int, mcts_searches: int,
                        mcts_batch_size: int, replay_buffer: Optional[collections.deque] = None,
                        net1_plays_first: Optional[bool] = None, trees_per_game: int = 2, node_capacity: Optional[int] = None,
-                       seed: int = 0) -> Dict[str, int]:
+                       seed: int = 0, solver: Union[None, bool, Tuple[bool, bool]] = None) -> Dict[str, int]:
     """``n_games`` independent ``play_game`` runs advanced in lock-step on the GPU (fresh trees per game =
     the ``mcts_stores=None`` semantics of play.py when ``trees_per_game=2``).  Returns the W/L/D tallies from
     net1's point of view plus counters; finished games' ``(state, player, probs, z)`` tuples are appended to
@@ -103,12 +103,23 @@ def play_games_batched(game, n_games: int, net1, net2, steps_before_tau_0: int, 
     reproduces the fp32 priors / values within 1e-3 on probe positions, the split-precision tower otherwise.
 
     Two different networks require lock-step plies, so each half of the games gets a fixed first player when
-    ``net1_plays_first`` is None (the reference draws it per game: same distribution, lib/utils.py:66)."""
+    ``net1_plays_first`` is None (the reference draws it per game: same distribution, lib/utils.py:66).
+
+    ``solver`` (extension, default off): True runs the MCTS solver for both sides, a pair (net1's, net2's) for each side
+    on its own (two trees per game); the counts ``solver_stopped`` / ``solver_proven`` are added to the result."""
+    if solver is None or solver is False:
+        mask = 0
+    elif solver is True:
+        mask = 3
+    else:
+        mask = (1 if solver[0] else 0) | (2 if solver[1] else 0)
     dn1 = net1 if isinstance(net1, model.DeviceNet) else model.DeviceNet(net1, game)
     dn2 = dn1 if net2 is net1 else (net2 if isinstance(net2, model.DeviceNet) else model.DeviceNet(net2, game))
     max_plies = _max_plies(game)
     cap = node_capacity or min(1 << 16, mcts_searches * mcts_batch_size * max_plies + 8)
     totals = {"wins": 0, "losses": 0, "draws": 0, "games": 0, "plies": 0, "leaf_evals": 0}
+    if mask:
+        totals.update(solver_stopped=0, solver_proven=0)
     if dn1 is dn2:
         plans = [(n_games, -1 if net1_plays_first is None else (0 if net1_plays_first else 1))]
     elif net1_plays_first is None:
@@ -120,8 +131,14 @@ def play_games_batched(game, n_games: int, net1, net2, steps_before_tau_0: int, 
             continue
         eng = SelfPlayEngine(game, count, trees_per_game=trees_per_game, max_batch=mcts_batch_size, node_capacity=cap,
                              replay_capacity=count * max_plies if replay_buffer is not None else 0, seed=seed + part)
+        if mask:
+            eng.set_solver(mask)
         eng.reset(first_player=first)
         run_to_completion(eng, dn1, dn2, steps_before_tau_0, mcts_searches, mcts_batch_size, first)
+        if mask:
+            sc = eng.solver_counters()
+            totals["solver_stopped"] += sc["stopped"]
+            totals["solver_proven"] += sc["proven"]
         c = eng.counters()
         assert c["errors"] == 0, "engine reported errors: %d" % c["errors"]
         totals["wins"] += c["wins_p0"]
@@ -206,14 +223,17 @@ class SelfPlayWorker:
 
     def __init__(self, game, games: int, mcts_searches: int, mcts_batch_size: int, steps_before_tau_0: int,
                  replay_steps: int = 4, min_replay: int = 5000, seed: int = 0, node_capacity: Optional[int] = None,
-                 compact_tree: bool = False, resign: Union[None, float, str] = None, resign_playthrough: float = 0.1):
+                 compact_tree: bool = False, resign: Union[None, float, str] = None, resign_playthrough: float = 0.1,
+                 solver: bool = False):
         """``compact_tree``: drop unreachable nodes after every move (CARO_FLAG_COMPACT_TREE: bit-identical play, arenas of a
         few moves' searches instead of a whole game's -- what large boards need).
         ``resign`` (extension, default off): None plays every game to its end; a float is a fixed resignation threshold
         with ``resign_playthrough`` of the games played through and logged; "auto" logs every game and never resigns
         until the log (the last RESIGN_WINDOW games of every rank, summed over ranks) yields a threshold whose
         false-positive rate is <= 5 %, then resigns at that threshold with ``resign_playthrough`` played through.  The
-        calibration runs after every step on every rank (one all-reduce)."""
+        calibration runs after every step on every rank (one all-reduce).
+        ``solver`` (extension, default off): the MCTS solver for the self-play searches (``SelfPlayEngine.set_solver``):
+        proven subtrees get no more descents, and pi / the replay rows keep no visit mass on proven-losing moves."""
         self.game, self.games = game, int(games)
         self.searches, self.batch, self.tau_plies = mcts_searches, mcts_batch_size, steps_before_tau_0
         max_plies = _max_plies(game)
@@ -224,6 +244,8 @@ class SelfPlayWorker:
         self.replay_capacity = max(int(min_replay), replay_steps * self.games * max_plies)
         self.engine = SelfPlayEngine(game, self.games, trees_per_game=1, max_batch=mcts_batch_size, node_capacity=cap,
                                      replay_capacity=self.replay_capacity, seed=seed, compact_tree=compact_tree)
+        if solver:
+            self.engine.set_solver(3)
         self._last = self.engine.counters()
         if not (resign is None or resign == "auto" or isinstance(resign, (int, float))):
             raise ValueError("resign must be None, a threshold or 'auto'")

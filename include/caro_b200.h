@@ -236,8 +236,9 @@ int caro_engine_create(const caro_engine_config* cfg, void* d_workspace, size_t 
 void caro_engine_destroy(caro_engine* e);
 
 /* Offset/size of a named region of the workspace (for zero-copy views from the host language):
- * "nodes" (int32 [nodes][4][Apad]: one record per node with rows N | W | P | cached child link; bit 31 of an N word =
- * "W has absorbed a float32 network value"; Q = f32(W / N) is not stored), "node_board","node_count","root_board",
+ * "nodes" (int32 [nodes][4][Apad]: one record per node with rows N | W | P | cached child link; bits 0-28 of an N word =
+ * the visit count, bits 29-30 = the solver's proof of the edge, bit 31 = "W has absorbed a float32 network value"; Q =
+ * f32(W / N) is not stored), "node_board","node_count","root_board",
  * "root_player","status","ply",
  * "result","leaf_board","leaf_player","leaf_count",
  * "desc" (one record per descent of the current minibatch, [G][max_batch]: bytes 0 kind, 1 side to move at the leaf,
@@ -334,6 +335,29 @@ int caro_engine_profile_read(caro_engine* e, double h_ms[5], uint64_t* h_launche
  * Returns CARO_E_ARG (before touching the device) for a null handle, a threshold that is NaN or outside [-1, 1], or a
  * playthrough share that is NaN or outside [0, 1]. */
 int caro_engine_set_resign(caro_engine* e, int enable, double threshold, double playthrough, void* stream);
+
+/* MCTS solver (extension, off by default; the reference's search never knows that a position is decided).  Switched at
+ * run time by caro_engine_set_solver; the mask lives in device memory (region "solver_params"), and the engine re-captures
+ * a ply graph of caro_engine_play_multi when the solver goes from off to on or back.
+ *   Edge status, for the side to move at the edge's node, in bits 29-30 of the edge's N word ("nodes" region; the visit
+ *   count is bits 0-28): 0 UNKNOWN, 1 WIN, 2 LOSS, 3 DRAW.  A node is WIN if a legal edge is WIN, LOSS if every legal
+ *   edge is LOSS, DRAW if every legal edge is proven, none WIN and one DRAW, else UNKNOWN.
+ *   Select (solver on for the root player): a descent that reaches a proven node below the root stops there as a terminal
+ *   with value +1 / -1 / 0 for the node's mover (no network evaluation); a proven root makes no descent; LOSS edges are left
+ *   out of the argmax (a node with a WIN edge, or with LOSS edges only, is proven and never scored).
+ *   Back-up: values as without the solver; then, in back-up queue order, each terminal entry proves its last edge (leaf
+ *   value -1: WIN, 0: DRAW, +1: LOSS) and walks up its own path while the node above is proven, setting the next edge to
+ *   the negated node status.
+ *   Root policy and advance: a proven-WIN root gives pi one-hot on its lowest WIN edge whatever tau is; otherwise LOSS
+ *   edges are zeroed in the visit counts pi and the move are drawn from (tau = 0: argmax over the rest), unless that
+ *   leaves no visit.  The pi the move was drawn from is the one written to the history and the replay ring; the Philox
+ *   choice stream is unchanged.
+ * Regions: "solver_params" {int32 players, int32 pad}, "solver_counters" uint64 [2]: [0] descents stopped at a proven node,
+ *          [1] edges proven.  They follow every other region. */
+/* players: bit p = searches whose root player is p use the solver (with two trees per game: tree p).  Returns CARO_E_ARG
+ * (before touching the device) for a null handle, a mask outside 0..3, a mask of 1 or 2 on an engine with one tree per
+ * game (its tree serves both players), and a non-zero mask on a virtual-loss engine.  Enqueued on `stream`. */
+int caro_engine_set_solver(caro_engine* e, int players, void* stream);
 
 /* Host copies of the 64-bit counters (synchronises `stream`): [0] leaf evaluations, [1] finished
  * games, [2] plies played, [3] wins of player 0, [4] wins of player 1, [5] draws, [6] descents,
