@@ -929,7 +929,7 @@ __device__ __forceinline__ void expand_backup_body(const View<typename R::Board>
     const int node = __shfl_sync(gmask, my_node, gbase + q);
     const int slot = __shfl_sync(gmask, my_slot, gbase + q);
     const size_t row = (nb + (size_t)node) * dm.RS;
-    float scale = 1.0f;
+    float denom = 1.0f;
     const bool mask = (dm.flags & FLAG_MASK_PRIORS) != 0u;
     typename R::Board nboard;
     if (mask) {  // extension: priors of illegal moves zeroed, the rest renormalised (the reference keeps the raw softmax)
@@ -941,13 +941,14 @@ __device__ __forceinline__ void expand_backup_body(const View<typename R::Board>
         if (legality.legal(nboard, a)) part += probs[(size_t)slot * dm.A + a];
 #pragma unroll
       for (int off = GW / 2; off > 0; off >>= 1) part += __shfl_xor_sync(gmask, part, off);
-      scale = part > 0.0f ? 1.0f / part : 1.0f;
+      denom = part > 0.0f ? part : 1.0f;  // no legal mass: the legal priors are all 0 and stay 0
     }
     for (int a = lane; a < dm.Apad; a += GW) {
       e.N[row + a] = 0;
       e.W[row + a] = 0.0f;
       float p = (a < dm.A) ? probs[(size_t)slot * dm.A + a] : 0.0f;
-      if (mask && a < dm.A) p = R{}.legal(nboard, a) ? p * scale : 0.0f;
+      // a division, not p * (1 / part): correctly rounded, and a lone legal move gets exactly 1
+      if (mask && a < dm.A) p = R{}.legal(nboard, a) ? __fdiv_rn(p, denom) : 0.0f;
       e.P[row + a] = p;
       e.C[row + a] = -1;
     }

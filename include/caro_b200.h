@@ -182,7 +182,9 @@ typedef struct {
 } caro_engine_config;
 
 /* Extensions, all off by default.  With any of them set the search is no longer the reference's (lib/mcts.py:248-287);
- * they are validated statistically (tests/test_gpu_round2.py), not bit for bit.
+ * virtual loss, masked priors and the fresh and recycled trees are checked bit for bit against their restatement in the test
+ * oracle (tests/test_gpu_search_matrix.py, tests/test_gpu_flag_matrix.py), and their effect on play statistically
+ * (tests/test_gpu_round2.py).
  *   VIRTUAL_LOSS   the batch_size descents of a minibatch are made one after the other per game, and every edge an
  *                  earlier descent of the same minibatch went through counts as one extra visit that lost
  *                  (N + 1, W - 1 in the PUCT score; the tree itself is not modified, so the back-up is unchanged): the
