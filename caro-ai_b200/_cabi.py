@@ -63,6 +63,8 @@ _SIGNATURES = {
     "caro_engine_counters": (C.c_int, [_P, C.POINTER(C.c_uint64 * 8), _P]),
     "caro_engine_set_resign": (C.c_int, [_P, C.c_int, C.c_double, C.c_double, _P]),
     "caro_engine_set_solver": (C.c_int, [_P, C.c_int, _P]),
+    "caro_engine_set_gumbel": (C.c_int, [_P, C.c_int, C.c_int, C.c_double, C.c_double, C.c_double, _P]),
+    "caro_engine_gumbel_plan": (C.c_int, [_P, C.c_int, C.c_int, C.c_int, C.c_int, _P]),
 }
 
 _lib = None

@@ -78,6 +78,8 @@ struct caro_engine {
   bool lean_tree = false;  // set while the parts pipeline issues launches: prefer tree kernels with few warps
   unsigned long long serial = 0;  // unique per created engine (keys the cached ply graph; heap addresses are reused)
   int solver_players = 0;  // the mask last enqueued by caro_engine_set_solver: picks the select / back-up instances
+  int gumbel_players = 0;  // the mask last enqueued by caro_engine_set_gumbel: picks the select / root policy / advance
+                           // instances and whether searches launch gumbel_plan_kernel
   size_t next_event() {
     if (events_used == events.size()) {
       cudaEvent_t ev;
@@ -154,6 +156,11 @@ void build_view(Carver& c, const Dims& dm, char* base, View<Board>* v) {
   // MCTS solver (extension): after the resignation regions, for the same reason
   CARVE(solver_params, "solver_params", SolverParams, 1);
   CARVE(solver_ctr, "solver_counters", unsigned long long, SCTR_COUNT);
+  // Gumbel root search (extension): after the solver regions, for the same reason
+  CARVE(gumbel_params, "gumbel_params", GumbelParams, 1);
+  CARVE(gumbel_g, "gumbel_g", double, dm.G, dm.A);
+  CARVE(gumbel_state, "gumbel_state", GumbelState, dm.G);
+  CARVE(gumbel_root, "gumbel_root", int16_t, dm.G, dm.B);
 #undef CARVE
 }
 
@@ -195,20 +202,20 @@ int fill_dims(const caro_engine_config* cfg, Dims* dm, int* max_plies) {
 inline cudaStream_t S(void* s) { return reinterpret_cast<cudaStream_t>(s); }
 
 // the select instance for the action count and the number of descents
-template <class R, bool SOLVER, class Board>
+template <class R, bool SOLVER, bool GUMBEL, class Board>
 void launch_select_kernel(const View<Board>& v, const R& rules, const Dims& dm, const SearchParams& sp, int batch,
                           const double* src, cudaStream_t st) {
   const long long groups = (long long)dm.G * batch;
   auto grid = [&](int gw) { return (unsigned)((groups * gw + 255) / 256); };
   const int A = dm.A;
-#define SELECT(GW, APL) select_kernel<R, GW, APL, SOLVER><<<grid(GW), 256, 0, st>>>(v, rules, dm, sp, batch, src)
+#define SELECT(GW, APL) select_kernel<R, GW, APL, SOLVER, GUMBEL><<<grid(GW), 256, 0, st>>>(v, rules, dm, sp, batch, src)
   // more descents than the GPU holds at once (5 blocks of 90-register threads per SM): the 72-register build keeps 7 blocks
   // per SM resident (-20 % at 16 k games, -12 % at 64 k; a few spilled words; CARO_SELECT_DENSE=0 switches it off)
   static const bool dense = !(getenv("CARO_SELECT_DENSE") && atoi(getenv("CARO_SELECT_DENSE")) == 0);
-  if (A <= 8 && dense && groups > 128ll * 5 * 148) select_thread_dense_kernel<R, 2, 7, SOLVER><<<(unsigned)((groups + 127) / 128), 128, 0, st>>>(v, rules, dm, sp, batch, src);
-  else if (A <= 8) select_thread_kernel<R, 2, SOLVER><<<(unsigned)((groups + 127) / 128), 128, 0, st>>>(v, rules, dm, sp, batch, src);
+  if (A <= 8 && dense && groups > 128ll * 5 * 148) select_thread_dense_kernel<R, 2, 7, SOLVER, GUMBEL><<<(unsigned)((groups + 127) / 128), 128, 0, st>>>(v, rules, dm, sp, batch, src);
+  else if (A <= 8) select_thread_kernel<R, 2, SOLVER, GUMBEL><<<(unsigned)((groups + 127) / 128), 128, 0, st>>>(v, rules, dm, sp, batch, src);
   else if constexpr (!std::is_same<R, C4Rules>::value) {  // lane-group kernels: m,n,k boards only (Connect4 has 7 actions)
-    if (A <= 16) select_thread_kernel<R, 4, SOLVER><<<(unsigned)((groups + 127) / 128), 128, 0, st>>>(v, rules, dm, sp, batch, src);
+    if (A <= 16) select_thread_kernel<R, 4, SOLVER, GUMBEL><<<(unsigned)((groups + 127) / 128), 128, 0, st>>>(v, rules, dm, sp, batch, src);
     else if (A <= 32) SELECT(32, 1);
     else if (A <= 64) SELECT(32, 2);
     else if (A <= 128) SELECT(32, 4);
@@ -220,7 +227,7 @@ void launch_select_kernel(const View<Board>& v, const R& rules, const Dims& dm, 
 // group width / actions per lane for the select and noise kernels
 template <class R, class Board>
 int launch_select(const View<Board>& v, const R& rules, const Dims& dm, const SearchParams& sp, int batch, int mb,
-                  const double* noise, double* noise_out, cudaStream_t st, int phase, bool solver) {
+                  const double* noise, double* noise_out, cudaStream_t st, int phase, bool solver, bool gumbel) {
   // phase 0: noise (unless injected) + select; 1: only generate the Philox noise of minibatch `mb` into v.noise;
   // 2: only select, reading v.noise as generated by an earlier phase-1 call (the self-play pipeline issues the
   // noise of minibatch i+1 underneath the network pass of minibatch i: it depends on (uid, ply, i) alone)
@@ -249,8 +256,9 @@ int launch_select(const View<Board>& v, const R& rules, const Dims& dm, const Se
     else select_vl_kernel<R><<<(unsigned)((dm.G + 63) / 64), 64, 0, st>>>(v, rules, dm, sp, batch, src);
     return caro_check_launch("select_vl_kernel");
   }
-  if (solver) launch_select_kernel<R, true>(v, rules, dm, sp, batch, src, st);
-  else launch_select_kernel<R, false>(v, rules, dm, sp, batch, src, st);
+  if (solver) launch_select_kernel<R, true, false>(v, rules, dm, sp, batch, src, st);
+  else if (gumbel) launch_select_kernel<R, false, true>(v, rules, dm, sp, batch, src, st);
+  else launch_select_kernel<R, false, false>(v, rules, dm, sp, batch, src, st);
   return caro_check_launch("select_kernel");
 }
 
@@ -423,9 +431,9 @@ int caro_engine_select(caro_engine* e, int batch, int minibatch_index, const dou
   if (batch <= 0 || batch > e->dm.B) return caro_fail(CARO_E_ARG, "batch exceeds max_batch");
   if (e->cfg.game == CARO_GAME_CONNECT4)
     return launch_select<C4Rules>(e->v_c4, C4Rules(), e->dm, e->sp, batch, minibatch_index, d_noise, d_noise_out, S(stream), 0,
-                                  e->solver_players != 0);
+                                  e->solver_players != 0, e->gumbel_players != 0);
   return launch_select<MnkRules>(e->v_mnk, e->mnk, e->dm, e->sp, batch, minibatch_index, d_noise, d_noise_out, S(stream), 0,
-                                 e->solver_players != 0);
+                                 e->solver_players != 0, e->gumbel_players != 0);
 }
 
 int caro_engine_plan(caro_engine* e, int batch, void* stream) {
@@ -479,14 +487,18 @@ int caro_engine_expand_backup(caro_engine* e, int batch, const float* d_probs, c
 // hand-offs are CUDA events, so that another engine's tree kernels can run underneath this engine's network pass.
 static int select_phase(caro_engine* e, int batch, int mb, int phase, cudaStream_t st) {
   if (e->cfg.game == CARO_GAME_CONNECT4)
-    return launch_select<C4Rules>(e->v_c4, C4Rules(), e->dm, e->sp, batch, mb, nullptr, nullptr, st, phase, e->solver_players != 0);
-  return launch_select<MnkRules>(e->v_mnk, e->mnk, e->dm, e->sp, batch, mb, nullptr, nullptr, st, phase, e->solver_players != 0);
+    return launch_select<C4Rules>(e->v_c4, C4Rules(), e->dm, e->sp, batch, mb, nullptr, nullptr, st, phase, e->solver_players != 0,
+                                  e->gumbel_players != 0);
+  return launch_select<MnkRules>(e->v_mnk, e->mnk, e->dm, e->sp, batch, mb, nullptr, nullptr, st, phase, e->solver_players != 0,
+                                 e->gumbel_players != 0);
 }
 
 // `prefetch`: 0 = noise + select as one step, 1 = minibatch i's noise was issued by the previous step, and this
 // step issues minibatch i+1's (if `more`) right behind its plan kernel, i.e. underneath its own network pass.
-static int search_step(caro_engine* e, caro_net* net, int i, int batch, int net_impl, cudaStream_t s_tree, cudaStream_t s_net,
-                       int prefetch = 0, bool more = false) {
+// Minibatch `k` of `count` of the search numbered `search_index` draws the noise of minibatch i = search_index + k.
+static int search_step(caro_engine* e, caro_net* net, int search_index, int k, int count, int batch, int net_impl,
+                       cudaStream_t s_tree, cudaStream_t s_net, int prefetch = 0, bool more = false) {
+  const int i = search_index + k;
   const bool c4 = e->cfg.game == CARO_GAME_CONNECT4;
   const void* lb = c4 ? (const void*)e->v_c4.leaf_board : (const void*)e->v_mnk.leaf_board;
   const uint8_t* lp = c4 ? e->v_c4.leaf_player : e->v_mnk.leaf_player;
@@ -504,6 +516,7 @@ static int search_step(caro_engine* e, caro_net* net, int i, int batch, int net_
     rc = select_phase(e, batch, i, 1, s_tree);
     e->span_end(4, s_tree);
   }
+  if (rc == CARO_OK && e->gumbel_players != 0) rc = caro_engine_gumbel_plan(e, search_index, k, count, batch, s_tree);
   e->span_begin(0, s_tree);
   if (rc == CARO_OK) rc = select_phase(e, batch, i, 2, s_tree);
   e->span_end(0, s_tree);
@@ -526,7 +539,7 @@ static int search_step(caro_engine* e, caro_net* net, int i, int batch, int net_
   e->span_begin(3, s_tree);
   if (rc == CARO_OK) rc = caro_engine_expand_backup(e, batch, pr, va, s_tree);
   e->span_end(3, s_tree);
-  e->launches += 5;
+  e->launches += e->gumbel_players != 0 ? 6 : 5;
   return rc;
 }
 
@@ -600,7 +613,7 @@ int caro_engine_search(caro_engine* e, caro_net* net, int count, int batch, int 
   if (!e || !net) return caro_fail(CARO_E_ARG, "null argument");
   if (first_minibatch < 0) return caro_fail(CARO_E_ARG, "first_minibatch must be >= 0");
   for (int i = 0; i < count; ++i) {
-    const int rc = search_step(e, net, first_minibatch + i, batch, net_impl, S(stream), S(stream));
+    const int rc = search_step(e, net, first_minibatch, i, count, batch, net_impl, S(stream), S(stream));
     if (rc != CARO_OK) return rc;
   }
   return CARO_OK;
@@ -619,7 +632,7 @@ static int multi_ply(caro_engine** es, int n, caro_net* net, int count, int batc
     ~LeanOff() { for (int h = 0; h < n; ++h) es[h]->lean_tree = false; }
   } lean_off{es, n};
   for (int i = 0; i < count && rc == CARO_OK; ++i)
-    for (int h = 0; h < n && rc == CARO_OK; ++h) rc = search_step(es[h], net, i, batch, net_impl, s_side[h], s_side[h], 1, i + 1 < count);
+    for (int h = 0; h < n && rc == CARO_OK; ++h) rc = search_step(es[h], net, 0, i, count, batch, net_impl, s_side[h], s_side[h], 1, i + 1 < count);
   for (int h = 0; h < n && rc == CARO_OK; ++h) {
     rc = caro_engine_advance(es[h], tau_plies, nullptr, auto_restart, first_player, nullptr, s_side[h]);
     es[h]->launches += 1;
@@ -718,10 +731,14 @@ int caro_engine_play_multi(caro_engine** engines, int n, caro_net* net, int move
 int caro_engine_root_policy(caro_engine* e, int tau_mode, int tau_plies, double* d_pi, float* d_q, int32_t* d_n, void* stream) {
   if (!e) return caro_fail(CARO_E_ARG, "null engine");
   const unsigned grid = (unsigned)((e->dm.G + 127) / 128);
-  if (e->cfg.game == CARO_GAME_CONNECT4)
-    root_policy_kernel<C4Rules><<<grid, 128, 0, S(stream)>>>(e->v_c4, C4Rules(), e->dm, tau_mode, tau_plies, d_pi, d_q, d_n);
-  else
-    root_policy_kernel<MnkRules><<<grid, 128, 0, S(stream)>>>(e->v_mnk, e->mnk, e->dm, tau_mode, tau_plies, d_pi, d_q, d_n);
+  const bool gum = e->gumbel_players != 0;
+  if (e->cfg.game == CARO_GAME_CONNECT4) {
+    if (gum) root_policy_kernel<C4Rules, true><<<grid, 128, 0, S(stream)>>>(e->v_c4, C4Rules(), e->dm, tau_mode, tau_plies, d_pi, d_q, d_n);
+    else root_policy_kernel<C4Rules, false><<<grid, 128, 0, S(stream)>>>(e->v_c4, C4Rules(), e->dm, tau_mode, tau_plies, d_pi, d_q, d_n);
+  } else {
+    if (gum) root_policy_kernel<MnkRules, true><<<grid, 128, 0, S(stream)>>>(e->v_mnk, e->mnk, e->dm, tau_mode, tau_plies, d_pi, d_q, d_n);
+    else root_policy_kernel<MnkRules, false><<<grid, 128, 0, S(stream)>>>(e->v_mnk, e->mnk, e->dm, tau_mode, tau_plies, d_pi, d_q, d_n);
+  }
   return caro_check_launch("root_policy_kernel");
 }
 
@@ -729,12 +746,17 @@ int caro_engine_advance(caro_engine* e, int tau_plies, const double* d_uniform, 
                         int32_t* d_action_out, void* stream) {
   if (!e) return caro_fail(CARO_E_ARG, "null engine");
   const unsigned grid = (unsigned)((e->dm.G + 127) / 128);
-  if (e->cfg.game == CARO_GAME_CONNECT4)
-    advance_kernel<C4Rules><<<grid, 128, 0, S(stream)>>>(e->v_c4, C4Rules(), e->dm, e->sp, tau_plies, d_uniform, auto_restart,
-                                                            first_player, d_action_out);
-  else
-    advance_kernel<MnkRules><<<grid, 128, 0, S(stream)>>>(e->v_mnk, e->mnk, e->dm, e->sp, tau_plies, d_uniform, auto_restart,
-                                                             first_player, d_action_out);
+#define LAUNCH_ADVANCE(R, V, RULES, GUM) \
+  advance_kernel<R, GUM><<<grid, 128, 0, S(stream)>>>(e->V, RULES, e->dm, e->sp, tau_plies, d_uniform, auto_restart, first_player, d_action_out)
+  const bool gum = e->gumbel_players != 0;
+  if (e->cfg.game == CARO_GAME_CONNECT4) {
+    if (gum) LAUNCH_ADVANCE(C4Rules, v_c4, C4Rules(), true);
+    else LAUNCH_ADVANCE(C4Rules, v_c4, C4Rules(), false);
+  } else {
+    if (gum) LAUNCH_ADVANCE(MnkRules, v_mnk, e->mnk, true);
+    else LAUNCH_ADVANCE(MnkRules, v_mnk, e->mnk, false);
+  }
+#undef LAUNCH_ADVANCE
   int rc = caro_check_launch("advance_kernel");
   if (rc == CARO_OK && (e->dm.flags & FLAG_COMPACT_TREE)) {  // drop what the move made unreachable, pack the arenas
     const int chunk = compact_chunk_nodes(e->dm);
@@ -796,6 +818,7 @@ int caro_engine_set_solver(caro_engine* e, int players, void* stream) {
     return caro_fail(CARO_E_ARG, "the solver does not run with virtual loss");
   if ((players == 1 || players == 2) && e->dm.tpg == 1)
     return caro_fail(CARO_E_ARG, "a per-player solver mask needs two trees per game (one tree serves both players)");
+  if (players != 0 && e->gumbel_players != 0) return caro_fail(CARO_E_ARG, "the solver does not run with the Gumbel root search");
   SolverParams p{};
   p.players = players;
   SolverParams* dst = e->cfg.game == CARO_GAME_CONNECT4 ? e->v_c4.solver_params : e->v_mnk.solver_params;
@@ -805,6 +828,48 @@ int caro_engine_set_solver(caro_engine* e, int players, void* stream) {
     caro_pipeline_forget(e->serial, 0);  // a captured ply graph holds the other select / back-up instances
   if (rc == CARO_OK) e->solver_players = players;
   return rc;
+}
+
+int caro_engine_set_gumbel(caro_engine* e, int players, int m, double c_visit, double c_scale, double gumbel_scale,
+                           void* stream) {
+  if (!e) return caro_fail(CARO_E_ARG, "null engine");
+  if (players < 0 || players > 3) return caro_fail(CARO_E_ARG, "gumbel players must be a mask in 0..3");
+  if ((players == 1 || players == 2) && e->dm.tpg == 1)
+    return caro_fail(CARO_E_ARG, "a per-player gumbel mask needs two trees per game (one tree serves both players)");
+  if (players != 0 && (e->dm.flags & FLAG_VIRTUAL_LOSS))
+    return caro_fail(CARO_E_ARG, "the Gumbel root search does not run with virtual loss");
+  if (players != 0 && e->solver_players != 0) return caro_fail(CARO_E_ARG, "the Gumbel root search does not run with the solver");
+  if (m < 1 || m > kGumbelMaxM) return caro_fail(CARO_E_ARG, "gumbel m must be in 1..32");
+  const double v[3] = {c_visit, c_scale, gumbel_scale};
+  for (double x : v)
+    if (!(x >= 0.0 && x <= 1.7976931348623157e308)) return caro_fail(CARO_E_ARG, "gumbel c_visit, c_scale and scale must be finite and >= 0");
+  GumbelParams p{};
+  p.players = players;
+  p.m = m;
+  p.c_visit = c_visit;
+  p.c_scale = c_scale;
+  p.gumbel_scale = gumbel_scale;
+  GumbelParams* dst = e->cfg.game == CARO_GAME_CONNECT4 ? e->v_c4.gumbel_params : e->v_mnk.gumbel_params;
+  set_gumbel_kernel<<<1, 1, 0, S(stream)>>>(dst, p);
+  const int rc = caro_check_launch("set_gumbel_kernel");
+  if (rc == CARO_OK && (players != 0) != (e->gumbel_players != 0))
+    caro_pipeline_forget(e->serial, 0);  // a captured ply graph holds the other instances (and no gumbel_plan_kernel)
+  if (rc == CARO_OK) e->gumbel_players = players;
+  return rc;
+}
+
+int caro_engine_gumbel_plan(caro_engine* e, int search_index, int minibatch, int count, int batch, void* stream) {
+  if (!e) return caro_fail(CARO_E_ARG, "null engine");
+  if (search_index < 0 || count < 1 || minibatch < 0 || minibatch >= count)
+    return caro_fail(CARO_E_ARG, "gumbel plan needs search_index >= 0 and 0 <= minibatch < count");
+  if (batch <= 0 || batch > e->dm.B) return caro_fail(CARO_E_ARG, "batch exceeds max_batch");
+  if (e->gumbel_players == 0) return CARO_OK;
+  const unsigned grid = (unsigned)(((long long)e->dm.G * 32 + 127) / 128);
+  if (e->cfg.game == CARO_GAME_CONNECT4)
+    gumbel_plan_kernel<C4Rules><<<grid, 128, 0, S(stream)>>>(e->v_c4, C4Rules(), e->dm, e->sp, search_index, minibatch, count, batch);
+  else
+    gumbel_plan_kernel<MnkRules><<<grid, 128, 0, S(stream)>>>(e->v_mnk, e->mnk, e->dm, e->sp, search_index, minibatch, count, batch);
+  return caro_check_launch("gumbel_plan_kernel");
 }
 
 int caro_engine_counters(caro_engine* e, uint64_t h_out[8], void* stream) {

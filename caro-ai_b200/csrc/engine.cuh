@@ -96,6 +96,26 @@ struct alignas(8) SolverParams {
 };
 enum { SCTR_STOPPED = 0, SCTR_PROVEN, SCTR_COUNT };
 
+// Gumbel root search (extension, off by default; include/caro_b200.h caro_engine_set_gumbel).  Read by
+// gumbel_plan_kernel and the GUMBEL instances of root_policy_kernel / advance_kernel at run time.
+struct alignas(8) GumbelParams {
+  int32_t players;      // bit p: searches whose root player is p search their root by Gumbel sequential halving
+  int32_t m;            // root actions sampled per search (1..32)
+  double c_visit, c_scale;  // sigma(q) = (c_visit + max_b N(b)) * c_scale * q
+  double gumbel_scale;  // scale of the Gumbel draws in the survivor score and the move
+};
+constexpr int kGumbelMaxM = 32;
+// Per game: where the current search stands (action indices only, so compaction and tree clears leave it valid)
+struct alignas(8) GumbelState {
+  int32_t i0;      // first minibatch of the search at which the root was in the tree (-1: not yet)
+  int32_t phase;   // current halving phase (-1: none ran)
+  int32_t kstart;  // local minibatch (k = i - i0) at which the current phase began
+  int16_t m;       // min(m, legal moves) of this search
+  int16_t r;       // current survivors
+  int16_t surv[kGumbelMaxM];  // survivors [0, r) in score order (best first)
+};
+static_assert(sizeof(GumbelState) == 80, "gumbel_state records are 80 bytes");
+
 struct SearchParams {
   double c_puct, alpha, explore;
   uint32_t seed_lo, seed_hi;
@@ -161,6 +181,11 @@ struct View {
   // ---- MCTS solver (extension) ------------------------------------------------------------------
   SolverParams* solver_params;     // [1]
   unsigned long long* solver_ctr;  // [SCTR_COUNT] descents stopped at a proven node, edges proven
+  // ---- Gumbel root search (extension) -----------------------------------------------------------
+  GumbelParams* gumbel_params;     // [1]
+  double* gumbel_g;                // [G][A] unscaled Gumbel draws of the current search
+  GumbelState* gumbel_state;       // [G]
+  int16_t* gumbel_root;            // [G][B] forced root action of each descent of the coming minibatch (-1: PUCT)
 };
 
 }  // namespace caro

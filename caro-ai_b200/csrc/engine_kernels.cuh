@@ -166,7 +166,9 @@ noise_kernel(const uint64_t* __restrict__ uid_g, const int32_t* __restrict__ ply
 // descent that reaches a proven node below the root stops there as a terminal (value +1 / -1 / 0 for the node's mover),
 // a proven root makes no descent at all, and LOSS edges are left out of the argmax.  (The lowest WIN edge of a node with
 // a WIN edge, and the argmax over LOSS edges when all legal edges are LOSS, are never taken here: such a node is proven.)
-template <class R, int GW, int APL, bool SOLVER>
+// GUMBEL (extension): a descent whose gumbel_root entry (written by gumbel_plan_kernel) is an action takes it at the root
+// without scoring the root; every other step, and every descent whose entry is -1, is the reference's.
+template <class R, int GW, int APL, bool SOLVER, bool GUMBEL>
 __device__ __forceinline__ void select_group_body(const View<typename R::Board>& e, const R& rules, const Dims& dm,
                                                   const SearchParams& sp, int batch, const double* __restrict__ noise_in,
                                                   long long gthread) {
@@ -185,6 +187,7 @@ __device__ __forceinline__ void select_group_body(const View<typename R::Board>&
   Board s = e.root_board[g];
   int who = e.root_player[g];
   const bool sol = SOLVER && solver_on(e, who);
+  const int forced = GUMBEL ? (int)e.gumbel_root[di] : -1;  // Gumbel root search: the planned root action, or -1
   const int tree = g * dm.tpg + (dm.tpg == 2 ? who : 0);
   const uint32_t gen = e.tree_gen[tree];
   const HashSlot* ht = e.ht + (size_t)tree * dm.hash_cap;
@@ -258,7 +261,10 @@ __device__ __forceinline__ void select_group_body(const View<typename R::Board>&
 
     double best = -INFINITY;
     int best_a = 0x7fffffff;
-    if (depth == 0) {
+    if (GUMBEL && depth == 0 && forced >= 0) {
+      best = 0.0;  // every lane agrees: the group argmax below keeps the forced action
+      best_a = forced;
+    } else if (depth == 0) {
       // ---- root: Dirichlet noise + float64 scores (lib/mcts.py:48-62,131-132) -------------
       double z[APL];
 #pragma unroll
@@ -347,7 +353,8 @@ __device__ __forceinline__ void select_group_body(const View<typename R::Board>&
 
 // SOLVER = false is the reference's search.  The host launches the SOLVER instance while the engine's solver mask is
 // non-zero (a run-time branch on the mask would cost the plain instances registers); it then checks the mask per game.
-template <class R, int GW, int APL, bool SOLVER>
+// GUMBEL instances likewise run only while the engine's Gumbel mask is non-zero (the two masks are never both non-zero).
+template <class R, int GW, int APL, bool SOLVER, bool GUMBEL>
 __global__ void __launch_bounds__(256, (APL == 1 && sizeof(typename R::Board) <= 16) ? 7 : (APL == 8 ? 2 : 1))
 select_kernel(View<typename R::Board> e, R rules, Dims dm, SearchParams sp, int batch,
               const double* __restrict__ noise_in) {
@@ -355,14 +362,14 @@ select_kernel(View<typename R::Board> e, R rules, Dims dm, SearchParams sp, int 
   if (gthread == 0) {
     *e.leaf_count = 0;  // plan_kernel (next launch on the stream) accumulates into it
   }
-  select_group_body<R, GW, APL, SOLVER>(e, rules, dm, sp, batch, noise_in, gthread);
+  select_group_body<R, GW, APL, SOLVER, GUMBEL>(e, rules, dm, sp, batch, noise_in, gthread);
 }
 
 // Thread-per-descent variant for small action spaces (A <= 16: Connect4, 3x3 / 4x4 boards).  The board update,
 // key and transposition probe are scalar work; with one lane-group per descent they are replicated on every
 // lane and the kernel becomes issue-bound (ncu: 12.7 M warp instructions per launch).  Here each lane owns a whole
 // descent and loops over the <= 16 actions; the arithmetic and its order are identical to select_kernel.
-template <class R, int ROWV, bool SOLVER>  // ROWV = Apad / 4 = number of 16-byte vectors per row; SOLVER: as select_group_body
+template <class R, int ROWV, bool SOLVER, bool GUMBEL>  // ROWV = Apad / 4 = number of 16-byte vectors per row; SOLVER, GUMBEL: as select_group_body
 __device__ __forceinline__ void select_thread_body(const View<typename R::Board>& e, const R& rules, const Dims& dm,
                                                    const SearchParams& sp, int batch, const double* __restrict__ noise_in,
                                                    long long grp) {
@@ -378,6 +385,7 @@ __device__ __forceinline__ void select_thread_body(const View<typename R::Board>
   Board s = e.root_board[g];
   int who = e.root_player[g];
   const bool sol = SOLVER && solver_on(e, who);
+  const int forced = GUMBEL ? (int)e.gumbel_root[di] : -1;  // Gumbel root search: the planned root action, or -1
   const int tree = g * dm.tpg + (dm.tpg == 2 ? who : 0);
   const uint32_t gen = e.tree_gen[tree];
   const HashSlot* ht = e.ht + (size_t)tree * dm.hash_cap;
@@ -441,7 +449,12 @@ __device__ __forceinline__ void select_thread_body(const View<typename R::Board>
     }
     double best = -INFINITY;
     int best_a = 0, best_c = -1;
-    if (depth == 0) {  // root: Dirichlet noise + float64 scores (lib/mcts.py:48-62,131-132)
+    if (GUMBEL && depth == 0 && forced >= 0) {
+      best_a = forced;
+#pragma unroll
+      for (int a = 0; a < ROWV * 4; ++a)
+        if (a == forced) best_c = c_loc[a];
+    } else if (depth == 0) {  // root: Dirichlet noise + float64 scores (lib/mcts.py:48-62,131-132)
       const double sq = sqrt((double)sum_n);
       const double* z = noise_in + ((size_t)g * batch + j) * A;
 #pragma unroll
@@ -505,24 +518,24 @@ __device__ __forceinline__ void select_thread_body(const View<typename R::Board>
   store_desc(e.desc + di, kind, who, depth, term_value, key, s);
 }
 
-template <class R, int ROWV, bool SOLVER>
+template <class R, int ROWV, bool SOLVER, bool GUMBEL>
 __global__ void __launch_bounds__(128)
 select_thread_kernel(View<typename R::Board> e, R rules, Dims dm, SearchParams sp, int batch,
                      const double* __restrict__ noise_in) {
   const long long grp = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (grp == 0) *e.leaf_count = 0;  // plan_kernel (next launch on the stream) accumulates into it
-  select_thread_body<R, ROWV, SOLVER>(e, rules, dm, sp, batch, noise_in, grp);
+  select_thread_body<R, ROWV, SOLVER, GUMBEL>(e, rules, dm, sp, batch, noise_in, grp);
 }
 
 // The same descent with at most 64 registers (8 blocks per SM instead of 5): for launches of more descents than fit the
 // GPU at once, where the number of resident warps, not the latency of one descent, sets the kernel's duration.
-template <class R, int ROWV, int BPS, bool SOLVER>
+template <class R, int ROWV, int BPS, bool SOLVER, bool GUMBEL>
 __global__ void __launch_bounds__(128, BPS)
 select_thread_dense_kernel(View<typename R::Board> e, R rules, Dims dm, SearchParams sp, int batch,
                            const double* __restrict__ noise_in) {
   const long long grp = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (grp == 0) *e.leaf_count = 0;
-  select_thread_body<R, ROWV, SOLVER>(e, rules, dm, sp, batch, noise_in, grp);
+  select_thread_body<R, ROWV, SOLVER, GUMBEL>(e, rules, dm, sp, batch, noise_in, grp);
 }
 
 // ------------------------------------------------------------- select with virtual loss (extension)
@@ -1107,7 +1120,230 @@ __device__ __forceinline__ int pi_count(int raw, const RootProof& rp) {
   return (rp.drop_loss && ((raw >> kProofShift) & 3) == PROOF_LOSS) ? 0 : (raw & kCountMask);
 }
 
+// ---------------------------------------------------------------------------------- Gumbel root search (extension)
+// The rule is stated in include/caro_b200.h (caro_engine_set_gumbel) and restated by tests/gumbel_reference.py.  All
+// arithmetic is float64, every sum runs in action order, ties go to the lowest action.
+template <class Board>
+__device__ __forceinline__ bool gumbel_on(const View<Board>& e, int who) { return (e.gumbel_params->players >> who) & 1; }
+
+// Q of a visited root edge as the root branch of select computes it: f32(W / N) once W has absorbed a float32 value,
+// else the float64 quotient of the python-float sum
+__device__ __forceinline__ double root_edge_q(int raw, float w) {
+  const int n = raw & kCountMask;
+  return raw < 0 ? (double)__fdiv_rn(w, (float)n) : __ddiv_rn((double)w, (double)n);
+}
+
+struct GumbelRoot {
+  double scale;  // (c_visit + max_b N(b)) * c_scale
+  double qbar;   // completed Q of an unvisited edge: prior-weighted mean Q of the visited legal edges (0: none visited)
+};
 template <class R>
+__device__ GumbelRoot gumbel_root_stats(const View<typename R::Board>& e, const R& rules, const typename R::Board& s, int A,
+                                        size_t row, const GumbelParams& gp) {
+  int max_n = 0;
+  double sp = 0.0, spq = 0.0;
+  for (int a = 0; a < A; ++a) {
+    if (!rules.legal(s, a)) continue;
+    const int raw = e.N[row + a];
+    const int n = raw & kCountMask;
+    max_n = n > max_n ? n : max_n;
+    if (n > 0) {
+      const double p = (double)e.P[row + a];
+      sp = __dadd_rn(sp, p);
+      spq = __dadd_rn(spq, __dmul_rn(p, root_edge_q(raw, e.W[row + a])));
+    }
+  }
+  GumbelRoot gr;
+  gr.scale = __dmul_rn(__dadd_rn(gp.c_visit, (double)max_n), gp.c_scale);
+  gr.qbar = sp > 0.0 ? __ddiv_rn(spq, sp) : 0.0;
+  return gr;
+}
+// sigma(q^(a)) with q^ = (q + 1) / 2
+template <class Board>
+__device__ __forceinline__ double gumbel_sigma(const View<Board>& e, size_t row, int a, const GumbelRoot& gr) {
+  const int raw = e.N[row + a];
+  const double q = (raw & kCountMask) > 0 ? root_edge_q(raw, e.W[row + a]) : gr.qbar;
+  return __dmul_rn(gr.scale, __dmul_rn(__dadd_rn(q, 1.0), 0.5));
+}
+// gumbel_scale * g + log P: the phase-0 score; score = that + sigma; the policy logit = log P + sigma
+__device__ __forceinline__ double gumbel_base(double gs, double g, float p) { return __dadd_rn(__dmul_rn(gs, g), log((double)p)); }
+
+// survivors kept by phase p of a search that samples m actions
+__device__ __forceinline__ int gumbel_survivors(int m, int p) {
+  const int c = (m + (1 << p) - 1) >> p;
+  const int r = c > 2 ? c : 2;
+  return r < m ? r : m;
+}
+__device__ __forceinline__ int gumbel_phases(int m) {  // H = ceil(log2 m)
+  int h = 0;
+  while ((1 << h) < m) ++h;
+  return h;
+}
+
+// pi' and the move of a Gumbel root, one thread (root_policy_kernel and advance_kernel)
+struct GumbelPolicy {
+  GumbelRoot gr;
+  double lmax, sum;  // largest legal logit; sum over legal actions of exp(logit - lmax), in action order
+  int nlegal, move;
+};
+template <class R>
+__device__ GumbelPolicy gumbel_policy(const View<typename R::Board>& e, const R& rules, const Dims& dm, int g, size_t row) {
+  const typename R::Board s = e.root_board[g];
+  const GumbelParams gp = *e.gumbel_params;
+  const int A = dm.A;
+  GumbelPolicy out;
+  out.gr = gumbel_root_stats<R>(e, rules, s, A, row, gp);
+  out.lmax = -INFINITY;
+  out.nlegal = 0;
+  for (int a = 0; a < A; ++a) {
+    if (!rules.legal(s, a)) continue;
+    ++out.nlegal;
+    const double l = __dadd_rn(log((double)e.P[row + a]), gumbel_sigma(e, row, a, out.gr));
+    out.lmax = l > out.lmax ? l : out.lmax;
+  }
+  out.sum = 0.0;
+  if (out.lmax > -INFINITY)
+    for (int a = 0; a < A; ++a)
+      if (rules.legal(s, a))
+        out.sum = __dadd_rn(out.sum, exp(__dsub_rn(__dadd_rn(log((double)e.P[row + a]), gumbel_sigma(e, row, a, out.gr)), out.lmax)));
+  // the move: argmax of the score over the current survivors, over every legal action when no phase ran
+  const GumbelState* st = e.gumbel_state + g;
+  const double* gg = e.gumbel_g + (size_t)g * A;
+  const int r = st->phase >= 0 ? st->r : 0;
+  double best = 0.0;
+  int best_a = -1;
+  for (int i = 0; i < (r > 0 ? r : A); ++i) {
+    const int a = r > 0 ? st->surv[i] : i;
+    if (r == 0 && !rules.legal(s, a)) continue;
+    const double sc = __dadd_rn(gumbel_base(gp.gumbel_scale, gg[a], e.P[row + a]), gumbel_sigma(e, row, a, out.gr));
+    if (best_a < 0 || sc > best || (sc == best && a < best_a)) {
+      best = sc;
+      best_a = a;
+    }
+  }
+  out.move = best_a;
+  return out;
+}
+// pi'(a) as stored (float32): softmax over the legal actions of log P + sigma, uniform when every legal logit is -inf
+template <class R>
+__device__ __forceinline__ float gumbel_pi(const GumbelPolicy& gpol, const View<typename R::Board>& e, const R& rules,
+                                           const typename R::Board& s, size_t row, int a) {
+  if (!rules.legal(s, a)) return 0.0f;
+  if (!(gpol.lmax > -INFINITY)) return (float)__ddiv_rn(1.0, (double)gpol.nlegal);
+  const double l = __dadd_rn(log((double)e.P[row + a]), gumbel_sigma(e, row, a, gpol.gr));
+  return (float)__ddiv_rn(exp(__dsub_rn(l, gpol.lmax)), gpol.sum);
+}
+
+// Before select, one warp per game: at minibatch 0 of a search the draws g and a fresh state; from the first minibatch i0
+// at which the root is in the tree, the survivors of the current phase and every descent's forced root action
+// (gumbel_root, -1 = PUCT as the reference).  Arguments by value, so a captured ply graph replays it correctly.
+template <class R>
+__global__ void __launch_bounds__(128)
+gumbel_plan_kernel(View<typename R::Board> e, R rules, Dims dm, SearchParams sp, int search_index, int mb, int count,
+                   int batch) {
+  constexpr int kMaxApl = 8;  // A <= 256
+  const int g = (int)(((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5);
+  const int lane = threadIdx.x & 31;
+  if (g >= dm.G) return;  // whole warps leave together
+  const int A = dm.A;
+  int16_t* out = e.gumbel_root + (size_t)g * dm.B;
+  GumbelState* st = e.gumbel_state + g;
+  const GumbelParams gp = *e.gumbel_params;
+  const bool on = e.status[g] == ST_ACTIVE && ((gp.players >> e.root_player[g]) & 1);
+  int i0 = -1, phase = -1, kstart = 0, m = 0, r = 0;
+  if (mb > 0) {
+    i0 = st->i0;
+    phase = st->phase;
+    kstart = st->kstart;
+    m = st->m;
+    r = st->r;
+  }
+  if (on && mb == 0) {
+    const uint64_t uid = e.uid[g];
+    for (int a = lane; a < A; a += 32)
+      e.gumbel_g[(size_t)g * A + a] = gumbel_draw(sp.seed_lo, sp.seed_hi, uid, (uint32_t)search_index, (uint32_t)e.ply[g], (uint32_t)a);
+  }
+  size_t nb = 0;
+  const int node = on ? root_node_of<R>(e, rules, dm, g, &nb) : -1;
+  if (node >= 0) {
+    const size_t row = (nb + (size_t)node) * dm.RS;
+    const typename R::Board s = e.root_board[g];
+    const double* gg = e.gumbel_g + (size_t)g * A;
+    if (i0 < 0) i0 = mb;
+    const int k = mb - i0, cp = count - i0;
+    if (phase < 0) {  // phase 0: the top m legal actions by gumbel_scale * g + log P
+      double bs[kMaxApl];
+      bool lg[kMaxApl];
+      int nl = 0, rank[kMaxApl];
+#pragma unroll
+      for (int i = 0; i < kMaxApl; ++i) {
+        const int a = lane + 32 * i;
+        lg[i] = a < A && rules.legal(s, a);
+        bs[i] = lg[i] ? gumbel_base(gp.gumbel_scale, gg[a], e.P[row + a]) : 0.0;
+        nl += lg[i] ? 1 : 0;
+        rank[i] = 0;
+      }
+#pragma unroll
+      for (int off = 16; off > 0; off >>= 1) nl += __shfl_xor_sync(0xffffffffu, nl, off);
+      m = gp.m < nl ? gp.m : nl;
+#pragma unroll
+      for (int i2 = 0; i2 < kMaxApl; ++i2) {
+        if (32 * i2 >= A) break;
+        for (int l = 0; l < 32; ++l) {
+          const double ob = __shfl_sync(0xffffffffu, bs[i2], l);
+          const int ol = __shfl_sync(0xffffffffu, lg[i2] ? 1 : 0, l);
+          const int b = l + 32 * i2;
+#pragma unroll
+          for (int i = 0; i < kMaxApl; ++i) {
+            const int a = lane + 32 * i;
+            rank[i] += (ol && (ob > bs[i] || (ob == bs[i] && b < a))) ? 1 : 0;
+          }
+        }
+      }
+#pragma unroll
+      for (int i = 0; i < kMaxApl; ++i)
+        if (lg[i] && rank[i] < m) st->surv[rank[i]] = (int16_t)(lane + 32 * i);
+      phase = 0;
+      kstart = 0;
+      r = m;
+      __syncwarp();
+    }
+    const int H = gumbel_phases(m);
+    const int p = (int)(((long long)k * H) / cp);
+    if (p != phase) {  // the top r_p of the current survivors by score on the tree as it stands
+      const GumbelRoot gr = gumbel_root_stats<R>(e, rules, s, A, row, gp);
+      const int rp = gumbel_survivors(m, p);
+      const int a = lane < r ? (int)st->surv[lane] : -1;
+      const double sc = lane < r ? __dadd_rn(gumbel_base(gp.gumbel_scale, gg[a], e.P[row + a]), gumbel_sigma(e, row, a, gr)) : 0.0;
+      int rank = 0;
+      for (int l = 0; l < r; ++l) {
+        const double ob = __shfl_sync(0xffffffffu, sc, l);
+        const int oa = __shfl_sync(0xffffffffu, a, l);
+        rank += (ob > sc || (ob == sc && oa < a)) ? 1 : 0;
+      }
+      __syncwarp();
+      if (lane < r && rank < rp) st->surv[rank] = (int16_t)a;
+      r = rp;
+      phase = p;
+      kstart = k;
+      __syncwarp();
+    }
+    for (int j = lane; j < batch; j += 32) out[j] = st->surv[((k - kstart) * batch + j) % r];
+  } else {
+    for (int j = lane; j < batch; j += 32) out[j] = -1;
+  }
+  if (lane == 0) {
+    st->i0 = i0;
+    st->phase = phase;
+    st->kstart = kstart;
+    st->m = (int16_t)m;
+    st->r = (int16_t)r;
+  }
+}
+
+// GUMBEL (extension): the instance the host launches while the engine's Gumbel mask is non-zero; a Gumbel root gives pi'
+// (tau_mode 1 or 2: the tau schedule does not apply) or a one-hot on the Gumbel move (tau_mode 0).
+template <class R, bool GUMBEL>
 __global__ void root_policy_kernel(View<typename R::Board> e, R rules, Dims dm, int tau_mode, int tau_plies,
                                    double* __restrict__ pi, float* __restrict__ qout, int32_t* __restrict__ nout) {
   const int g = blockIdx.x * blockDim.x + threadIdx.x;
@@ -1124,6 +1360,17 @@ __global__ void root_policy_kernel(View<typename R::Board> e, R rules, Dims dm, 
     return;
   }
   const size_t row = (nb + (size_t)node) * dm.RS;
+  if (GUMBEL && gumbel_on(e, e.root_player[g])) {
+    const GumbelPolicy gpol = gumbel_policy<R>(e, rules, dm, g, row);
+    const typename R::Board s = e.root_board[g];
+    for (int a = 0; a < A; ++a) {
+      const int n = e.N[row + a] & kCountMask;
+      if (pi) pi[(size_t)g * A + a] = tau_mode == 0 ? (a == gpol.move ? 1.0 : 0.0) : (double)gumbel_pi<R>(gpol, e, rules, s, row, a);
+      if (qout) qout[(size_t)g * A + a] = n > 0 ? __fdiv_rn(e.W[row + a], (float)n) : 0.0f;
+      if (nout) nout[(size_t)g * A + a] = n;
+    }
+    return;
+  }
   const int tau = tau_mode == 2 ? (e.ply[g] < tau_plies ? 1 : 0) : tau_mode;
   const RootProof rp = root_proof<R>(e, rules, dm, g, row);
   long long total = 0;
@@ -1274,7 +1521,8 @@ __device__ __forceinline__ void resign_game_start(const View<Board>& e, const Se
 
 // ----------------------------------------------------------------------------------- advance
 // One ply of lib/utils.py:76-106 for every active game.  One thread per game.
-template <class R>
+// GUMBEL (extension): as root_policy_kernel; a Gumbel root plays the Gumbel move and records pi' whatever the ply.
+template <class R, bool GUMBEL>
 __global__ void advance_kernel(View<typename R::Board> e, R rules, Dims dm, SearchParams sp, int tau_plies,
                                const double* __restrict__ uniform_in, int auto_restart, int first_player,
                                int32_t* __restrict__ action_out) {
@@ -1347,7 +1595,12 @@ __global__ void advance_kernel(View<typename R::Board> e, R rules, Dims dm, Sear
   const bool one_hot = tau == 0 || total <= 0 || pf.win_a >= 0;
   if (pf.win_a >= 0) best_a = pf.win_a;
   int action = best_a;
-  if (!one_hot) {
+  const bool gum = GUMBEL && node >= 0 && gumbel_on(e, who);
+  GumbelPolicy gpol;
+  if (gum) {
+    gpol = gumbel_policy<R>(e, rules, dm, g, row);
+    action = gpol.move;
+  } else if (!one_hot) {
     double last = 0.0;
     for (int a = 0; a < A; ++a) last = __dadd_rn(last, __ddiv_rn((double)pi_count(e.N[row + a], pf), (double)total));
     double c = 0.0;
@@ -1368,7 +1621,8 @@ __global__ void advance_kernel(View<typename R::Board> e, R rules, Dims dm, Sear
   e.hist_player[h] = (uint8_t)who;
   for (int a = 0; a < A; ++a) {
     float p;
-    if (one_hot) p = (a == best_a) ? 1.0f : 0.0f;
+    if (gum) p = gumbel_pi<R>(gpol, e, rules, e.root_board[g], row, a);
+    else if (one_hot) p = (a == best_a) ? 1.0f : 0.0f;
     else p = (float)__ddiv_rn((double)pi_count(e.N[row + a], pf), (double)total);
     e.hist_pi[h * A + a] = p;
   }
@@ -1509,6 +1763,7 @@ replay_gather_kernel(View<typename R::Board> e, R rules, Dims dm, const long lon
 // One thread: the parameters arrive by value and are stored on the stream, behind every earlier ply.
 __global__ void set_resign_kernel(ResignParams* __restrict__ dst, ResignParams p) { *dst = p; }
 __global__ void set_solver_kernel(SolverParams* __restrict__ dst, SolverParams p) { *dst = p; }
+__global__ void set_gumbel_kernel(GumbelParams* __restrict__ dst, GumbelParams p) { *dst = p; }
 
 // ------------------------------------------------------------------------------------- reset
 template <class R>

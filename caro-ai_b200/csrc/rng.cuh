@@ -42,7 +42,19 @@ CARO_HD double u01d(uint32_t hi, uint32_t lo) {
 
 // Stream tags
 enum : uint32_t { kStreamDirichlet = 0x44495243u, kStreamChoice = 0x43484F49u, kStreamFirst = 0x46495253u,
-                  kStreamResign = 0x52455347u };
+                  kStreamResign = 0x52455347u, kStreamGumbel = 0x47554D42u };
+
+// Gumbel(0, 1) draw of the Gumbel root search: g = -log(-log(u)) in double, u = k * 2^-53 from the top 53 bits k of the
+// Philox word pair, with k = 0 replaced by 1/2 so that u lies in the open interval (0, 1) and g is always finite.
+// Addressed by (seed, game uid, search index, ply, action).
+CARO_HD double gumbel_draw(uint32_t seed_lo, uint32_t seed_hi, uint64_t uid, uint32_t search_index, uint32_t ply,
+                           uint32_t action) {
+  const Philox4 r = philox4x32_10((uint32_t)uid, (uint32_t)(uid >> 32), search_index, (ply << 8) | action,
+                                  seed_lo ^ kStreamGumbel, seed_hi);
+  const uint64_t k = ((((uint64_t)r.v[0]) << 32) | r.v[1]) >> 11;
+  const double u = (k == 0 ? 0.5 : (double)k) * (1.0 / 9007199254740992.0);
+  return -log(-log(u));
+}
 
 // Device code uses the fast-math intrinsics: the noise only has to be distributed correctly, and whatever is
 // generated is what both the engine and (through noise_out) the oracle consume.

@@ -88,6 +88,8 @@ class SelfPlayEngine:
             e = elem.value
             if e == 1:
                 t = raw.view(shape)
+            elif e == 2:
+                t = raw.view(torch.int16).view(shape)
             elif e == 4:
                 t = raw.view(torch.int32).view(shape)
             elif e == 8:
@@ -201,6 +203,7 @@ class SelfPlayEngine:
         (CUDA tensors).  One host sync per minibatch (the leaf count)."""
         for i in range(count):
             noise = noise_fn(i) if noise_fn is not None else None
+            self.gumbel_plan(0, i, count, batch)
             self.select(batch, i, noise)
             self.plan(batch)
             n = self.leaf_count()
@@ -291,6 +294,35 @@ class SelfPlayEngine:
         """{"stopped": descents stopped at a proven node, "proven": edges proven}."""
         c = self.region("solver_counters").cpu().numpy()
         return {"stopped": int(c[0]), "proven": int(c[1])}
+
+    # ------------------------------------------------------------------ Gumbel root search (extension)
+    def set_gumbel(self, players: int, m: int = 16, c_visit: float = 50.0, c_scale: float = 0.1, scale: float = 1.0):
+        """Gumbel root search (extension, off by default; include/caro_b200.h caro_engine_set_gumbel): bit p of ``players``
+        makes the searches whose root player is p sample ``m`` root moves by Gumbel-top-k, split the descents over them
+        by sequential halving, record softmax(log P + sigma(completed Q)) as pi and play the best survivor.  0 switches it
+        off; 1 and 2 need two trees per game.  The defaults are the paper's and mctx's.  Enqueued on the current stream."""
+        _cabi.check(_cabi.lib().caro_engine_set_gumbel(self.handle, int(players), int(m), float(c_visit), float(c_scale),
+                                                       float(scale), self._stream()))
+
+    def gumbel_plan(self, search_index: int, minibatch: int, count: int, batch: int):
+        """The Gumbel step of the split API, before ``select`` of minibatch ``minibatch`` of a ``count``-minibatch search
+        (no-op while Gumbel is off)."""
+        _cabi.check(_cabi.lib().caro_engine_gumbel_plan(self.handle, int(search_index), int(minibatch), int(count), int(batch),
+                                                        self._stream()))
+
+    GUMBEL_STATE_DTYPE = np.dtype([("i0", np.int32), ("phase", np.int32), ("kstart", np.int32), ("m", np.int16),
+                                   ("r", np.int16), ("surv", np.int16, (32,))])
+
+    def gumbel_state(self) -> Dict[str, np.ndarray]:
+        """Host copies of the Gumbel regions: "g" float64 [G, A] draws of the current search, "i0", "phase", "kstart", "m",
+        "r" int [G] (i0 / phase -1: not yet), "survivors" (list per game, score order) and "forced" int [G, max_batch]
+        (the coming minibatch's forced root actions, -1 = PUCT)."""
+        st = self.region("gumbel_state").cpu().numpy().view(self.GUMBEL_STATE_DTYPE).reshape(-1)
+        out = {k: st[k].astype(np.int64) for k in ("i0", "phase", "kstart", "m", "r")}
+        out["survivors"] = [[int(a) for a in st["surv"][g][:max(int(st["r"][g]), 0)]] for g in range(self.G)]
+        out["g"] = self.region("gumbel_g").cpu().numpy().view(np.float64).reshape(self.G, self.A)
+        out["forced"] = self.region("gumbel_root").cpu().numpy().astype(np.int64)
+        return out
 
     RESIGN_RECORD_DTYPE = np.dtype([("min_stat", np.float64, (2,)), ("result", np.int32), ("plies", np.int32)])
 

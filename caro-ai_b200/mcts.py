@@ -36,11 +36,15 @@ EXPLORE = 0.25
 
 class MCTS:
     def __init__(self, game, node_capacity: int = 1 << 16, max_batch: int = 32, seed: int = 0,
-                 noise_fn: Optional[Callable[[int, int], np.ndarray]] = None, solver: bool = False):
+                 noise_fn: Optional[Callable[[int, int], np.ndarray]] = None, solver: bool = False, gumbel: bool = False):
         """``noise_fn(batch, actions) -> float64 [batch, actions]`` injects the Dirichlet draws (tests).
         ``solver`` (extension, default off): the MCTS solver (``SelfPlayEngine.set_solver``) for both players of the
-        shared tree; ``proof`` then shows which edges it proved."""
+        shared tree; ``proof`` then shows which edges it proved.
+        ``gumbel`` (extension, default off): every ``search_batch`` searches the root by Gumbel sequential halving
+        (``SelfPlayEngine.set_gumbel``, default parameters); ``get_policy_value`` then returns the improved policy for
+        tau 1 and a one-hot on the best survivor for tau 0."""
         self.solver = bool(solver)
+        self.gumbel = bool(gumbel)
         self.c_puct = C_PUCT
         self.precision = "auto"  # nn.Module nets: one-pass bf16 tower while it holds 1e-3 on probe positions, else bf16x3
         self.game = game
@@ -61,6 +65,8 @@ class MCTS:
                                           explore=EXPLORE, seed=self._cfg["seed"])
             if self.solver:
                 self._engine.set_solver(3)
+            if self.gumbel:
+                self._engine.set_gumbel(3)
         return self._engine
 
     @staticmethod
@@ -146,10 +152,14 @@ class MCTS:
             eng.search(dn, count, batch_size, first_minibatch=self._minibatches & 0x3FFFF)
             self._minibatches += count
             return
-        for _ in range(count):
-            self._step(eng, batch_size, net)
+        first = self._minibatches & 0x3FFFF
+        for i in range(count):
+            self._step(eng, batch_size, net, (first, i, count))
 
-    def _step(self, eng: SelfPlayEngine, batch: int, net) -> None:
+    def _step(self, eng: SelfPlayEngine, batch: int, net, search: Tuple[int, int, int] = None) -> None:
+        """``search`` = (search index, minibatch, count) of the Gumbel plan; a lone minibatch is a search of its own."""
+        first, i, count = search if search is not None else (self._minibatches & 0x3FFFF, 0, 1)
+        eng.gumbel_plan(first, i, count, batch)
         eng.select(batch, self._minibatches & 0x3FFFF, self._noise(batch))
         self._minibatches += 1
         eng.plan(batch)

@@ -28,6 +28,8 @@ def main(argv=None):
                         help="tensor-core precision: auto (default) keeps the one-pass bf16 tower only while it reproduces the fp32 priors to 1e-3 on probe positions")
     parser.add_argument("--solver", default=False, action="store_true",
                         help="extension: both players' searches use the MCTS solver (proven wins, losses and draws)")
+    parser.add_argument("--gumbel", default=False, action="store_true",
+                        help="extension: both players search their roots by Gumbel sequential halving")
     args = parser.parse_args(argv)
     game = get_game(args.game)
     nets = []
@@ -43,7 +45,7 @@ def main(argv=None):
             ts = time.time()
             s = play_games_batched(game, args.rounds, n1[1], n2[1], steps_before_tau_0=0, mcts_searches=cfg.PLAY_MCTS_SEARCHES,
                                    mcts_batch_size=cfg.PLAY_MCTS_BATCH_SIZE, trees_per_game=2, seed=idx1 * 1000 + idx2,
-                                   solver=args.solver or None)
+                                   solver=args.solver or None, gumbel=args.gumbel or None)
             wins, losses, draws = s["wins"], s["losses"], s["draws"]
             speed_games = args.rounds / (time.time() - ts)
             name_1, name_2 = n1[0], n2[0]

@@ -10,9 +10,11 @@ BOT_MCTS_BATCH_SIZE = 8  # config.py:23
 
 
 class Session:
-    def __init__(self, game, model_file, player_moves_first, solver: bool = False):
+    def __init__(self, game, model_file, player_moves_first, solver: bool = False, gumbel: bool = False):
         """``solver`` (extension, default off): the bot's search proves wins, losses and draws and never plays a move it
-        has proven to lose while another is left."""
+        has proven to lose while another is left.
+        ``gumbel`` (extension, default off): the bot searches its root by Gumbel sequential halving and plays the best
+        survivor."""
         self.game = game
         self.BOT_PLAYER = game.player_black
         self.USER_PLAYER = game.player_white
@@ -23,7 +25,7 @@ class Session:
         self.value = None
         self.player_moves_first = player_moves_first
         self.moves = []
-        self.mcts_store = mcts.MCTS(game, solver=solver)  # one tree for the whole session (play_session.py:20)
+        self.mcts_store = mcts.MCTS(game, solver=solver, gumbel=gumbel)  # one tree for the whole session (play_session.py:20)
 
     def move_player(self, move: int) -> bool:
         self.moves.append(move)

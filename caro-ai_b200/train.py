@@ -189,6 +189,11 @@ def parse_args(argv=None):
     p.add_argument("--solver", action="store_true",
                    help="extension: MCTS solver in the self-play searches (proven wins, losses and draws); the arena keeps "
                         "the reference's search")
+    p.add_argument("--gumbel", action="store_true",
+                   help="extension: Gumbel sequential halving at the self-play roots, trained on the improved policy; the "
+                        "arena keeps the reference's search")
+    p.add_argument("--gumbel-m", type=int, default=16, choices=range(1, 33), metavar="{1..32}",
+                   help="root moves sampled per self-play search with --gumbel")
     p.add_argument("--evaluate-every", type=int, default=cfg.EVALUATE_EVERY_STEP, help="arena evaluation period in steps")
     p.add_argument("--blocks", type=int, default=5, choices=range(1, 21), metavar="{1..20}",
                    help="residual blocks of the network (reference: 5)")
@@ -219,7 +224,7 @@ def main(argv=None):
     worker = SelfPlayWorker(game, args.games, cfg.MCTS_SEARCHES, cfg.MCTS_BATCH_SIZE, cfg.STEPS_BEFORE_TAU_0,
                             replay_steps=args.replay_steps, min_replay=cfg.REPLAY_BUFFER, seed=1000003 * rank + 17,
                             compact_tree=args.compact_tree, resign=args.resign, resign_playthrough=args.resign_playthrough,
-                            solver=args.solver)
+                            solver=args.solver, gumbel=args.gumbel_m if args.gumbel else False)
     step_idx = best_idx = 0
     with TBMeanTracker(writer, batch_size=10) as tb:
         while args.max_steps == 0 or step_idx < args.max_steps:

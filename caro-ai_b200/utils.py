@@ -90,10 +90,20 @@ def run_to_completion(eng: SelfPlayEngine, dn1, dn2, steps_before_tau_0: int, mc
             break
 
 
+def _player_mask(flag) -> int:
+    """None / False -> 0, True -> both players, a pair (net1's side, net2's side) -> bits 0 / 1."""
+    if flag is None or flag is False:
+        return 0
+    if flag is True:
+        return 3
+    return (1 if flag[0] else 0) | (2 if flag[1] else 0)
+
+
 def play_games_batched(game, n_games: int, net1, net2, steps_before_tau_0: int, mcts_searches: int,
                        mcts_batch_size: int, replay_buffer: Optional[collections.deque] = None,
                        net1_plays_first: Optional[bool] = None, trees_per_game: int = 2, node_capacity: Optional[int] = None,
-                       seed: int = 0, solver: Union[None, bool, Tuple[bool, bool]] = None) -> Dict[str, int]:
+                       seed: int = 0, solver: Union[None, bool, Tuple[bool, bool]] = None,
+                       gumbel: Union[None, bool, Tuple[bool, bool]] = None) -> Dict[str, int]:
     """``n_games`` independent ``play_game`` runs advanced in lock-step on the GPU (fresh trees per game =
     the ``mcts_stores=None`` semantics of play.py when ``trees_per_game=2``).  Returns the W/L/D tallies from
     net1's point of view plus counters; finished games' ``(state, player, probs, z)`` tuples are appended to
@@ -106,13 +116,11 @@ def play_games_batched(game, n_games: int, net1, net2, steps_before_tau_0: int, 
     ``net1_plays_first`` is None (the reference draws it per game: same distribution, lib/utils.py:66).
 
     ``solver`` (extension, default off): True runs the MCTS solver for both sides, a pair (net1's, net2's) for each side
-    on its own (two trees per game); the counts ``solver_stopped`` / ``solver_proven`` are added to the result."""
-    if solver is None or solver is False:
-        mask = 0
-    elif solver is True:
-        mask = 3
-    else:
-        mask = (1 if solver[0] else 0) | (2 if solver[1] else 0)
+    on its own (two trees per game); the counts ``solver_stopped`` / ``solver_proven`` are added to the result.
+
+    ``gumbel`` (extension, default off): True searches both sides' roots by Gumbel sequential halving with the default
+    parameters (``SelfPlayEngine.set_gumbel``), a pair (net1's, net2's) each side on its own (two trees per game)."""
+    mask, gmask = _player_mask(solver), _player_mask(gumbel)
     dn1 = net1 if isinstance(net1, model.DeviceNet) else model.DeviceNet(net1, game)
     dn2 = dn1 if net2 is net1 else (net2 if isinstance(net2, model.DeviceNet) else model.DeviceNet(net2, game))
     max_plies = _max_plies(game)
@@ -133,6 +141,8 @@ def play_games_batched(game, n_games: int, net1, net2, steps_before_tau_0: int, 
                              replay_capacity=count * max_plies if replay_buffer is not None else 0, seed=seed + part)
         if mask:
             eng.set_solver(mask)
+        if gmask:
+            eng.set_gumbel(gmask)
         eng.reset(first_player=first)
         run_to_completion(eng, dn1, dn2, steps_before_tau_0, mcts_searches, mcts_batch_size, first)
         if mask:
@@ -224,7 +234,7 @@ class SelfPlayWorker:
     def __init__(self, game, games: int, mcts_searches: int, mcts_batch_size: int, steps_before_tau_0: int,
                  replay_steps: int = 4, min_replay: int = 5000, seed: int = 0, node_capacity: Optional[int] = None,
                  compact_tree: bool = False, resign: Union[None, float, str] = None, resign_playthrough: float = 0.1,
-                 solver: bool = False):
+                 solver: bool = False, gumbel: Union[bool, int] = False):
         """``compact_tree``: drop unreachable nodes after every move (CARO_FLAG_COMPACT_TREE: bit-identical play, arenas of a
         few moves' searches instead of a whole game's -- what large boards need).
         ``resign`` (extension, default off): None plays every game to its end; a float is a fixed resignation threshold
@@ -233,7 +243,10 @@ class SelfPlayWorker:
         false-positive rate is <= 5 %, then resigns at that threshold with ``resign_playthrough`` played through.  The
         calibration runs after every step on every rank (one all-reduce).
         ``solver`` (extension, default off): the MCTS solver for the self-play searches (``SelfPlayEngine.set_solver``):
-        proven subtrees get no more descents, and pi / the replay rows keep no visit mass on proven-losing moves."""
+        proven subtrees get no more descents, and pi / the replay rows keep no visit mass on proven-losing moves.
+        ``gumbel`` (extension, default off): True, or an ``m`` (root moves sampled per search), searches every self-play
+        root by Gumbel sequential halving (``SelfPlayEngine.set_gumbel``); the replay rows then hold the improved policy
+        softmax(log P + sigma(completed Q)) instead of the visit distribution."""
         self.game, self.games = game, int(games)
         self.searches, self.batch, self.tau_plies = mcts_searches, mcts_batch_size, steps_before_tau_0
         max_plies = _max_plies(game)
@@ -246,6 +259,8 @@ class SelfPlayWorker:
                                      replay_capacity=self.replay_capacity, seed=seed, compact_tree=compact_tree)
         if solver:
             self.engine.set_solver(3)
+        if gumbel:
+            self.engine.set_gumbel(3, m=16 if gumbel is True else int(gumbel))
         self._last = self.engine.counters()
         if not (resign is None or resign == "auto" or isinstance(resign, (int, float))):
             raise ValueError("resign must be None, a threshold or 'auto'")

@@ -361,6 +361,58 @@ int caro_engine_set_resign(caro_engine* e, int enable, double threshold, double 
  * game (its tree serves both players), and a non-zero mask on a virtual-loss engine.  Enqueued on `stream`. */
 int caro_engine_set_solver(caro_engine* e, int players, void* stream);
 
+/* Gumbel root search (extension, off by default; Danihelka et al., "Policy improvement by planning with Gumbel", ICLR
+ * 2022).  Switched at run time by caro_engine_set_gumbel; the parameters live in device memory (region "gumbel_params"),
+ * and the engine re-captures a ply graph of caro_engine_play_multi when Gumbel goes from off to on or back.  Only the ROOT
+ * of a Gumbel player's searches changes: below it descents keep PUCT, and plan, expansion and back-up are unchanged.
+ * A search is one caro_engine_search / play / play_multi call: C minibatches i = 0 .. C-1 of b descents.
+ *   1. Draws.  At minibatch 0, for every action a: g(a) = -log(-log(u)) in double, u = k * 2^-53 with k the top 53 bits
+ *      of Philox stream kStreamGumbel addressed by (uid, search_index, ply, a) (k = 0 is replaced by 1/2: u lies in the
+ *      open interval (0, 1)).  search_index is 0 for play / play_multi and first_minibatch for caro_engine_search.  The
+ *      draws are stored unscaled in "gumbel_g" (double [G][A]); illegal actions' draws are never read.
+ *   2. Scores, all in double, with P the stored prior and N masked with the count mask:
+ *        q(a)     = Q of a visited edge as the root branch of select computes it (f32(W/N), or the float64 quotient of
+ *                   an edge whose W has absorbed no float32 value); for an unvisited edge, the prior-weighted mean
+ *                   sum_b P(b) q(b) / sum_b P(b) over the visited legal edges b (sums in action order), or 0 when no
+ *                   legal edge is visited.  (mctx's completed Q also mixes in the network value of the root, which the
+ *                   node record does not keep; it is left out.)
+ *        sigma(a) = ((c_visit + max_b N(b)) * c_scale) * ((q(a) + 1) * 0.5)
+ *        base(a)  = gumbel_scale * g(a) + log P(a)          (P = 0 gives -inf)
+ *        score(a) = base(a) + sigma(a);   logit(a) = log P(a) + sigma(a)
+ *      Every comparison breaks ties towards the lowest action index.
+ *   3. Schedule.  m = min(m_param, legal moves); H = ceil(log2 m) phases; phase p keeps r_p = min(m, max(2, ceil(m/2^p)))
+ *      survivors.  i0 = the first minibatch at which the root is in the tree; before it descents are not forced (the
+ *      first one expands the root as without Gumbel).  Local minibatch k = i - i0 of C' = C - i0 is in phase
+ *      floor(k H / C') (0 when H = 0).  At k = 0 (phase 0) the survivors are the top m legal actions by base; whenever the
+ *      phase changes (phases are skipped when C' < H) they become the top r_p of the current survivors by score, on the
+ *      tree as it stands after the previous minibatch's back-up.  Survivors are kept in score order (best first); descent j
+ *      of minibatch k takes survivor number ((k - k_phase_start) * b + j) mod r_p at the root.
+ *   4. Policy target pi'(a) = softmax over the legal actions of logit, on the final tree: exp(logit - max) summed over the
+ *      legal actions in action order, each quotient stored as float32; uniform over the legal moves when every legal
+ *      logit is -inf.  pi' replaces the visit distribution in the history and the replay ring (z is unchanged), and
+ *      caro_engine_root_policy returns it for tau_mode 1 and 2 (the tau schedule does not apply).
+ *   5. Move = argmax of score over the current survivors on the final tree (over every legal action when no phase ran).
+ *      caro_engine_root_policy with tau_mode 0 returns a one-hot on it.  The Philox choice stream is not consumed
+ *      differently, so a non-Gumbel player's moves do not shift.
+ * Regions: "gumbel_params" {int32 players, int32 m, double c_visit, double c_scale, double gumbel_scale};
+ *          "gumbel_g" double [G][A]; "gumbel_state" [G] records of 80 bytes {int32 i0 (-1: root not yet in the tree),
+ *          int32 phase (-1: none ran), int32 k_phase_start, int16 m, int16 r, int16 survivors[32]}; "gumbel_root"
+ *          int16 [G][max_batch]: the forced root action of each descent of the coming minibatch, or -1.  They follow every
+ *          other region; zero means off. */
+/* players: bit p = searches whose root player is p use the Gumbel root search.  Returns CARO_E_ARG (before touching the
+ * device) for a null handle, a mask outside 0..3, a mask of 1 or 2 with one tree per game, a non-zero mask on a
+ * virtual-loss engine or while the solver mask is non-zero, m outside 1..32, and a negative, NaN or infinite c_visit,
+ * c_scale or gumbel_scale.  (caro_engine_set_solver in turn refuses a non-zero mask while Gumbel is on.)  Enqueued on
+ * `stream`.  Defaults of the paper and mctx: m 16, c_visit 50, c_scale 0.1, gumbel_scale 1. */
+int caro_engine_set_gumbel(caro_engine* e, int players, int m, double c_visit, double c_scale, double gumbel_scale,
+                           void* stream);
+/* The split-API step that callers supplying their own network outputs enqueue before caro_engine_select of minibatch
+ * `minibatch` (0 .. count-1) of a search of `count` minibatches (caro_engine_search, play and play_multi enqueue it
+ * themselves): the draws at minibatch 0, the phase and survivors, and "gumbel_root".  Returns CARO_E_ARG for a null
+ * handle, search_index < 0, count < 1, minibatch outside 0..count-1 or a batch outside 1..max_batch; does nothing while
+ * Gumbel is off. */
+int caro_engine_gumbel_plan(caro_engine* e, int search_index, int minibatch, int count, int batch, void* stream);
+
 /* Host copies of the 64-bit counters (synchronises `stream`): [0] leaf evaluations, [1] finished
  * games, [2] plies played, [3] wins of player 0, [4] wins of player 1, [5] draws, [6] descents,
  * [7] error flags (bit 0 arena full, bit 1 replay overrun, bit 2 illegal action sampled). */
